@@ -72,7 +72,12 @@ def parse():
     ap.add_argument("--band-width", type=int, default=32768)
     ap.add_argument("--band-steps", type=int, default=10)
     ap.add_argument("--sigma", type=float, default=SIGMA)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the edge maps of the last step (rank 0's share) to DIR/*.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs dumps the B200 arm's maps; --impl reference has none")
+    return a
 
 
 def peaks():
@@ -83,6 +88,31 @@ def peaks():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md, 6.65 TB/s)"
+
+
+DUMP_SAMPLE_PX = 4 << 20   # float32 values + float64 indices: 48 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(directory, edges):
+    """--dump-outputs: what the timed path returned in its last step, for comparing two builds output for output.  The inputs are
+    seeded, so the same arguments give the same frames and the same sample on every run.
+      edges.npy            float32 0 / 255: every pixel of the maps, or a fixed, seeded sample of DUMP_SAMPLE_PX pixels when larger
+      edges_index.npy      float64: the flat C-order index of each value of edges.npy in the (frames, height, width) maps
+      edges_per_frame.npy  float64: edge pixels of every frame, counted over the whole map (covers what the sample leaves out)"""
+    import numpy as np
+    import torch
+
+    maps = edges.reshape(-1, edges.shape[-2], edges.shape[-1])
+    flat = maps.reshape(-1)
+    if flat.numel() <= DUMP_SAMPLE_PX:
+        idx = np.arange(flat.numel(), dtype=np.int64)
+    else:
+        idx = np.unique(np.random.default_rng(1234).integers(0, flat.numel(), DUMP_SAMPLE_PX, dtype=np.int64))
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "edges.npy", flat[torch.from_numpy(idx).to(flat.device)].float().cpu().numpy())
+    np.save(out / "edges_index.npy", idx.astype(np.float64))
+    np.save(out / "edges_per_frame.npy", torch.count_nonzero(maps.reshape(maps.shape[0], -1), dim=1).cpu().numpy().astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -308,6 +338,8 @@ def run_b200(a, rank, world, local_rank):
     launches = ctx.kernel_launches - l0
     ms = env.max_over_ranks(e0.elapsed_time(e1))
     value = n_total * h * w * a.steps / (ms * 1e-3) / 1e6
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, d_out[:n])   # before the legs below reuse d_out
 
     edges = C.c_ulonglong()
     check(lib.b200_count_edges_device(ctx.handle, d_out.data_ptr(), px, C.byref(edges)))
@@ -580,9 +612,10 @@ def run_b200(a, rank, world, local_rank):
 # ----------------------------------------------------------------------------------------------------
 # GPU arm, row bands of one image
 # ----------------------------------------------------------------------------------------------------
-def bands_measure(a, env, steps, warmup):
+def bands_measure(a, env, steps, warmup, dump=None):
     """configs[4]: one --band-height x --band-width image, row-band sharded over the GPUs; a step = halo exchange + front kernel +
-    band-local labelling + boundary-record exchange + cross-band union + finalisation (b200_bands_run, csrc/bands_mgpu.cu)."""
+    band-local labelling + boundary-record exchange + cross-band union + finalisation (b200_bands_run, csrc/bands_mgpu.cu).
+    dump: directory for rank 0's band of the p2p run's last map (dump_outputs)."""
     torch, dist, check, lib, ctx = env.torch, env.dist, env.check, env.lib, env.ctx
     from canny_edge_b200 import sharded
 
@@ -619,6 +652,8 @@ def bands_measure(a, env, steps, warmup):
         pipe.check()
         launches = ctx.kernel_launches - l0
         ms = env.max_over_ranks(e0.elapsed_time(e1))
+        if dump and rank == 0 and name == "p2p":
+            dump_outputs(dump, edges)
         cnt, hsh = C.c_ulonglong(), C.c_ulonglong()
         check(lib.b200_count_edges_device(ctx.handle, edges.data_ptr(), edges.numel(), C.byref(cnt)))
         check(lib.b200_hash_edges_device(ctx.handle, edges.data_ptr(), edges.numel(), g.row0 * W, C.byref(hsh)))
@@ -656,7 +691,7 @@ def bands_measure(a, env, steps, warmup):
 
 def run_bands(a, rank, world, local_rank):
     env = Env(rank, world, local_rank)
-    b = bands_measure(a, env, a.steps, a.warmup)
+    b = bands_measure(a, env, a.steps, a.warmup, dump=a.dump_outputs)
     if rank == 0:
         peak, peak_src = peaks()
         print(json.dumps({

@@ -1,7 +1,8 @@
 """CPU tests that PIN the oracle (oracle/canny_oracle.c):
   1. every value-pinning vector of the reference's own tests/utils/test_utils.cpp;
   2. golden fixtures generated from the compiled, unmodified reference (tests/golden/make_golden.py);
-  3. when oracle/_ref/libcanny_ref.so is present, the compiled reference itself on seeded random input.
+  3. stored outputs on 400 seeded random cases and a 1080p frame (tests/golden/make_golden_cases.py), checked against the compiled
+     reference itself wherever oracle/_ref/libcanny_ref.so is present.
 """
 import hashlib
 import json
@@ -160,8 +161,16 @@ def test_golden_hysteresis_cases(oracle):
         assert ((oracle.hysteresis(z[f"h{i}_in"], 20, 60) == 255) == (z[f"h{i}_out"] == 1)).all(), i
 
 
-# ---- the compiled reference itself (authoring container / prebuilt .so) -------------------------------
-def test_oracle_equals_reference_random(oracle, ref):
+# ---- seeded random cases and a 1080p frame: stored outputs, and the compiled reference where it is built ----------
+# tests/golden/reference_random_cases.json and reference_1080p.npz hold, for every case, sha256 digests of the five planes (and
+# the 1080p edge map bit-packed); tests/golden/make_golden_cases.py writes them.  Both tests compare the oracle with those stored
+# outputs on every checkout and, where oracle/_ref/libcanny_ref.so is built, also check the stored outputs against the compiled
+# reference itself.
+PLANES = ("blur", "mag", "ang", "nms", "edges")
+
+
+def reference_random_cases():
+    """The 400 seeded cases: (t, img, sigma, lo, hi)."""
     rng = np.random.default_rng(1)
     for t in range(400):
         h, w = (int(v) for v in rng.integers(2, 48, 2))
@@ -176,19 +185,53 @@ def test_oracle_equals_reference_random(oracle, ref):
         img = img.astype(np.uint8)
         lo = int(rng.integers(0, 100))
         hi = int(rng.integers(lo + 1, 256))
-        blur, mag, ang, nms, edges = oracle.canny(img, sigma, lo, hi, steps=True)
-        b2 = ref.gaussian(img, sigma)
-        m2, a2 = ref.sobel(b2)
-        n2 = ref.nonmaximal(m2, a2)
-        assert (blur == b2).all() and (mag == m2).all() and (ang == a2).all() and (nms == n2).all(), t
-        assert (edges == ref.canny(img, sigma, lo, hi)).all(), t
-        assert (oracle.gaussian_kernel(sigma)[0] == ref.gaussian_kernel(sigma)[0]).all()
+        yield t, img, sigma, lo, hi
 
 
-def test_oracle_equals_reference_1080p(oracle, ref):
+def reference_planes(ref, img, sigma, lo, hi):
+    """The compiled reference's five planes, stage by stage, with its whole-pipeline edge map checked against the staged one."""
+    blur = ref.gaussian(img, sigma)
+    mag, ang = ref.sobel(blur)
+    nms = ref.nonmaximal(mag, ang)
+    edges = ref.canny(img, sigma, lo, hi)
+    assert (ref.hysteresis(nms, lo, hi) == edges).all()
+    return blur, mag, ang, nms, edges
+
+
+def frame_1080p():
     import canny_edge_b200 as cb
-    img = cb.synth_host(1, 1080, 1920, kind=0, seed=1234)[0]
-    assert (oracle.canny(img, 1.4, 20, 60) == ref.canny(img, 1.4, 20, 60)).all()
+    return cb.synth_host(1, 1080, 1920, kind=0, seed=1234)[0]
+
+
+def test_oracle_equals_reference_random(oracle):
+    from oracle.bindings import Ref
+    ref = Ref() if Ref.available() else None
+    gold = json.loads((GOLD / "reference_random_cases.json").read_text())
+    assert len(gold["cases"]) == 400
+    for t, img, sigma, lo, hi in reference_random_cases():
+        want = gold["cases"][t]
+        assert (sha(img), sigma, lo, hi) == (want["img"], want["sigma"], want["lo"], want["hi"]), f"case {t}: the seeded input changed"
+        got = oracle.canny(img, sigma, lo, hi, steps=True)
+        for name, plane in zip(PLANES, got):
+            assert sha(plane) == want[name], f"case {t} {img.shape} sigma={sigma} {lo}/{hi}: {name} differs from the stored output"
+        assert sha(oracle.gaussian_kernel(sigma)[0]) == gold["kernels"][str(sigma)]
+        if ref is not None:
+            for name, plane in zip(PLANES, reference_planes(ref, img, sigma, lo, hi)):
+                assert sha(plane) == want[name], f"case {t}: the compiled reference's {name} differs from the stored output"
+            assert sha(ref.gaussian_kernel(sigma)[0]) == gold["kernels"][str(sigma)]
+
+
+def test_oracle_equals_reference_1080p(oracle):
+    from oracle.bindings import Ref
+    z = np.load(GOLD / "reference_1080p.npz")
+    img = frame_1080p()
+    assert sha(img) == str(z["img_sha256"]), "the seeded 1080p input changed"
+    want = np.unpackbits(z["edges_bits"])[: img.size].reshape(img.shape).astype(np.int16) * 255
+    assert int((want == 255).sum()) == int(z["edge_pixels"])
+    got = oracle.canny(img, 1.4, 20, 60)
+    assert (got == want).all(), f"{int((got != want).sum())} pixels differ from the stored edge map"
+    if Ref.available():
+        assert (Ref().canny(img, 1.4, 20, 60) == want).all(), "the compiled reference differs from the stored edge map"
 
 
 def test_oracle_workload_generator_matches_product_generator():

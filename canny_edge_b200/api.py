@@ -202,6 +202,27 @@ def canny_batch_device_bgr_ptr(ctx: Context, d_bgr: int, n: int, h: int, w: int,
                                              int(max_val), C.c_void_p(d_edges)))
 
 
+def canny_batch_device_strided_ptr(ctx: Optional[Context], d_frames: int, in_row_pitch: int, in_frame_stride: int, n: int, h: int,
+                                   w: int, sigma: float, min_val: int, max_val: int, d_edges: int, out_row_pitch: int,
+                                   out_frame_stride: int) -> None:
+    """Raw device pointers with byte strides (b200_canny_batch_device_strided): pixel (f, y, x) is read at
+    d_frames + f*in_frame_stride + y*in_row_pitch + x and written at d_edges + f*out_frame_stride + y*out_row_pitch + x; no other
+    byte of the output is touched.  Asynchronous on the context's stream."""
+    check(load().b200_canny_batch_device_strided(_h(ctx), C.c_void_p(d_frames), int(in_row_pitch), int(in_frame_stride), n, h, w,
+                                                 C.c_float(sigma), int(min_val), int(max_val), C.c_void_p(d_edges),
+                                                 int(out_row_pitch), int(out_frame_stride)))
+
+
+def canny_batch_device_bgr_strided_ptr(ctx: Optional[Context], d_bgr: int, in_row_pitch: int, in_frame_stride: int, n: int, h: int,
+                                       w: int, sigma: float, min_val: int, max_val: int, d_edges: int, out_row_pitch: int,
+                                       out_frame_stride: int) -> None:
+    """Interleaved B,G,R frames with byte strides (b200_canny_batch_device_bgr_strided): pixel (f, y, x) is the 3 bytes at
+    d_bgr + f*in_frame_stride + y*in_row_pitch + 3*x.  Asynchronous on the context's stream."""
+    check(load().b200_canny_batch_device_bgr_strided(_h(ctx), C.c_void_p(d_bgr), int(in_row_pitch), int(in_frame_stride), n, h, w,
+                                                     C.c_float(sigma), int(min_val), int(max_val), C.c_void_p(d_edges),
+                                                     int(out_row_pitch), int(out_frame_stride)))
+
+
 def synth_host(n: int, h: int, w: int, kind: int = 0, seed: int = 1234, first_frame: int = 0) -> np.ndarray:
     out = np.empty((n, h, w), np.uint8)
     check(load().b200_synth_host(_ptr(out), n, h, w, kind, C.c_uint64(seed), first_frame))

@@ -316,18 +316,29 @@ static int check_thresholds(int lo, int hi) {
     return B200_OK;
 }
 
+// Byte strides of the caller's frames and edge maps (b200_canny_batch_device_strided); null means dense: rows of width (3*width
+// for BGR) bytes, frames of height rows
+struct FrameLayout {
+    long long in_pitch, in_frame_stride, out_pitch, out_frame_stride;
+};
+
 // Runs front + hysteresis on device-resident frames [f0, f0+nf) using workspace slot `slot` on stream st.
 // bgr: d_in holds interleaved B,G,R frames (3 bytes per pixel) and the front kernel converts while staging (front3_bgr_supports)
 // bands_hint > 0: row bands per frame for the front kernel's grid (0: the launcher's own choice)
+// lay: strides of d_in and d_out (null: dense).  The union-find slots and the weak-pixel list stay dense whatever they are.
 static int run_frames_device(b200_ctx* ctx, cudaStream_t st, int slot, const uint8_t* d_in, uint8_t* d_out, int nf, int h,
                              int w, int lo, int hi, int16_t* blur, int16_t* mag, int16_t* ang, int16_t* nms, bool bgr = false,
-                             int bands_hint = 0) {
+                             int bands_hint = 0, const FrameLayout* lay = nullptr) {
     const long long px = (long long)h * w;
+    const int bpp = bgr ? 3 : 1;
+    const FrameLayout dense_layout = {bpp * (long long)w, bpp * px, w, px};
+    if (!lay) lay = &dense_layout;
     FrontParams fp;
     memset(&fp, 0, sizeof(fp));
-    fp.in = d_in; fp.in_frame_stride = bgr ? 3 * px : px; fp.in_bgr = bgr ? 1 : 0;
+    fp.in = d_in; fp.in_pitch = lay->in_pitch; fp.in_frame_stride = lay->in_frame_stride; fp.in_bgr = bgr ? 1 : 0;
     fp.in_row0 = 0; fp.in_rows = h; fp.width = w; fp.height = h;
-    fp.out_row0 = 0; fp.out_rows = h; fp.n_frames = nf; fp.cls = d_out; fp.out_frame_stride = px;
+    fp.out_row0 = 0; fp.out_rows = h; fp.n_frames = nf; fp.out_frame_stride = px;
+    fp.cls = d_out; fp.cls_pitch = lay->out_pitch; fp.cls_frame_stride = lay->out_frame_stride;
     fp.blur = blur; fp.mag = mag; fp.ang = ang; fp.nms = nms;
     fp.tiles_y = bands_hint;
     fp.w = ctx->gauss.d_w; fp.count = ctx->gauss.d_count; fp.radius = ctx->gauss.radius;
@@ -350,7 +361,7 @@ static int run_frames_device(b200_ctx* ctx, cudaStream_t st, int slot, const uin
     const long long thresh = (long long)nf * px / dense_div;   // n * dense_div > px  <=>  n > floor(px / dense_div)
     HystParams hp;
     memset(&hp, 0, sizeof(hp));
-    hp.cls = d_out;
+    hp.cls = d_out; hp.cls_pitch = lay->out_pitch; hp.cls_frame_stride = lay->out_frame_stride;
     hp.list = (sparse && !dense) ? fp.kept_list : nullptr;
     hp.ctr = sparse ? fp.kept_count : nullptr;
     hp.h_kept = ctx->d_kept + slot;
@@ -370,11 +381,12 @@ static int run_frames_device(b200_ctx* ctx, cudaStream_t st, int slot, const uin
 }
 
 // whether launch_front takes these interleaved B,G,R frames directly (fused conversion) under the context's current sigma
-static bool bgr_fused_ok(const b200_ctx* ctx, const uint8_t* d_bgr, int h, int w) {
+static bool bgr_fused_ok(const b200_ctx* ctx, const uint8_t* d_bgr, int n, int h, int w, long long pitch, long long frame_stride) {
     static const int force = [] { const char* e = getenv("B200_CANNY_FRONT"); return e ? atoi(e) : 0; }();
     FrontParams fp;
     memset(&fp, 0, sizeof(fp));
-    fp.in = d_bgr; fp.in_frame_stride = 3LL * h * w; fp.width = w; fp.radius = ctx->gauss.radius;
+    fp.in = d_bgr; fp.in_pitch = pitch; fp.in_frame_stride = frame_stride; fp.n_frames = n; fp.in_rows = h; fp.width = w;
+    fp.radius = ctx->gauss.radius;
     return force == 0 && !ctx->gauss.tiny && front3_bgr_supports(fp);
 }
 
@@ -438,6 +450,7 @@ int b200_ctx_create(int device, b200_ctx** out) {
             CB_CUDA(cudaEventCreateWithFlags(&c->ev_in[i], cudaEventDisableTiming));
         }
         CB_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
+        CB_CUDA(cudaEventCreateWithFlags(&c->ev_switch, cudaEventDisableTiming));
         CB_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&c->h_kept), 4 * sizeof(unsigned int), cudaHostAllocMapped));
         memset(c->h_kept, 0, 4 * sizeof(unsigned int));
         CB_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void**>(&c->d_kept), c->h_kept, 0));
@@ -472,6 +485,7 @@ int b200_ctx_destroy(b200_ctx* c) {
     }
     delete c->pool;
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
+    if (c->ev_switch) cudaEventDestroy(c->ev_switch);
     if (c->own_stream) cudaStreamDestroy(c->own_stream);
     {
         std::lock_guard<std::mutex> lk(g_default_mu);
@@ -533,7 +547,15 @@ int b200_ctx_front_kernel_stats(const b200_ctx* ctx, long long* fast_launches, l
 
 int b200_ctx_set_stream(b200_ctx* ctx, void* cuda_stream) {
     CB_TRY(resolve_ctx(ctx));
-    ctx->stream = cuda_stream ? reinterpret_cast<cudaStream_t>(cuda_stream) : ctx->own_stream;
+    cudaStream_t next = cuda_stream ? reinterpret_cast<cudaStream_t>(cuda_stream) : ctx->own_stream;
+    if (next != ctx->stream) {
+        // Work already issued through the context (every call joins its side streams back into ctx->stream) uses the context's
+        // workspace — union-find slots, weak-pixel lists and their counters: the new stream starts after it, so calls on two
+        // streams never run on the same slots at once.
+        CB_CUDA(cudaEventRecord(ctx->ev_switch, ctx->stream));
+        CB_CUDA(cudaStreamWaitEvent(next, ctx->ev_switch, 0));
+        ctx->stream = next;
+    }
     return B200_OK;
 }
 int b200_ctx_synchronize(b200_ctx* ctx) {
@@ -599,8 +621,8 @@ int b200_gaussian(b200_ctx* ctx, const uint8_t* img, float sigma, int h, int w, 
     CB_CUDA(cudaMemcpyAsync(pl.in, img, (size_t)px, cudaMemcpyHostToDevice, st));
     FrontParams fp;
     memset(&fp, 0, sizeof(fp));
-    fp.in = pl.in; fp.in_frame_stride = px; fp.in_rows = h; fp.width = w; fp.height = h; fp.out_rows = h; fp.n_frames = 1;
-    fp.cls = pl.cls; fp.out_frame_stride = px; fp.blur = pl.p16[0];
+    fp.in = pl.in; fp.in_pitch = w; fp.in_frame_stride = px; fp.in_rows = h; fp.width = w; fp.height = h; fp.out_rows = h; fp.n_frames = 1;
+    fp.cls = pl.cls; fp.cls_pitch = w; fp.cls_frame_stride = px; fp.out_frame_stride = px; fp.blur = pl.p16[0];
     fp.w = ctx->gauss.d_w; fp.count = ctx->gauss.d_count; fp.radius = ctx->gauss.radius;
     fill_thresholds(fp, 1 << 20, 1 << 20);  // nothing is a candidate: the later phases do the minimum
     CB_TRY(launch_front(ctx, st, fp));
@@ -670,7 +692,7 @@ int b200_hysteresis(b200_ctx* ctx, int16_t* nms_inout, int h, int w, int lo, int
     CB_TRY(launch_classify_i16(ctx, st, pl.p16[0], pl.cls, (size_t)px, lo, effective_hi(hi)));
     HystParams hp;
     memset(&hp, 0, sizeof(hp));
-    hp.cls = pl.cls; hp.parent = reinterpret_cast<int32_t*>(ctx->ws_parent[0].ptr);
+    hp.cls = pl.cls; hp.cls_pitch = w; hp.cls_frame_stride = px; hp.parent = reinterpret_cast<int32_t*>(ctx->ws_parent[0].ptr);
     hp.frame_stride = px; hp.rows = h; hp.width = w; hp.row0 = 0; hp.n_frames = 1;
     CB_TRY(launch_hysteresis(ctx, st, hp));
     CB_TRY(launch_expand_u8_to_i16(ctx, st, pl.cls, pl.p16[1], (size_t)px));
@@ -752,7 +774,7 @@ int b200_canny_bgr(b200_ctx* ctx, const uint8_t* bgr, float sigma, int lo, int h
         h_src = reinterpret_cast<const uint8_t*>(ctx->host_in[0].ptr);
     }
     CB_CUDA(cudaMemcpyAsync(d_bgr, h_src, (size_t)px * 3, cudaMemcpyHostToDevice, st));
-    if (!gray_out && bgr_fused_ok(ctx, d_bgr, h, w)) {
+    if (!gray_out && bgr_fused_ok(ctx, d_bgr, 1, h, w, 3LL * w, 3 * px)) {
         // nobody wants the gray plane: the front kernel converts while it stages (no 4 B/px pass, no gray plane in HBM)
         CB_TRY(run_frames_device(ctx, st, 0, d_bgr, pl.cls, 1, h, w, lo, hi, nullptr, nullptr, nullptr, nullptr, /*bgr=*/true));
     } else {
@@ -785,15 +807,47 @@ int b200_canny_bgr(b200_ctx* ctx, const uint8_t* bgr, float sigma, int lo, int h
 }
 
 // ---- batched --------------------------------------------------------------------------------------------
+// Argument checks of a strided device batch; all of them run before any device work.  bpp: bytes per input pixel.
+static int check_strided(const uint8_t* in, long long in_pitch, long long in_fs, int n, int h, int w, const uint8_t* out,
+                         long long out_pitch, long long out_fs, int bpp) {
+    CB_TRY(check_image(in, out, h, w));
+    if (n <= 0) { set_error("n_frames must be positive"); return B200_ERR_INVALID_ARG; }
+    if (in_pitch < 0 || in_fs < 0 || out_pitch < 0 || out_fs < 0) {
+        set_error("negative stride (in: pitch %lld, frame %lld; out: pitch %lld, frame %lld)", in_pitch, in_fs, out_pitch, out_fs);
+        return B200_ERR_INVALID_ARG;
+    }
+    const long long in_row = (long long)bpp * w;
+    if (in_pitch < in_row) { set_error("input row pitch %lld is smaller than a row (%lld bytes)", in_pitch, in_row); return B200_ERR_INVALID_ARG; }
+    if (out_pitch < w) { set_error("output row pitch %lld is smaller than a row (%d bytes)", out_pitch, w); return B200_ERR_INVALID_ARG; }
+    // extents in 128-bit arithmetic: no stride, however large, can wrap a product and slip past the checks below
+    typedef __int128 i128;
+    const i128 in_frame = (i128)(h - 1) * in_pitch + in_row, out_frame = (i128)(h - 1) * out_pitch + w;
+    if (n > 1 && in_fs < in_frame) { set_error("input frames overlap: frame stride %lld < %.0f bytes per frame", in_fs, (double)in_frame); return B200_ERR_INVALID_ARG; }
+    if (n > 1 && out_fs < out_frame) { set_error("output frames overlap: frame stride %lld < %.0f bytes per frame", out_fs, (double)out_frame); return B200_ERR_INVALID_ARG; }
+    // the extents: first byte of frame 0 to one past the last byte of frame n-1
+    const i128 in_ext = (i128)(n - 1) * in_fs + in_frame, out_ext = (i128)(n - 1) * out_fs + out_frame;
+    const i128 kMaxExtent = (i128)1 << 48;   // more than any device address space
+    if (in_ext > kMaxExtent || out_ext > kMaxExtent) {
+        set_error("strides span more than 2^48 bytes (input %.3g, output %.3g bytes)", (double)in_ext, (double)out_ext);
+        return B200_ERR_INVALID_ARG;
+    }
+    const i128 in_lo = (i128)reinterpret_cast<uintptr_t>(in), out_lo = (i128)reinterpret_cast<uintptr_t>(out);
+    if (in_lo < out_lo + out_ext && out_lo < in_lo + in_ext) { set_error("the output's extent overlaps the input's"); return B200_ERR_INVALID_ARG; }
+    return B200_OK;
+}
+
 // bpp: bytes per input pixel — 1 gray, 3 interleaved B,G,R (converted by the front kernel while staging when it can, else chunk by
-// chunk into a gray scratch plane first)
-static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, int n_frames, int h, int w, float sigma, int lo, int hi,
-                             uint8_t* d_edges, int bpp) {
-    CB_TRY(check_image(d_frames, d_edges, h, w));
+// chunk into a gray scratch plane first).  Strides in bytes (b200_canny_batch_device_strided); the dense entry points pass
+// pitch = bpp*width and frame stride = height*pitch.
+static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, long long in_pitch, long long in_fs, int n_frames, int h, int w,
+                             float sigma, int lo, int hi, uint8_t* d_edges, long long out_pitch, long long out_fs, int bpp) {
+    CB_TRY(check_strided(d_frames, in_pitch, in_fs, n_frames, h, w, d_edges, out_pitch, out_fs, bpp));
     CB_TRY(check_thresholds(lo, hi));
-    if (n_frames <= 0) { set_error("n_frames must be positive"); return B200_ERR_INVALID_ARG; }
     CB_TRY(resolve_ctx(ctx));
     CB_TRY(prepare_gauss(ctx, sigma));
+    // a single frame's stride is never used: make it the one that keeps the tensor map and the word stores eligible
+    if (n_frames == 1) { in_fs = (long long)h * in_pitch; out_fs = (long long)h * out_pitch; }
+    const FrameLayout lay = {in_pitch, in_fs, out_pitch, out_fs};
     const long long px = (long long)h * w;
     const int chunk = auto_chunk_frames(ctx, h, w, n_frames);
     const int n_chunks = (n_frames + chunk - 1) / chunk;
@@ -803,18 +857,23 @@ static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, int n_frame
     // high-priority streams on top of that measured 222)
     const int n_slots = std::min(3, n_chunks);
     const bool bgr = bpp == 3;
-    const bool fused = bgr && bgr_fused_ok(ctx, d_frames, h, w);
+    const bool fused = bgr && bgr_fused_ok(ctx, d_frames, std::min(chunk, n_frames), h, w, in_pitch, in_fs);
+    const bool bgr_dense = in_pitch == 3LL * w && in_fs == 3 * px;
     for (int s = 0; s < n_slots; ++s) {
         CB_TRY(ensure_ws(ctx->ws_parent[s], (size_t)px * 4 * (size_t)chunk));
         CB_TRY(ensure_ws(ctx->ws_list[s], list_bytes(chunk, h, w)));
         if (bgr && !fused) CB_TRY(ensure_ws(ctx->dev_in[s], (size_t)px * (size_t)chunk));   // gray scratch of one chunk
     }
     auto run_chunk = [&](cudaStream_t st, int s, int f0, int nf) -> int {
-        const uint8_t* src = d_frames + (long long)f0 * px * bpp;
+        const uint8_t* src = d_frames + (long long)f0 * in_fs;
+        FrameLayout cl = lay;
         if (bgr && !fused) {
+            // the gray scratch plane is dense whatever the B,G,R frames' strides
             uint8_t* gray = reinterpret_cast<uint8_t*>(ctx->dev_in[s].ptr);
-            CB_TRY(launch_bgr_to_gray(ctx, st, src, gray, (size_t)px * (size_t)nf));
+            if (bgr_dense) CB_TRY(launch_bgr_to_gray(ctx, st, src, gray, (size_t)px * (size_t)nf));
+            else CB_TRY(launch_bgr_to_gray_strided(ctx, st, src, in_pitch, in_fs, nf, h, w, gray));
             src = gray;
+            cl.in_pitch = w; cl.in_frame_stride = px;
         }
         // The last full chunk of a call is cut into four row bands per frame: a front CTA otherwise marches a whole strip of a frame
         // (0.3 ms at 4K) and the call ends with SMs idling while the last of those finish.  Measured on 64-frame calls (one GPU's
@@ -823,7 +882,8 @@ static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, int n_frame
         static const int tail_chunks = [] { const char* e = getenv("B200_CANNY_TAIL_CHUNKS"); return e ? atoi(e) : 1; }();
         int bands = 0;
         if (n_chunks > 1 && f0 + nf > n_frames - tail_chunks * chunk && nf == chunk && tail_bands > 1 && h / tail_bands >= 256) bands = tail_bands;
-        return run_frames_device(ctx, st, s, src, d_edges + (long long)f0 * px, nf, h, w, lo, hi, nullptr, nullptr, nullptr, nullptr, fused, bands);
+        return run_frames_device(ctx, st, s, src, d_edges + (long long)f0 * out_fs, nf, h, w, lo, hi, nullptr, nullptr, nullptr, nullptr,
+                                 fused, bands, &cl);
     };
     if (n_slots == 1) return run_chunk(ctx->stream, 0, 0, n_frames);
     // the side streams take the chunks in turn so one chunk's tail waves overlap the next chunks' heads
@@ -843,12 +903,28 @@ static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, int n_frame
 
 int b200_canny_batch_device(b200_ctx* ctx, const uint8_t* d_frames, int n_frames, int h, int w, float sigma, int lo,
                             int hi, uint8_t* d_edges) {
-    return batch_device_impl(ctx, d_frames, n_frames, h, w, sigma, lo, hi, d_edges, 1);
+    const long long px = (long long)h * w;
+    return batch_device_impl(ctx, d_frames, w, px, n_frames, h, w, sigma, lo, hi, d_edges, w, px, 1);
 }
 
 int b200_canny_batch_device_bgr(b200_ctx* ctx, const uint8_t* d_bgr, int n_frames, int h, int w, float sigma, int lo,
                                 int hi, uint8_t* d_edges) {
-    return batch_device_impl(ctx, d_bgr, n_frames, h, w, sigma, lo, hi, d_edges, 3);
+    const long long px = (long long)h * w;
+    return batch_device_impl(ctx, d_bgr, 3LL * w, 3 * px, n_frames, h, w, sigma, lo, hi, d_edges, w, px, 3);
+}
+
+int b200_canny_batch_device_strided(b200_ctx* ctx, const uint8_t* d_frames, int64_t in_row_pitch, int64_t in_frame_stride,
+                                    int n_frames, int h, int w, float sigma, int lo, int hi, uint8_t* d_edges,
+                                    int64_t out_row_pitch, int64_t out_frame_stride) {
+    return batch_device_impl(ctx, d_frames, in_row_pitch, in_frame_stride, n_frames, h, w, sigma, lo, hi, d_edges, out_row_pitch,
+                             out_frame_stride, 1);
+}
+
+int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int64_t in_row_pitch, int64_t in_frame_stride,
+                                        int n_frames, int h, int w, float sigma, int lo, int hi, uint8_t* d_edges,
+                                        int64_t out_row_pitch, int64_t out_frame_stride) {
+    return batch_device_impl(ctx, d_bgr, in_row_pitch, in_frame_stride, n_frames, h, w, sigma, lo, hi, d_edges, out_row_pitch,
+                             out_frame_stride, 3);
 }
 
 // Host buffers in, host buffers out: frames -> 0 / 255 edge maps, as bytes (edges8) or as the reference's int16 (edges16).

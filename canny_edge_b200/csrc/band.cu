@@ -157,12 +157,13 @@ int band_front_rows(b200_ctx* ctx, cudaStream_t st, const BandGeom& g, int sub_r
     FrontParams fp;
     memset(&fp, 0, sizeof(fp));
     fp.in = g.d_rows;
+    fp.in_pitch = g.width;
     fp.in_frame_stride = (long long)(g.above + g.rows + g.below) * g.width;
     fp.in_row0 = g.row0 - g.above;
     fp.in_rows = g.above + g.rows + g.below;
     fp.width = g.width; fp.height = g.height;
     fp.out_row0 = sub_row0; fp.out_rows = sub_rows; fp.plane_row0 = g.row0; fp.n_frames = 1;
-    fp.cls = g.d_edges; fp.out_frame_stride = px;
+    fp.cls = g.d_edges; fp.cls_pitch = g.width; fp.cls_frame_stride = px; fp.out_frame_stride = px;
     fp.w = ctx->gauss.d_w; fp.count = ctx->gauss.d_count; fp.radius = ctx->gauss.radius;
     fill_thresholds(fp, g.lo, g.hi);
     fp.parent = reinterpret_cast<int32_t*>(ctx->ws_band_parent.ptr);
@@ -192,7 +193,7 @@ int band_label(b200_ctx* ctx, cudaStream_t st, const BandGeom& g) {
     hp.h_kept = ctx->d_kept + 3;
     hp.kept_prev = prev_kept;
     hp.kept_thresh = (unsigned int)(px / 8);
-    hp.cls = g.d_edges; hp.parent = reinterpret_cast<int32_t*>(ctx->ws_band_parent.ptr);
+    hp.cls = g.d_edges; hp.cls_pitch = g.width; hp.cls_frame_stride = px; hp.parent = reinterpret_cast<int32_t*>(ctx->ws_band_parent.ptr);
     hp.frame_stride = px; hp.rows = g.rows; hp.width = g.width; hp.row0 = g.row0; hp.n_frames = 1;
     CB_TRY(launch_ccl_label(ctx, st, hp));
     ctx->list_dirty[3] = false;
@@ -280,7 +281,7 @@ int b200_band_finalize(b200_ctx* ctx, const b200_band_record* d_all, int n_bands
     CB_CUDA(cudaGetLastError());
     HystParams hp;
     memset(&hp, 0, sizeof(hp));
-    hp.cls = d_edges; hp.parent = parent;
+    hp.cls = d_edges; hp.cls_pitch = width; hp.cls_frame_stride = (long long)band_rows * width; hp.parent = parent;
     hp.list = ctx->band_sparse ? reinterpret_cast<const uint32_t*>(ctx->ws_band_list.ptr) + 16 : nullptr;
     hp.ctr = reinterpret_cast<unsigned int*>(ctx->ws_band_list.ptr);   // the resolve kernel reads the retired count, ctr[2]
     hp.frame_stride = (long long)band_rows * width; hp.rows = band_rows; hp.width = width; hp.row0 = ctx->band_row0; hp.n_frames = 1;

@@ -166,7 +166,7 @@ front_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 const int by = y - p.in_row0;
                 unsigned char v = 0;
                 if (y >= 0 && y < H && by >= 0 && by < p.in_rows && x >= 0 && x < W)
-                    v = in_frame[(long long)by * W + x];
+                    v = in_frame[(long long)by * p.in_pitch + x];
                 dst[i] = v;
             }
         }
@@ -419,10 +419,11 @@ front_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                         if (SPILL) { magv[e] = (int16_t)mag; angv[e] = (int16_t)(dir * 45); nmsv[e] = keep ? (int16_t)mag : (int16_t)0; }
                     }
                     const long long o = (long long)frame * p.out_frame_stride + (long long)(y - p.plane_row0) * W + xw;
-                    if (((W & 3) == 0) && xw + 3 < W) {
-                        *reinterpret_cast<uint32_t*>(p.cls + o) = cls_word;
+                    uint8_t* oc = p.cls + (long long)frame * p.cls_frame_stride + (long long)(y - p.plane_row0) * p.cls_pitch + xw;
+                    if (p.cls_words && xw + 3 < W) {
+                        *reinterpret_cast<uint32_t*>(oc) = cls_word;
                     } else {
-                        for (int e = 0; e < 4 && xw + e < W; ++e) p.cls[o + e] = (uint8_t)(cls_word >> (8 * e));
+                        for (int e = 0; e < 4 && xw + e < W; ++e) oc[e] = (uint8_t)(cls_word >> (8 * e));
                     }
                     if (SPILL) {
                         for (int e = 0; e < 4 && xw + e < W; ++e) {
@@ -503,16 +504,16 @@ int choose_bands(const b200_ctx* ctx, int out_rows, int strips, int frames, int 
 }
 
 // Builds the 3-D u8 tensor map {width, rows in the buffer, frames} with a box of box_cols x box_rows x 1.  TMA needs a
-// 16 B aligned base and row pitch; *use_tma is false when the image does not qualify (the kernels then run their
-// generic staging variant — same kernel, byte loads instead of the bulk copy).
+// 16 B aligned base, row pitch and frame stride (input_tma_layout_ok); *use_tma is false when the image does not qualify
+// (the kernels then run their generic staging variant — same kernel, byte loads instead of the bulk copy).  Columns past
+// `width` (a padded pitch) arrive as zeros like those left of the image.
 int make_input_tensor_map(const FrontParams& p, int box_cols, int box_rows, CUtensorMap* tmap, bool* use_tma) {
     static const bool tma_env_off = [] { const char* e = getenv("B200_CANNY_NO_TMA"); return e && e[0] == '1'; }();
     memset(tmap, 0, sizeof(*tmap));
-    *use_tma = !tma_env_off && (p.width % 16 == 0) && ((reinterpret_cast<uintptr_t>(p.in) & 15) == 0) &&
-               (p.in_frame_stride % 16 == 0) && get_encode_fn() != nullptr;
+    *use_tma = !tma_env_off && input_tma_layout_ok(p) && get_encode_fn() != nullptr;
     if (!*use_tma) return B200_OK;
     const cuuint64_t dims[3] = {(cuuint64_t)p.width, (cuuint64_t)p.in_rows, (cuuint64_t)p.n_frames};
-    const cuuint64_t strides[2] = {(cuuint64_t)p.width, (cuuint64_t)p.in_frame_stride};
+    const cuuint64_t strides[2] = {(cuuint64_t)p.in_pitch, (cuuint64_t)input_tma_frame_stride(p)};
     const cuuint32_t box[3] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = get_encode_fn()(tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t*>(p.in), dims, strides, box, estr,
@@ -526,12 +527,12 @@ int make_input_tensor_map(const FrontParams& p, int box_cols, int box_rows, CUte
 }
 
 // Interleaved B,G,R frames as a tensor of 32-bit elements (a box row of a u8 map holds at most 256 bytes; the staged row is 528):
-// 3*width/4 elements per row, out-of-range elements zero-filled like the gray map's.
+// 3*width/4 elements per row (rows in_pitch bytes apart), out-of-range elements zero-filled like the gray map's.
 int make_bgr_tensor_map(const FrontParams& p, int box_words, int box_rows, CUtensorMap* tmap) {
     memset(tmap, 0, sizeof(*tmap));
     if (get_encode_fn() == nullptr) { set_error("cuTensorMapEncodeTiled is not available"); return B200_ERR_UNSUPPORTED; }
     const cuuint64_t dims[3] = {(cuuint64_t)(3 * (long long)p.width / 4), (cuuint64_t)p.in_rows, (cuuint64_t)p.n_frames};
-    const cuuint64_t strides[2] = {(cuuint64_t)(3 * (long long)p.width), (cuuint64_t)p.in_frame_stride};
+    const cuuint64_t strides[2] = {(cuuint64_t)p.in_pitch, (cuuint64_t)input_tma_frame_stride(p)};
     const cuuint32_t box[3] = {(cuuint32_t)box_words, (cuuint32_t)box_rows, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = get_encode_fn()(tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t*>(p.in), dims, strides, box, estr,
@@ -573,6 +574,11 @@ int launch_front(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, bool* 
     FrontParams p = p_in;
     if (sparse_out) *sparse_out = false;
     p.ieee_div = ctx->gauss.tiny ? 1 : 0;
+    if (p.in_pitch < (p.in_bgr ? 3LL : 1LL) * p.width || p.cls_pitch < p.width) {
+        set_error("internal: front launch without input / class-map pitch (%lld, %lld for width %d)", p.in_pitch, p.cls_pitch, p.width);
+        return B200_ERR_INVALID_ARG;
+    }
+    p.cls_words = ((reinterpret_cast<uintptr_t>(p.cls) | (uintptr_t)p.cls_pitch | (uintptr_t)p.cls_frame_stride) & 3) == 0;
     const int radius = p.radius;
     if (radius < 1 || radius > B200_MAX_RADIUS) {
         set_error("gaussian radius %d outside [1,%d]", radius, B200_MAX_RADIUS);

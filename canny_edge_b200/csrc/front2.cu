@@ -186,7 +186,7 @@ front2_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 const int y = gy + r, x = in_x0 + c;
                 const int by = y - p.in_row0;
                 unsigned char v = 0;
-                if (y >= 0 && y < H && by >= 0 && by < p.in_rows && x >= 0 && x < W) v = in_frame[(long long)by * W + x];
+                if (y >= 0 && y < H && by >= 0 && by < p.in_rows && x >= 0 && x < W) v = in_frame[(long long)by * p.in_pitch + x];
                 dst[i] = v;
             }
         }
@@ -417,17 +417,17 @@ front2_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                     *reinterpret_cast<int4*>(s_np + q * kNpPitch + 4 * lane) = nq;
                 }
                 const uint32_t zero_word = 0x01010101u * (uint32_t)p.cls_zero;
-                const bool word_ok = ((W & 3) == 0) && lane < kTW / 4 && (x0 + 4 * lane + 3 < W);  // the aligned 32-bit store applies
+                const bool word_ok = p.cls_words && lane < kTW / 4 && (x0 + 4 * lane + 3 < W);  // the aligned 32-bit store applies
                 const bool tail_ok = !word_ok && lane < kTW / 4 && (x0 + 4 * lane < W);            // ragged right edge: byte stores
                 const unsigned lt_mask = (1u << lane) - 1u;
                 int q = cq_lo + ((warp - cq_lo) & 7);         // first class row of this warp (rows q = warp mod 8)
                 const int32_t* vrow = s_vu + q * kVuPitch + 4 * lane;
                 int32_t* nrow = s_np + q * kNpPitch + 4 * lane;
-                uint8_t* o = p.cls + (long long)frame * p.out_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * W + (x0 + 4 * lane);
+                uint8_t* o = p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * p.cls_pitch + (x0 + 4 * lane);
                 int ent = ((q - 1) << 6) | (lane << 1);
-                const long long o_step = 8LL * W;
+                const long long o_step = 8LL * p.cls_pitch;
                 // two copies of the loop so the store form is decided once, not per row: the aligned 32-bit store (every strip of
-                // an image whose width is a multiple of 4, except a ragged last strip) or byte stores
+                // a class map whose base, pitch and frame stride are multiples of 4, except a ragged last strip) or byte stores
                 auto class_row = [&](const int32_t* vr, int32_t* nr, int e16) {
                     const int4 nq = n_of_row(vr);
                     *reinterpret_cast<int4*>(nr) = nq;
@@ -463,7 +463,7 @@ front2_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
         // ===================== phase 3b: direction, NMS and thresholds for the candidates only =====================
         {
             const long long out_off = (long long)frame * p.out_frame_stride + (long long)(y_base - p.plane_row0) * W + (x0 - 2) + 1;
-            uint8_t* out_base = p.cls + out_off;
+            uint8_t* out_base = p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base - p.plane_row0) * p.cls_pitch + (x0 - 2) + 1;
             int32_t* par_base = p.parent + out_off;                           // only dereferenced when `sparse`
             const int idx_base = (int)out_off;                                // launch-relative pixel index of (class row 0, column j = 1)
             for (int i = lane; i < my_count; i += 32) {
@@ -476,7 +476,7 @@ front2_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 const int32_t* nrow = s_np + (rr + 1) * kNpPitch + c0;     // n[j] lives at word j - 1
                 const int2 n2 = *reinterpret_cast<const int2*>(nrow);
                 const int nc[2] = {n2.x, n2.y};
-                uint8_t* orow = out_base + (long long)rr * W + c0;
+                uint8_t* orow = out_base + (long long)rr * p.cls_pitch + c0;
                 // branch-free up to the local-maximum test so the two pixels' chains overlap
                 int na[2], nb[2];
                 bool pass[2];

@@ -121,7 +121,11 @@ __device__ __forceinline__ void red_or_shared_if(bool on, uint32_t* ptr, uint32_
 // register file free, so blocks of the small latency-bound hysteresis kernels of the PREVIOUS chunk (other stream) become
 // resident next to them instead of waiting for a front CTA to retire: the front kernel alone gets 1.7 % slower, the chunk
 // pipeline 2.3 % faster on the bench frames and 8 % faster on photographic content (112 / 104 / 88 / 80 measured too: 96 wins).
-template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false>
+// PITCHED: the input or the class map has a row pitch / frame stride of its own, or the map is not word-aligned
+// (b200_canny_batch_device_strided; layout_pitched()).  Dense layouts (the batch and host paths) keep the dense addressing, whose
+// class and union-find offsets are one and the same, so their instruction stream and register allocation are those of the
+// dense-only kernel.
+template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false, bool PITCHED = false>
 #ifndef F3_MAXREG
 #define F3_MAXREG 96
 #endif
@@ -225,7 +229,7 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 const int y = gy + r, x = in_x0 + c;
                 const int by = y - p.in_row0;
                 unsigned char v = 0;
-                if (y >= 0 && y < H && by >= 0 && by < p.in_rows && x >= 0 && x < W) v = in_frame[(long long)by * W + x];
+                if (y >= 0 && y < H && by >= 0 && by < p.in_rows && x >= 0 && x < W) v = in_frame[(long long)by * (PITCHED ? p.in_pitch : (long long)W) + x];
                 dst[i] = v;
             }
         }
@@ -543,17 +547,20 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                     *reinterpret_cast<float4*>(s_np + q * kNpPitch + 4 * lane) = nq;
                 }
                 const uint32_t zero_word = 0x01010101u * (uint32_t)p.cls_zero;
-                const bool word_ok = ((W & 3) == 0) && lane < kTW / 4 && (x0 + 4 * lane + 3 < W);  // the aligned 32-bit store applies
+                // dense layouts: base aligned (layout_pitched), so word stores need a width that is a multiple of 4
+                const bool words = PITCHED ? p.cls_words != 0 : ((W & 3) == 0);
+                const bool word_ok = words && lane < kTW / 4 && (x0 + 4 * lane + 3 < W);  // the aligned 32-bit store applies
                 const bool tail_ok = !word_ok && lane < kTW / 4 && (x0 + 4 * lane < W);            // ragged right edge: byte stores
                 const unsigned lt_mask = (1u << lane) - 1u;
                 int q = cq_lo + ((warp - cq_lo) & 7);         // first class row of this warp (rows q = warp mod 8)
                 const int32_t* vrow = s_vu + q * kVuPitch + 4 * lane;
                 float* nrow = s_np + q * kNpPitch + 4 * lane;
-                uint8_t* o = p.cls + (long long)frame * p.out_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * W + (x0 + 4 * lane);
+                uint8_t* o = PITCHED ? p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * p.cls_pitch + (x0 + 4 * lane)
+                                     : p.cls + (long long)frame * p.out_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * W + (x0 + 4 * lane);
                 int ent = ((q - 1) << 6) | (lane << 1);
-                const long long o_step = 8LL * W;
+                const long long o_step = 8LL * (PITCHED ? p.cls_pitch : (long long)W);
                 // two copies of the loop so the store form is decided once, not per row: the aligned 32-bit store (every strip of
-                // an image whose width is a multiple of 4, except a ragged last strip) or byte stores
+                // a class map whose base, pitch and frame stride are multiples of 4, except a ragged last strip) or byte stores
                 auto class_row_nq = [&](const float4 nq, float* nr, int e16) {
                     *reinterpret_cast<float4*>(nr) = nq;
                     // one entry per PAIR of pixels (columns 4*lane+1.. +2 and 4*lane+3.. +4) that holds a candidate: candidates
@@ -567,8 +574,8 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 };
                 auto class_row = [&](const int32_t* vr, float* nr, int e16) { class_row_nq(n_of_row(vr), nr, e16); };
                 // every class word starts out as "suppressed"; phase 3b overwrites the bytes of surviving pixels
-                if (cq_lo == 1 && cq_hi == kSlab && ((W & 3) == 0)) {
-                    // the common slab (all 64 class rows, image width a multiple of 4): the warp's eight rows unrolled, every address an
+                if (cq_lo == 1 && cq_hi == kSlab && words) {
+                    // the common slab (all 64 class rows, word-aligned class map): the warp's eight rows unrolled, every address an
                     // immediate offset from the first row's (word_ok is false for the columns past a ragged right edge)
                     // The next row's Sobel words are fetched before this row's stores: the compiler cannot move a shared-memory load
                     // above the n-plane / list stores of the row before (it cannot prove they do not alias), and every row would
@@ -611,8 +618,10 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
         // dependent chains (entry -> Sobel words -> direction -> neighbours -> truncated-magnitude test) overlap: with 16 warps
         // per SM this phase is bound by those chains, not by issue slots.
         {
+            // PITCHED: the class byte is addressed through the caller's pitches; the union-find slot and the list index stay dense
             const long long out_off = (long long)frame * p.out_frame_stride + (long long)(y_base - p.plane_row0) * W + (x0 - 2) + 1;
-            uint8_t* out_base = p.cls + out_off;
+            uint8_t* out_base = PITCHED ? p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base - p.plane_row0) * p.cls_pitch + (x0 - 2) + 1
+                                        : p.cls + out_off;
             int32_t* par_base = p.parent + out_off;                           // only dereferenced when `sparse`
             const int idx_base = (int)out_off;                                // launch-relative pixel index of (class row 0, column j = 1)
             for (int i = lane; i < my_count; i += 64) {
@@ -631,7 +640,7 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 for (int u = 0; u < 2; ++u) {
                     const int rr = ent[u] >> 6, c0 = 2 * (ent[u] & 63);        // pixels j = c0 + 1 and c0 + 2 of class row rr
                     rel[u] = rr * W + c0;                                      // < 2^31: rr < 64, W < 2^24
-                    orow[u] = out_base + (unsigned)rel[u];
+                    orow[u] = PITCHED ? out_base + ((long long)rr * p.cls_pitch + c0) : out_base + (unsigned)rel[u];
                     prow[u] = par_base + (unsigned)rel[u];
                     const int32_t* vrow = s_vu + (rr + 1) * kVuPitch + c0;     // VU words j-1 .. j+2 = c0 .. c0+3
                     const uint2 qa = *reinterpret_cast<const uint2*>(vrow);
@@ -743,26 +752,36 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false>
+template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false, bool PITCHED = false>
 static int launch_one3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CUtensorMap& tmap, dim3 grid) {
     const f3::SmemLayout L = f3::smem_layout(R, SLAB, BGR);
     static bool configured[64] = {false};  // per instantiation, per device
     if (!configured[ctx->device & 63]) {
-        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
+        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
         configured[ctx->device & 63] = true;
     }
     {
         ProfScope ps(ctx, st, 0);
-        f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR><<<grid, f3::kThreads, L.total, st>>>(p, tmap);
+        f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED><<<grid, f3::kThreads, L.total, st>>>(p, tmap);
     }
     CB_CUDA(cudaGetLastError());
     ctx->launches++;
     return B200_OK;
 }
 
+// whether the kernel needs the pitched addressing: an input whose rows are not `width` bytes (3*width for B,G,R) apart, a class map
+// whose rows are not `width` bytes apart or whose frames are not out_frame_stride bytes apart, or a class map off a 4-byte boundary
+static bool layout_pitched(const FrontParams& p) {
+    return p.in_pitch != (p.in_bgr ? 3LL : 1LL) * p.width || p.cls_pitch != p.width || p.cls_frame_stride != p.out_frame_stride ||
+           (reinterpret_cast<uintptr_t>(p.cls) & 3) != 0;
+}
+
 template <int R, int SLAB>
 static int launch_r3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CUtensorMap& tmap, dim3 grid, bool use_tma, int div) {
+    // layouts with pitches of their own: one instantiation per staging form, the always-valid division
+    if (layout_pitched(p)) return use_tma ? launch_one3<R, true, 5, SLAB, false, true>(ctx, st, p, tmap, grid)
+                                       : launch_one3<R, false, 5, SLAB, false, true>(ctx, st, p, tmap, grid);
     if (use_tma) {
         if (div == 1) return launch_one3<R, true, 1, SLAB>(ctx, st, p, tmap, grid);
         if (div == 3) return launch_one3<R, true, 3, SLAB>(ctx, st, p, tmap, grid);
@@ -775,13 +794,15 @@ static int launch_r3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const
 // interleaved B,G,R input: TMA only, the three exact divisions
 template <int R, int SLAB>
 static int launch_r3_bgr(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CUtensorMap& tmap, dim3 grid, int div) {
+    if (layout_pitched(p)) return launch_one3<R, true, 5, SLAB, true, true>(ctx, st, p, tmap, grid);
     if (div == 1) return launch_one3<R, true, 1, SLAB, true>(ctx, st, p, tmap, grid);
     if (div == 3) return launch_one3<R, true, 3, SLAB, true>(ctx, st, p, tmap, grid);
     return launch_one3<R, true, 5, SLAB, true>(ctx, st, p, tmap, grid);
 }
 
 // The fused-conversion variant exists for half-windows up to 9 (one staged input buffer is what larger ones use anyway) and needs
-// the TMA path: rows of 3W bytes on 16 B boundaries.
+// the TMA path: a width that is a multiple of 16 (whole 32-bit elements per staged row), base, row pitch and frame stride on 16 B
+// boundaries.
 bool front3_bgr_supports(const FrontParams& p) {
     static const bool tma_env_off = [] { const char* e = getenv("B200_CANNY_NO_TMA"); return e && e[0] == '1'; }();
     static const bool fuse_off = [] { const char* e = getenv("B200_CANNY_BGR_FUSED"); return e && e[0] == '0'; }();
@@ -789,7 +810,7 @@ bool front3_bgr_supports(const FrontParams& p) {
         case 2: case 3: case 5: case 6: case 9: break;
         default: return false;
     }
-    return !tma_env_off && !fuse_off && (p.width % 16 == 0) && ((reinterpret_cast<uintptr_t>(p.in) & 15) == 0) && (p.in_frame_stride % 16 == 0);
+    return !tma_env_off && !fuse_off && (p.width % 16 == 0) && input_tma_layout_ok(p);
 }
 
 bool front3_supports(int radius) {
@@ -839,7 +860,7 @@ int launch_front3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in) {
     const int div3 = ctx->gauss.div_mode;
     p.div_c = ctx->gauss.div_c;
     if (p.in_bgr) {
-        if (!front3_bgr_supports(p)) { set_error("fused BGR input needs width %% 16 == 0, 16-byte aligned frames and a half-window <= 9"); return B200_ERR_UNSUPPORTED; }
+        if (!front3_bgr_supports(p)) { set_error("fused BGR input needs width %% 16 == 0, a 16-byte aligned base, row pitch and frame stride and a half-window <= 9"); return B200_ERR_UNSUPPORTED; }
         CB_TRY(make_bgr_tensor_map(p, 3 * f3::in_pitch_for(radius) / 4, slab, &tmap));
         switch (radius) {
             case 2: return launch_r3_bgr<2, 64>(ctx, st, p, tmap, grid, div3);

@@ -45,15 +45,16 @@ ccl_local_kernel(const HystParams p) {
     const int tid = threadIdx.x;
     const int x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile;
     const int frame = blockIdx.z;
-    const uint8_t* cls = p.cls + (long long)frame * p.frame_stride;
+    const uint8_t* cls = p.cls + (long long)frame * p.cls_frame_stride;
     int32_t* parent = p.parent + (long long)frame * p.frame_stride;
     const int W = p.width, Hh = p.rows;
+    const long long cp = p.cls_pitch;
 
     if (tid == 0) s_any = 0;
     __syncthreads();
 
     // ---- load the tile (16 B per thread-iteration when aligned), remember whether it has any candidate ----
-    const bool vec_ok = ((W & 15) == 0) && ((reinterpret_cast<uintptr_t>(cls) & 15) == 0);
+    const bool vec_ok = ((cp & 15) == 0) && ((reinterpret_cast<uintptr_t>(cls) & 15) == 0);
     int any = 0;
     for (int i = tid; i < kTile * (kTile / 16); i += kCclThreads) {
         const int r = i >> 2, q = i & 3;
@@ -61,10 +62,10 @@ ccl_local_kernel(const HystParams p) {
         uint4 v = make_uint4(0, 0, 0, 0);
         if (y < Hh) {
             if (vec_ok && x + 15 < W) {
-                v = __ldg(reinterpret_cast<const uint4*>(cls + (long long)y * W + x));
+                v = __ldg(reinterpret_cast<const uint4*>(cls + (long long)y * cp + x));
             } else {
                 unsigned char tmp[16];
-                for (int e = 0; e < 16; ++e) tmp[e] = (x + e < W) ? cls[(long long)y * W + x + e] : 0;
+                for (int e = 0; e < 16; ++e) tmp[e] = (x + e < W) ? cls[(long long)y * cp + x + e] : 0;
                 v = *reinterpret_cast<uint4*>(tmp);
             }
         }
@@ -160,36 +161,40 @@ ccl_merge_kernel(const HystParams p) {
     const int n_hb = p.tiles_y - 1, n_vb = p.tiles_x - 1;
     const long long n_h = (long long)n_hb * W, n_v = (long long)n_vb * Hh;
     const int frame = blockIdx.y;
-    const uint8_t* cls = p.cls + (long long)frame * p.frame_stride;
+    const uint8_t* cls = p.cls + (long long)frame * p.cls_frame_stride;
     int32_t* parent = p.parent + (long long)frame * p.frame_stride;
+    const long long cp = p.cls_pitch;
+    // a: dense index of the pixel (union-find slots), ca: its class byte
     for (long long it = (long long)blockIdx.x * blockDim.x + threadIdx.x; it < n_h + n_v;
          it += (long long)gridDim.x * blockDim.x) {
         if (it < n_h) {
             const int b = (int)(it / W), x = (int)(it - (long long)b * W);
             const int y = (b + 1) * kTile - 1;  // upper row of the boundary; y+1 < Hh because the tile below exists
             const int a = y * W + x;
-            if (cls[a] == 0) continue;
+            const long long ca = y * cp + x;
+            if (cls[ca] == 0) continue;
             const int below = a + W;
             // (0,1)-(1,0), the one pair that must not be joined, never straddles a tile boundary (kTile > 1).
-            if (cls[below] != 0) {
+            if (cls[ca + cp] != 0) {
                 // the two diagonals sit next to `below` in row y+1, so they reach `a` through it
                 g_union(parent, a, below);
             } else {
-                if (x > 0 && cls[below - 1] != 0) g_union(parent, a, below - 1);
-                if (x < W - 1 && cls[below + 1] != 0) g_union(parent, a, below + 1);
+                if (x > 0 && cls[ca + cp - 1] != 0) g_union(parent, a, below - 1);
+                if (x < W - 1 && cls[ca + cp + 1] != 0) g_union(parent, a, below + 1);
             }
         } else {
             const long long j = it - n_h;
             const int b = (int)(j / Hh), y = (int)(j - (long long)b * Hh);
             const int x = (b + 1) * kTile - 1;  // left column of the boundary; x+1 < W because the tile to the right exists
             const int a = y * W + x;
-            if (cls[a] == 0) continue;
+            const long long ca = y * cp + x;
+            if (cls[ca] == 0) continue;
             const int right = a + 1;
-            if (cls[right] != 0) {
+            if (cls[ca + 1] != 0) {
                 g_union(parent, a, right);  // (y-1,x+1) and (y+1,x+1) are vertical neighbours of `right`
             } else {
-                if (y > 0 && cls[right - W] != 0) g_union(parent, a, right - W);
-                if (y < Hh - 1 && cls[right + W] != 0) g_union(parent, a, right + W);
+                if (y > 0 && cls[ca + 1 - cp] != 0) g_union(parent, a, right - W);
+                if (y < Hh - 1 && cls[ca + 1 + cp] != 0) g_union(parent, a, right + W);
             }
         }
     }
@@ -203,13 +208,14 @@ ccl_final_kernel(const HystParams p) {
     __shared__ int s_qroot;
     const int W = p.width, Hh = p.rows;
     const int frame = blockIdx.y;
-    uint8_t* cls = p.cls + (long long)frame * p.frame_stride;
+    uint8_t* cls = p.cls + (long long)frame * p.cls_frame_stride;
     const int32_t* parent = p.parent + (long long)frame * p.frame_stride;
+    const long long cp = p.cls_pitch;
 
     // the one-way link (0,1) -> (1,0) of the global image (see file header)
     if (threadIdx.x == 0) {
         int q = kNone;
-        if (p.row0 == 0 && Hh >= 2 && W >= 2 && cls[1] != 0 && cls[W] != 0) {
+        if (p.row0 == 0 && Hh >= 2 && W >= 2 && cls[1] != 0 && cls[cp] != 0) {
             if (g_find(parent, 1) == kSuper) q = g_find(parent, W);
         }
         s_qroot = q;
@@ -218,6 +224,20 @@ ccl_final_kernel(const HystParams p) {
     const int qroot = s_qroot;
 
     const long long n = (long long)Hh * W;
+    if (cp != W) {
+        // class map rows with a pitch of their own: blocks take rows, threads columns; only the rows' own bytes are read and written
+        for (int y = blockIdx.x; y < Hh; y += gridDim.x) {
+            uint8_t* row = cls + y * cp;
+            for (int x = threadIdx.x; x < W; x += blockDim.x) {
+                if (row[x] == 1) {
+                    const int root = g_find(parent, y * W + x);
+                    row[x] = (root == kSuper || root == qroot) ? 255 : 0;
+                }
+            }
+        }
+        return;
+    }
+    // dense rows: the frame is one flat run of bytes, walked 16 at a time (whole vectors are written back)
     const bool vec_ok = ((n & 15) == 0) && ((reinterpret_cast<uintptr_t>(cls) & 15) == 0);
     if (vec_ok) {
         const long long n16 = n >> 4;
@@ -269,6 +289,16 @@ ccl_final_kernel(const HystParams p) {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
+// The list holds DENSE launch-relative indices g = f*frame_stride + y*width + x (the union-find slots); the class byte of that
+// pixel is at f*cls_frame_stride + y*cls_pitch + x, which is g itself when the map is dense.
+__device__ __forceinline__ long long cls_index(const HystParams& p, unsigned int g) {
+    if (p.cls_pitch == p.width && p.cls_frame_stride == p.frame_stride) return g;
+    const unsigned int fs = (unsigned int)p.frame_stride;
+    const unsigned int f = g / fs, rel = g - f * fs;
+    const unsigned int y = rel / (unsigned int)p.width, x = rel - y * (unsigned int)p.width;
+    return (long long)f * p.cls_frame_stride + (long long)y * p.cls_pitch + x;
+}
+
 __global__ void __launch_bounds__(256)
 ccl_sparse_link_kernel(const HystParams p) {
     pdl_launch_dependents();
@@ -278,23 +308,24 @@ ccl_sparse_link_kernel(const HystParams p) {
     const uint32_t* const walk = p.list;
     const int W = p.width, Hh = p.rows;
     const unsigned int fs = (unsigned int)p.frame_stride;
+    const long long cp = p.cls_pitch;
     for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const unsigned int g = walk[i];
-        const unsigned int rel = g % fs;
+        const unsigned int f = g / fs, rel = g - f * fs;
         const int y = (int)(rel / (unsigned int)W), x = (int)(rel - (unsigned int)y * (unsigned int)W);
-        const uint8_t* c = p.cls + g;
+        const uint8_t* c = p.cls + ((long long)f * p.cls_frame_stride + y * cp + x);
         const bool has_n = y > 0, has_s = y + 1 < Hh, has_w = x > 0, has_e = x + 1 < W;
         const bool top_rows = (p.row0 + y) <= 1;
         const bool q01 = top_rows && (p.row0 + y == 0) && (x == 1);   // this pixel is (0,1): its SW neighbour (1,0) is off limits
         const bool q10 = top_rows && (p.row0 + y == 1) && (x == 0);   // this pixel is (1,0): its NE neighbour (0,1) is off limits
-        const int c_nw = (has_n && has_w) ? c[-W - 1] : 0;
-        const int c_n = has_n ? c[-W] : 0;
-        const int c_ne = (has_n && has_e && !q10) ? c[-W + 1] : 0;
+        const int c_nw = (has_n && has_w) ? c[-cp - 1] : 0;
+        const int c_n = has_n ? c[-cp] : 0;
+        const int c_ne = (has_n && has_e && !q10) ? c[-cp + 1] : 0;
         const int c_w = has_w ? c[-1] : 0;
         const int c_e = has_e ? c[1] : 0;
-        const int c_sw = (has_s && has_w && !q01) ? c[W - 1] : 0;
-        const int c_s = has_s ? c[W] : 0;
-        const int c_se = (has_s && has_e) ? c[W + 1] : 0;
+        const int c_sw = (has_s && has_w && !q01) ? c[cp - 1] : 0;
+        const int c_s = has_s ? c[cp] : 0;
+        const int c_se = (has_s && has_e) ? c[cp + 1] : 0;
         // classes are 0, 1 or 255: a strong neighbour anywhere around makes the component strong
         if (((c_nw | c_n | c_ne | c_w | c_e | c_sw | c_s | c_se) & 0x80) != 0) g_union_halve(p.parent, (int)g, kSuper);
         if (c_e == 1) g_union_halve(p.parent, (int)g, (int)g + 1);
@@ -320,7 +351,8 @@ ccl_sparse_link_kernel(const HystParams p) {
     if (p.row0 == 0 && Hh >= 2 && W >= 2) {
         for (int f = threadIdx.x; f < p.n_frames; f += blockDim.x) {
             const unsigned int f0 = (unsigned int)f * fs;
-            const int c01 = p.cls[f0 + 1], c10 = p.cls[f0 + W];
+            const uint8_t* cf = p.cls + (long long)f * p.cls_frame_stride;
+            const int c01 = cf[1], c10 = cf[cp];
             if (c10 == 1 && (c01 == 255 || (c01 == 1 && g_find_halve(p.parent, (int)f0 + 1) == kSuper)))
                 g_union_halve(p.parent, (int)f0 + W, kSuper);
         }
@@ -350,7 +382,7 @@ ccl_sparse_resolve_kernel(const HystParams p) {
     const unsigned int n = p.ctr[2];
     for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const unsigned int g = p.list[i];
-        p.cls[g] = (g_find_halve(p.parent, (int)g) == kSuper) ? 255 : 0;
+        p.cls[cls_index(p, g)] = (g_find_halve(p.parent, (int)g) == kSuper) ? 255 : 0;
     }
 }
 
@@ -380,8 +412,17 @@ static cudaError_t launch_list_kernel(void (*kernel)(const HystParams), int grid
     return cudaLaunchKernelEx(&cfg, kernel, p);
 }
 
+static int check_hyst_params(const HystParams& p) {
+    if (p.cls_pitch < p.width || p.cls_frame_stride < 0) {
+        set_error("internal: hysteresis launch without a class-map pitch (%lld for width %d)", p.cls_pitch, p.width);
+        return B200_ERR_INVALID_ARG;
+    }
+    return B200_OK;
+}
+
 int launch_ccl_label(b200_ctx* ctx, cudaStream_t st, const HystParams& p_in) {
     HystParams p = p_in;
+    CB_TRY(check_hyst_params(p));
     if (p.list) {
         ProfScope ps(ctx, st, 1);
         CB_CUDA(launch_list_kernel(ccl_sparse_link_kernel, sparse_grid(ctx, p), st, p));
@@ -419,6 +460,7 @@ int launch_ccl_label(b200_ctx* ctx, cudaStream_t st, const HystParams& p_in) {
 
 int launch_ccl_resolve(b200_ctx* ctx, cudaStream_t st, const HystParams& p_in) {
     HystParams p = p_in;
+    CB_TRY(check_hyst_params(p));
     if (p.list) {
         ProfScope ps(ctx, st, 3);
         CB_CUDA(launch_list_kernel(ccl_sparse_resolve_kernel, sparse_grid(ctx, p), st, p));

@@ -51,11 +51,12 @@ struct GaussTables {
 struct FrontParams {
     const uint8_t* in;      // first byte of buffer row 0 of frame 0
     long long in_frame_stride;  // bytes between frames in `in`
-    int in_bgr;             // 1: `in` holds interleaved B,G,R bytes (3 per pixel, rows of 3*width bytes, in_frame_stride in BYTES):
+    long long in_pitch;     // bytes between rows of `in` (>= width, >= 3*width for BGR)
+    int in_bgr;             // 1: `in` holds interleaved B,G,R bytes (3 per pixel, in_pitch >= 3*width bytes per row):
                             // front3's fused-conversion variant (front3_bgr_supports); 0: one gray byte per pixel
     int in_row0;            // global row index of buffer row 0 (0 for whole frames; row0-halo for bands)
     int in_rows;            // rows present in the buffer
-    int width;              // image width == pitch of every plane
+    int width;              // image width == pitch of every internal plane (parent, list indices, spill planes)
     int height;             // GLOBAL image height (border rules key off this)
     int out_row0;           // first global row this launch produces
     int out_rows;           // number of rows produced
@@ -63,8 +64,13 @@ struct FrontParams {
                             // produces only part of the plane's rows (row bands: interior rows first, the rows that need the
                             // neighbours' halo once it has arrived; bands_mgpu.cu)
     int n_frames;
-    uint8_t* cls;           // out: class map (0 / 1 weak / 255 strong), out_rows*width per frame
-    long long out_frame_stride;  // elements between frames in every output plane
+    uint8_t* cls;           // out: class map (0 / 1 weak / 255 strong) in the caller's layout: pixel (f, y, x) at
+                            // f*cls_frame_stride + (y - plane_row0)*cls_pitch + x; no other byte of it is written
+    long long cls_pitch;         // bytes between rows of cls
+    long long cls_frame_stride;  // bytes between frames of cls
+    int cls_words;               // 1: base, pitch and frame stride of cls are multiples of 4, so four pixels at a column that is a
+                                 // multiple of 4 are one aligned 32-bit store (set by launch_front from the three; else byte stores)
+    long long out_frame_stride;  // elements between frames in the dense internal planes (parent, list indices, spill planes)
     int16_t* blur;          // optional spill planes (steps / stage API); may be null
     int16_t* mag;
     int16_t* ang;
@@ -79,11 +85,21 @@ struct FrontParams {
     int ieee_div;           // 1: weights so small that sums can fall below 2^-100 -> use IEEE division instead of div_exact
     int tiles_x, tiles_y;
     // sparse hand-over to the hysteresis kernels (front2.cu only; both null -> not produced):
-    int32_t* parent;        // union-find slots, indexed like cls: every WEAK pixel is initialised to its own launch-relative index
-                            // frame*out_frame_stride + pixel (strong pixels need no slot: they are final)
+    int32_t* parent;        // union-find slots, dense: every WEAK pixel is initialised to its own launch-relative index
+                            // frame*out_frame_stride + (y - plane_row0)*width + x (strong pixels need no slot: they are final)
     uint32_t* kept_list;    // launch-relative indices of all weak pixels, in no particular order
     unsigned int* kept_count;  // number of entries: word 0 of the list's counter block (see HystParams::ctr); zero at launch
 };
+
+// The input layout a TMA tensor map can describe: base, row pitch and frame stride on 16-byte boundaries, frames that do not
+// overlap (a single frame's stride is never used).  Other layouts take the kernels' byte-load staging.
+inline bool input_tma_layout_ok(const FrontParams& p) {
+    return ((reinterpret_cast<uintptr_t>(p.in) & 15) == 0) && (p.in_pitch % 16 == 0) && (p.in_frame_stride % 16 == 0) &&
+           (p.n_frames <= 1 || p.in_frame_stride >= (long long)p.in_rows * p.in_pitch);
+}
+inline long long input_tma_frame_stride(const FrontParams& p) {
+    return p.n_frames <= 1 ? (long long)p.in_rows * p.in_pitch : p.in_frame_stride;
+}
 
 // ---- thresholds ---------------------------------------------------------------------------------
 // The reference accepts any int pair (only its CLI checks 0 <= minVal < maxVal <= 255, src/main.cpp:63-76).  What
@@ -109,9 +125,10 @@ inline void fill_thresholds(FrontParams& p, int lo, int hi) {
 
 // ---- parameters of the hysteresis (connected components) kernels ---------------------------------
 struct HystParams {
-    uint8_t* cls;          // in/out: 0 / 1 / 255 -> 0 / 255   (rows*width per frame)
-    int32_t* parent;       // workspace: union-find parent per pixel (only candidate entries are defined)
-    long long frame_stride;  // elements between frames (cls and parent)
+    uint8_t* cls;          // in/out: 0 / 1 / 255 -> 0 / 255; pixel (f, y, x) at f*cls_frame_stride + y*cls_pitch + x
+    long long cls_pitch, cls_frame_stride;   // bytes between rows / frames of cls
+    int32_t* parent;       // workspace: union-find parent per pixel (only candidate entries are defined), dense
+    long long frame_stride;  // elements between frames of parent (and of the list's pixel indices: f*frame_stride + y*width + x)
     int rows, width;       // rows in this launch's plane (whole frame or band)
     int row0;              // global row of plane row 0 (the missing-link quirk lives at global (1,0)->(0,1))
     int n_frames;
@@ -160,6 +177,7 @@ struct b200_ctx {
     cudaStream_t stream = nullptr;       // stream work is issued on (own_stream or the user's)
     cudaStream_t side[3] = {nullptr, nullptr, nullptr};  // chunk pipelining / copy overlap
     cudaEvent_t ev_fork = nullptr, ev_join[3] = {nullptr, nullptr, nullptr};
+    cudaEvent_t ev_switch = nullptr;     // b200_ctx_set_stream: the new stream waits for what was issued on the old one
     cb::GaussTables gauss;
     cb::Workspace ws_parent[3];   // int32 union-find slots for one chunk, per pipeline slot
     cb::Workspace ws_list[3];     // kept-pixel lists for one chunk ([0..15] = counter block, entries from word 16), per pipeline slot
@@ -246,6 +264,9 @@ int launch_sobel(b200_ctx* ctx, cudaStream_t st, const int16_t* blur, int h, int
 int launch_nonmaximal(b200_ctx* ctx, cudaStream_t st, const int16_t* mag, const int16_t* ang, int h,
                       int w, int16_t* out);
 int launch_bgr_to_gray(b200_ctx* ctx, cudaStream_t st, const uint8_t* bgr, uint8_t* gray, size_t n_px);
+// n_frames x h rows of w pixels from a pitched B,G,R source into a dense n_frames*h*w gray plane
+int launch_bgr_to_gray_strided(b200_ctx* ctx, cudaStream_t st, const uint8_t* bgr, long long pitch, long long frame_stride,
+                               int n_frames, int h, int w, uint8_t* gray);
 // band.cu: one row band's local stages in pieces
 struct BandGeom {
     const uint8_t* d_rows;   // global row (row0 - above) of the band buffer

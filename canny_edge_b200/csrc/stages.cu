@@ -6,6 +6,8 @@
 // global-memory stencils.
 #include <math.h>
 
+#include <algorithm>
+
 #include "canny_math.h"
 #include "internal.h"
 
@@ -157,6 +159,30 @@ int launch_bgr_to_gray(b200_ctx* ctx, cudaStream_t st, const uint8_t* bgr, uint8
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     bgr_to_gray_kernel<<<(int)blocks, 256, 0, st>>>(bgr, gray, n_px);
+    CB_CUDA(cudaGetLastError());
+    ctx->launches++;
+    return B200_OK;
+}
+
+// The same conversion from pitched frames (row y of frame f at f*frame_stride + y*pitch) into a dense gray plane: what BGR frames
+// the front kernel cannot convert while staging go through.  One block-row per image row; byte loads, so any pitch and offset work.
+__global__ void bgr_to_gray_strided_kernel(const uint8_t* __restrict__ bgr, long long pitch, long long frame_stride, int h, int w,
+                                           long long rows, uint8_t* __restrict__ gray) {
+    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
+        const long long f = r / h, y = r - f * h;
+        const uint8_t* src = bgr + f * frame_stride + y * pitch;
+        uint8_t* dst = gray + r * w;
+        for (int x = threadIdx.x; x < w; x += blockDim.x)
+            dst[x] = (uint8_t)gray_of(__ldcs(src + 3 * x), __ldcs(src + 3 * x + 1), __ldcs(src + 3 * x + 2));
+    }
+}
+
+int launch_bgr_to_gray_strided(b200_ctx* ctx, cudaStream_t st, const uint8_t* bgr, long long pitch, long long frame_stride,
+                               int n_frames, int h, int w, uint8_t* gray) {
+    const long long rows = (long long)n_frames * h;
+    const long long cap = 32LL * (ctx->sm_count > 0 ? ctx->sm_count : 148);
+    const int blocks = (int)std::max<long long>(1, std::min(rows, cap));
+    bgr_to_gray_strided_kernel<<<blocks, 256, 0, st>>>(bgr, pitch, frame_stride, h, w, rows, gray);
     CB_CUDA(cudaGetLastError());
     ctx->launches++;
     return B200_OK;

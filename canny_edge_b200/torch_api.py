@@ -1,0 +1,118 @@
+"""torch front end of the device batch path: CUDA uint8 tensors in, uint8 0/255 tensors out.
+
+Any view whose rows are contiguous goes straight to the kernels with its strides — a crop `x[:, y0:y1, x0:x1]`, one channel of an
+`(N, C, H, W)` tensor, frames padded for alignment — through b200_canny_batch_device_strided; nothing is copied.  Layouts the
+kernels cannot address (rows that are not unit-stride, frames that overlap, broadcast frames) raise ValueError rather than being
+copied behind the caller's back.
+
+Work is issued on torch.cuda.current_stream(frames.device): the context is pointed at that stream on every call, so results are
+ordered with the caller's other torch work like any torch op.  When consecutive calls come from different streams, the later
+stream first waits for the earlier call (b200_ctx_set_stream), because calls on one context share its workspace.  torch is imported inside the functions, as in sharded.py.
+"""
+from __future__ import annotations
+
+import threading
+from typing import Dict, Optional, Tuple
+
+from .api import Context, canny_batch_device_bgr_strided_ptr, canny_batch_device_strided_ptr
+
+_contexts: Dict[int, Context] = {}
+_contexts_lock = threading.Lock()
+_call_lock = threading.Lock()   # a context's stream is state: pointing it at a stream and issuing the call happen together
+
+_CUDA_STREAM_LEGACY = 0x1   # cudaStreamLegacy (driver_types.h)
+_CONTIGUOUS_HINT = "pass a view whose rows are contiguous (e.g. call .contiguous() first)"
+
+
+def frame_layout(t, bgr: bool = False) -> Tuple[int, int, int, int, int]:
+    """(n_frames, height, width, row pitch, frame stride) of a uint8 tensor as the strided C calls take them, strides in bytes.
+
+    Gray: (H, W) or (N, H, W).  BGR: (H, W, 3) or (N, H, W, 3).  Raises ValueError for a layout the kernels cannot address."""
+    import torch
+
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"expected a torch.Tensor, got {type(t).__name__}")
+    if t.dtype != torch.uint8:
+        raise ValueError(f"expected a uint8 tensor, got {t.dtype}")
+    shape, stride = tuple(t.shape), tuple(t.stride())
+    if bgr:
+        if t.dim() not in (3, 4) or shape[-1] != 3:
+            raise ValueError(f"expected (H, W, 3) or (N, H, W, 3) B,G,R frames, got shape {shape}")
+        if stride[-1] != 1 or stride[-2] != 3:
+            raise ValueError(f"B,G,R pixels must be 3 contiguous bytes (strides (..., 3, 1), got {stride}); {_CONTIGUOUS_HINT}")
+        shape, stride = shape[:-1], stride[:-1]
+        row_bytes = 3 * shape[-1]
+    else:
+        if t.dim() not in (2, 3):
+            raise ValueError(f"expected (H, W) or (N, H, W) gray frames, got shape {shape}")
+        if stride[-1] != 1:
+            raise ValueError(f"rows must be contiguous (last stride 1, got {stride}); {_CONTIGUOUS_HINT}")
+        row_bytes = shape[-1]
+    h, w = shape[-2], shape[-1]
+    pitch = stride[-2]
+    n = shape[0] if len(shape) == 3 else 1
+    if h < 2 or w < 2:
+        raise ValueError(f"frames must be at least 2 x 2 pixels (got {h} x {w})")
+    if n < 1:
+        raise ValueError("no frames")
+    if pitch < row_bytes:
+        raise ValueError(f"rows overlap (row stride {pitch} < {row_bytes} bytes per row); {_CONTIGUOUS_HINT}")
+    frame_bytes = (h - 1) * pitch + row_bytes
+    frame_stride = stride[0] if len(shape) == 3 else h * pitch
+    if n > 1 and frame_stride < frame_bytes:
+        raise ValueError(f"frames overlap or are broadcast (frame stride {frame_stride} < {frame_bytes} bytes per frame); "
+                         f"{_CONTIGUOUS_HINT}")
+    if n == 1:
+        frame_stride = h * pitch
+    return n, h, w, pitch, frame_stride
+
+
+def _context(device_index: int) -> Context:
+    with _contexts_lock:
+        ctx = _contexts.get(device_index)
+        if ctx is None:
+            ctx = _contexts[device_index] = Context(device_index)
+        return ctx
+
+
+def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool):
+    import torch
+
+    n, h, w, in_pitch, in_fs = frame_layout(frames, bgr)
+    out_shape = tuple(frames.shape[:-1]) if bgr else tuple(frames.shape)
+    if not frames.is_cuda:
+        raise ValueError(f"frames must be a CUDA tensor (got device {frames.device})")
+    if out is None:
+        out = torch.empty(out_shape, dtype=torch.uint8, device=frames.device)
+    else:
+        if tuple(out.shape) != out_shape:
+            raise ValueError(f"out has shape {tuple(out.shape)}, expected {out_shape}")
+        if out.device != frames.device:
+            raise ValueError(f"out is on {out.device}, frames on {frames.device}")
+    _, _, _, out_pitch, out_fs = frame_layout(out, False)
+    dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
+    if ctx is None:
+        ctx = _context(dev)
+    elif ctx.device != dev:
+        raise ValueError(f"context is on cuda:{ctx.device}, frames on cuda:{dev}")
+    with _call_lock, torch.cuda.device(dev):
+        # torch's default stream has the handle 0, which the library reads as "the context's own stream": name the legacy default
+        # stream (cudaStreamLegacy) instead, so the work is ordered with the caller's
+        ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)
+        call = canny_batch_device_bgr_strided_ptr if bgr else canny_batch_device_strided_ptr
+        call(ctx, frames.data_ptr(), in_pitch, in_fs, n, h, w, sigma, min_val, max_val, out.data_ptr(), out_pitch, out_fs)
+    return out
+
+
+def canny(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx: Optional[Context] = None):
+    """Canny edge maps of gray frames: a CUDA uint8 tensor of shape (H, W) or (N, H, W), any strides with contiguous rows.
+
+    Returns a uint8 tensor of the same shape holding 0 / 255 (`out` when given: it may be a strided view, only its elements are
+    written).  Asynchronous on torch.cuda.current_stream(frames.device); ctx defaults to one cached Context per device."""
+    return _run(frames, sigma, min_val, max_val, out, ctx, bgr=False)
+
+
+def canny_bgr(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx: Optional[Context] = None):
+    """canny() for interleaved B,G,R frames (cv2 / cv::Mat layout): (H, W, 3) or (N, H, W, 3), each pixel's 3 bytes contiguous,
+    rows and frames with any stride.  The gray conversion is OpenCV's COLOR_BGR2GRAY, bit for bit.  Returns (H, W) or (N, H, W)."""
+    return _run(frames, sigma, min_val, max_val, out, ctx, bgr=True)

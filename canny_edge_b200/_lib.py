@@ -27,6 +27,12 @@ class BandRecord(C.Structure):
     _fields_ = [("label", C.c_int32), ("flags", C.c_int32)]
 
 
+class Frame(C.Structure):
+    """b200_frame: one frame of a b200_canny_frames_device list (device pointers, byte pitches)."""
+    _fields_ = [("in_", C.c_void_p), ("in_row_pitch", C.c_int64), ("out", C.c_void_p), ("out_row_pitch", C.c_int64),
+                ("height", C.c_int32), ("width", C.c_int32)]
+
+
 _u8p, _i16p, _f32p = C.c_void_p, C.c_void_p, C.c_void_p  # raw addresses (numpy .ctypes.data / tensor.data_ptr())
 _ctx = C.c_void_p
 
@@ -64,6 +70,8 @@ SIGNATURES = {
                                                   C.c_int, _u8p, C.c_int64, C.c_int64]),
     "b200_canny_batch_device_bgr_strided": (C.c_int, [_ctx, _u8p, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int,
                                                       C.c_int, _u8p, C.c_int64, C.c_int64]),
+    "b200_canny_frames_device": (C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_float, C.c_int, C.c_int]),
+    "b200_canny_frames_device_bgr": (C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_float, C.c_int, C.c_int]),
     "b200_profile_stages_device": (C.c_int, [_ctx, _u8p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, _u8p, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "b200_profile_pipeline_device": (C.c_int, [_ctx, _u8p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, _u8p, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "b200_hash_edges_device": (C.c_int, [_ctx, _u8p, C.c_size_t, C.c_ulonglong, C.POINTER(C.c_ulonglong)]),

@@ -223,6 +223,24 @@ def canny_batch_device_bgr_strided_ptr(ctx: Optional[Context], d_bgr: int, in_ro
                                                      int(out_row_pitch), int(out_frame_stride)))
 
 
+def frame_list(descs) -> C.Array:
+    """(in_ptr, in_pitch, out_ptr, out_pitch, h, w) tuples -> the ctypes array of b200_frame that b200_canny_frames_device takes."""
+    descs = list(descs)
+    arr = (_lib.Frame * max(1, len(descs)))()
+    for i, (in_ptr, in_pitch, out_ptr, out_pitch, h, w) in enumerate(descs):
+        arr[i] = _lib.Frame(in_ptr, int(in_pitch), out_ptr, int(out_pitch), int(h), int(w))
+    return arr
+
+
+def canny_frames_device_ptr(ctx: Optional[Context], descs, sigma: float, min_val: int, max_val: int, bgr: bool = False) -> None:
+    """Frames of different sizes in one call (b200_canny_frames_device[_bgr]).  descs: a sequence of (in_ptr, in_pitch, out_ptr,
+    out_pitch, h, w) with device pointers and byte pitches: pixel (y, x) of a frame is read at in_ptr + y*in_pitch + x (3 bytes at
+    + 3*x for B,G,R) and written at out_ptr + y*out_pitch + x.  Asynchronous on the context's stream."""
+    descs = list(descs)
+    fn = load().b200_canny_frames_device_bgr if bgr else load().b200_canny_frames_device
+    check(fn(_h(ctx), frame_list(descs), len(descs), C.c_float(sigma), int(min_val), int(max_val)))
+
+
 def synth_host(n: int, h: int, w: int, kind: int = 0, seed: int = 1234, first_frame: int = 0) -> np.ndarray:
     out = np.empty((n, h, w), np.uint8)
     check(load().b200_synth_host(_ptr(out), n, h, w, kind, C.c_uint64(seed), first_frame))

@@ -16,6 +16,8 @@
 #include <mutex>
 #include <thread>
 
+#include <cuda.h>
+
 #include "canny_math.h"
 #include "internal.h"
 
@@ -448,6 +450,7 @@ int b200_ctx_create(int device, b200_ctx** out) {
             CB_CUDA(cudaEventCreateWithFlags(&c->ev_join[i], cudaEventDisableTiming));
             CB_CUDA(cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming | cudaEventBlockingSync));
             CB_CUDA(cudaEventCreateWithFlags(&c->ev_in[i], cudaEventDisableTiming));
+            CB_CUDA(cudaEventCreateWithFlags(&c->ev_ragged[i], cudaEventDisableTiming));
         }
         CB_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
         CB_CUDA(cudaEventCreateWithFlags(&c->ev_switch, cudaEventDisableTiming));
@@ -479,6 +482,9 @@ int b200_ctx_destroy(b200_ctx* c) {
         if (c->ev_join[i]) cudaEventDestroy(c->ev_join[i]);
         if (c->ev_chunk[i]) cudaEventDestroy(c->ev_chunk[i]);
         if (c->ev_in[i]) cudaEventDestroy(c->ev_in[i]);
+        if (c->ev_ragged[i]) cudaEventDestroy(c->ev_ragged[i]);
+        rel(c->ws_ragged[i], false);
+        rel(c->host_ragged[i], true);
         rel(c->host_in[i], true);
         rel(c->dev_bits[i], false);
         rel(c->host_bits[i], true);
@@ -925,6 +931,229 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
                                         int64_t out_row_pitch, int64_t out_frame_stride) {
     return batch_device_impl(ctx, d_bgr, in_row_pitch, in_frame_stride, n_frames, h, w, sigma, lo, hi, d_edges, out_row_pitch,
                              out_frame_stride, 3);
+}
+
+// ---- ragged lists: frames of different sizes in one call ------------------------------------------------
+// Argument checks of b200_canny_frames_device[_bgr]; all of them run before any device work.  Overlaps are found by sorting the
+// extents (a list can hold thousands of frames): the outputs among themselves, then every output against the merged inputs.
+static int check_frames(const b200_frame* fr, int n, int bpp) {
+    if (!fr) { set_error("null frame list"); return B200_ERR_INVALID_ARG; }
+    if (n <= 0) { set_error("n_frames must be positive"); return B200_ERR_INVALID_ARG; }
+    typedef __int128 i128;
+    struct Ext { i128 lo, hi; int idx; };
+    std::vector<Ext> ins((size_t)n), outs((size_t)n);
+    for (int i = 0; i < n; ++i) {
+        const b200_frame& f = fr[i];
+        if (!f.in || !f.out) { set_error("frame %d: null image pointer", i); return B200_ERR_INVALID_ARG; }
+        if (f.height < 2 || f.width < 2) { set_error("frame %d: height and width must be >= 2 (got %dx%d)", i, f.height, f.width); return B200_ERR_INVALID_ARG; }
+        if (f.in_row_pitch < 0 || f.out_row_pitch < 0) {
+            set_error("frame %d: negative row pitch (in %lld, out %lld)", i, (long long)f.in_row_pitch, (long long)f.out_row_pitch);
+            return B200_ERR_INVALID_ARG;
+        }
+        const long long in_row = (long long)bpp * f.width;
+        if (f.in_row_pitch < in_row) { set_error("frame %d: input row pitch %lld is smaller than a row (%lld bytes)", i, (long long)f.in_row_pitch, in_row); return B200_ERR_INVALID_ARG; }
+        if (f.out_row_pitch < f.width) { set_error("frame %d: output row pitch %lld is smaller than a row (%d bytes)", i, (long long)f.out_row_pitch, f.width); return B200_ERR_INVALID_ARG; }
+        // extents in 128-bit arithmetic, as check_strided
+        const i128 in_ext = (i128)(f.height - 1) * f.in_row_pitch + in_row, out_ext = (i128)(f.height - 1) * f.out_row_pitch + f.width;
+        const i128 kMaxExtent = (i128)1 << 48;
+        if (in_ext > kMaxExtent || out_ext > kMaxExtent) {
+            set_error("frame %d: pitches span more than 2^48 bytes (input %.3g, output %.3g bytes)", i, (double)in_ext, (double)out_ext);
+            return B200_ERR_INVALID_ARG;
+        }
+        if ((long long)f.height * f.width >= (1LL << 31)) { set_error("frame %d: %dx%d pixels exceed int indexing", i, f.height, f.width); return B200_ERR_UNSUPPORTED; }
+        const i128 in_lo = (i128)reinterpret_cast<uintptr_t>(f.in), out_lo = (i128)reinterpret_cast<uintptr_t>(f.out);
+        ins[(size_t)i] = Ext{in_lo, in_lo + in_ext, i};
+        outs[(size_t)i] = Ext{out_lo, out_lo + out_ext, i};
+    }
+    auto by_lo = [](const Ext& a, const Ext& b) { return a.lo < b.lo || (a.lo == b.lo && a.idx < b.idx); };
+    std::sort(outs.begin(), outs.end(), by_lo);
+    for (size_t k = 1; k < outs.size(); ++k)
+        if (outs[k].lo < outs[k - 1].hi) { set_error("the outputs of frames %d and %d overlap", outs[k - 1].idx, outs[k].idx); return B200_ERR_INVALID_ARG; }
+    // inputs may overlap each other: merge them, then look up each output's first merged run that ends after its start
+    std::sort(ins.begin(), ins.end(), by_lo);
+    std::vector<Ext> runs;
+    for (const Ext& e : ins) {
+        if (!runs.empty() && e.lo < runs.back().hi) { if (e.hi > runs.back().hi) runs.back().hi = e.hi; }
+        else runs.push_back(e);
+    }
+    for (const Ext& o : outs) {
+        auto it = std::upper_bound(runs.begin(), runs.end(), o.lo, [](i128 v, const Ext& r) { return v < r.hi; });
+        if (it != runs.end() && it->lo < o.hi) { set_error("the output of frame %d overlaps an input", o.idx); return B200_ERR_INVALID_ARG; }
+    }
+    return B200_OK;
+}
+
+constexpr long long kRaggedChunkPx = 75LL << 20;   // the uniform path's chunk budget (auto_chunk_frames): a chunk's class map fits L2
+
+static size_t align16(size_t v) { return (v + 15) & ~(size_t)15; }
+
+// One chunk of a ragged list on slot s / stream st: table (descriptors, tensor maps, work items, B,G,R jobs) built on the host into
+// the slot's pinned staging and sent up with one copy; then [B,G,R -> gray], the front kernel (one launch per staging form, both
+// appending to the same weak-pixel list) and the list-driven hysteresis kernels.
+static int run_ragged_chunk(b200_ctx* ctx, cudaStream_t st, int s, const b200_frame* fr, int nf, int lo, int hi, bool bgr) {
+    const int radius = ctx->gauss.radius;
+    std::vector<int> hs((size_t)nf), ws((size_t)nf);
+    std::vector<const uint8_t*> src((size_t)nf);
+    std::vector<long long> src_pitch((size_t)nf), gray_off((size_t)nf);
+    long long px = 0, gray_bytes = 0;
+    for (int i = 0; i < nf; ++i) {
+        hs[(size_t)i] = fr[i].height; ws[(size_t)i] = fr[i].width;
+        px += (long long)fr[i].height * fr[i].width;
+        if (bgr) {
+            // every converted frame takes TMA: 16-byte aligned base and row pitch in the chunk's gray scratch
+            const long long pitch = (fr[i].width + 15) & ~15LL;
+            gray_off[(size_t)i] = gray_bytes;
+            src[(size_t)i] = reinterpret_cast<const uint8_t*>(ctx->dev_in[s].ptr) + gray_bytes;
+            src_pitch[(size_t)i] = pitch;
+            gray_bytes += pitch * fr[i].height;
+        } else {
+            src[(size_t)i] = fr[i].in;
+            src_pitch[(size_t)i] = fr[i].in_row_pitch;
+        }
+    }
+    std::vector<CUtensorMap> maps((size_t)nf);
+    std::vector<RaggedItem> items_tma, items_byte;
+    const int band_rows = ragged_band_rows3(ctx, hs.data(), ws.data(), nf, radius);
+    for (int i = 0; i < nf; ++i) {
+        bool use_tma = false;
+        CB_TRY(ragged_tensor_map3(src[(size_t)i], src_pitch[(size_t)i], hs[(size_t)i], ws[(size_t)i], radius, &maps[(size_t)i], &use_tma));
+        ragged_items3(i, hs[(size_t)i], ws[(size_t)i], band_rows, use_tma ? items_tma : items_byte);
+    }
+    // the longest CTAs first (frames shorter than the band height have shorter ones): the launch ends on short CTAs
+    auto longer = [](const RaggedItem& a, const RaggedItem& b) { return a.ye - a.yb > b.ye - b.yb; };
+    std::stable_sort(items_tma.begin(), items_tma.end(), longer);
+    std::stable_sort(items_byte.begin(), items_byte.end(), longer);
+    const size_t n_items = items_tma.size() + items_byte.size();
+    // table: tensor maps (128 B, 64-byte aligned) | frame descriptors | bases | work items | B,G,R jobs
+    const size_t off_frames = (size_t)nf * sizeof(CUtensorMap);
+    const size_t off_bases = align16(off_frames + (size_t)nf * sizeof(RaggedFrame));
+    const size_t off_items = align16(off_bases + (size_t)nf * sizeof(uint32_t));
+    const size_t off_jobs = align16(off_items + n_items * sizeof(RaggedItem));
+    const size_t bytes = off_jobs + (bgr ? (size_t)nf * sizeof(RaggedGrayJob) : 0);
+    // the staging of this slot is rewritten only once the copy out of it (previous chunk or call on this slot) has completed
+    if (ctx->ragged_busy[s]) { CB_CUDA(cudaEventSynchronize(ctx->ev_ragged[s])); ctx->ragged_busy[s] = false; }
+    CB_TRY(ensure_ws(ctx->host_ragged[s], bytes, /*pinned_host=*/true));
+    CB_TRY(ensure_ws(ctx->ws_ragged[s], bytes));
+    uint8_t* h = reinterpret_cast<uint8_t*>(ctx->host_ragged[s].ptr);
+    uint8_t* d = reinterpret_cast<uint8_t*>(ctx->ws_ragged[s].ptr);
+    memcpy(h, maps.data(), off_frames);
+    RaggedFrame* hf = reinterpret_cast<RaggedFrame*>(h + off_frames);
+    uint32_t* hb = reinterpret_cast<uint32_t*>(h + off_bases);
+    RaggedGrayJob* hj = reinterpret_cast<RaggedGrayJob*>(h + off_jobs);
+    long long base = 0, row0 = 0;
+    for (int i = 0; i < nf; ++i) {
+        const b200_frame& f = fr[i];
+        RaggedFrame& r = hf[i];
+        r.in = src[(size_t)i]; r.in_pitch = src_pitch[(size_t)i];
+        r.cls = f.out; r.cls_pitch = f.out_row_pitch;
+        r.height = f.height; r.width = f.width;
+        r.base = (int)base;
+        r.cls_words = ((reinterpret_cast<uintptr_t>(f.out) | (uintptr_t)f.out_row_pitch) & 3) == 0;
+        hb[i] = (uint32_t)base;
+        base += (long long)f.height * f.width;
+        if (bgr) {
+            hj[i] = RaggedGrayJob{f.in, f.in_row_pitch, const_cast<uint8_t*>(src[(size_t)i]), src_pitch[(size_t)i], (int)row0, f.width};
+            row0 += f.height;
+        }
+    }
+    memcpy(h + off_items, items_tma.data(), items_tma.size() * sizeof(RaggedItem));
+    memcpy(h + off_items + items_tma.size() * sizeof(RaggedItem), items_byte.data(), items_byte.size() * sizeof(RaggedItem));
+    CB_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, st));
+    CB_CUDA(cudaEventRecord(ctx->ev_ragged[s], st));
+    ctx->ragged_busy[s] = true;
+    if (bgr) CB_TRY(launch_bgr_to_gray_ragged(ctx, st, reinterpret_cast<const RaggedGrayJob*>(d + off_jobs), nf, row0));
+
+    FrontParams fp;
+    memset(&fp, 0, sizeof(fp));
+    fp.out_rows = 1; fp.tiles_y = 1;
+    fp.w = ctx->gauss.d_w; fp.count = ctx->gauss.d_count; fp.radius = radius;
+    fill_thresholds(fp, lo, hi);
+    fp.parent = reinterpret_cast<int32_t*>(ctx->ws_parent[s].ptr);
+    fp.kept_count = reinterpret_cast<unsigned int*>(ctx->ws_list[s].ptr);
+    fp.kept_list = reinterpret_cast<uint32_t*>(ctx->ws_list[s].ptr) + 16;
+    fp.rframes = reinterpret_cast<const RaggedFrame*>(d + off_frames);
+    fp.rtmaps = reinterpret_cast<const CUtensorMap*>(d);
+    // the list's counter block is zero here (see run_frames_device)
+    if (ctx->list_dirty[s]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
+    ctx->list_dirty[s] = true;
+    const RaggedItem* d_items = reinterpret_cast<const RaggedItem*>(d + off_items);
+    fp.ritems = d_items;
+    CB_TRY(launch_front3_ragged(ctx, st, fp, (int)items_tma.size(), true));
+    fp.ritems = d_items + items_tma.size();
+    CB_TRY(launch_front3_ragged(ctx, st, fp, (int)items_byte.size(), false));
+    RaggedHystParams hp;
+    memset(&hp, 0, sizeof(hp));
+    hp.frames = fp.rframes;
+    hp.bases = reinterpret_cast<const uint32_t*>(d + off_bases);
+    hp.n_frames = nf;
+    hp.parent = fp.parent; hp.list = fp.kept_list; hp.ctr = fp.kept_count;
+    hp.px = px;
+    CB_TRY(launch_hysteresis_ragged(ctx, st, hp));
+    ctx->list_dirty[s] = false;
+    return B200_OK;
+}
+
+static int frames_device_impl(b200_ctx* ctx, const b200_frame* fr, int n, float sigma, int lo, int hi, int bpp) {
+    CB_TRY(check_frames(fr, n, bpp));
+    CB_TRY(check_thresholds(lo, hi));
+    CB_TRY(resolve_ctx(ctx));
+    CB_TRY(prepare_gauss(ctx, sigma));
+    static const int force = [] { const char* e = getenv("B200_CANNY_FRONT"); return e ? atoi(e) : 0; }();
+    if (force != 0 || ctx->gauss.tiny || !front3_supports(ctx->gauss.radius)) {
+        // no ragged kernel for this sigma (or a front kernel forced for A/B runs): each frame through the strided path
+        for (int i = 0; i < n; ++i) {
+            const b200_frame& f = fr[i];
+            CB_TRY(batch_device_impl(ctx, f.in, f.in_row_pitch, f.height * f.in_row_pitch, 1, f.height, f.width, sigma, lo, hi, f.out,
+                                     f.out_row_pitch, f.height * f.out_row_pitch, bpp));
+        }
+        return B200_OK;
+    }
+    // chunks in call order: about the uniform path's pixel budget each, at most chunk_frames (b200_ctx_set_chunk_frames) frames;
+    // a frame above the budget has a chunk of its own
+    const int cap = std::min(ctx->chunk_frames > 0 ? ctx->chunk_frames : kMaxChunkFrames, kMaxChunkFrames);
+    std::vector<int> starts;
+    long long chunk_px = 0, max_px = 0, max_gray = 0, gray = 0;
+    for (int i = 0; i < n; ++i) {
+        const long long fpx = (long long)fr[i].height * fr[i].width;
+        if (i == 0 || (chunk_px + fpx > kRaggedChunkPx || i - starts.back() >= cap)) {
+            starts.push_back(i);
+            chunk_px = 0;
+            gray = 0;
+        }
+        chunk_px += fpx;
+        gray += ((fr[i].width + 15) & ~15LL) * fr[i].height;
+        max_px = std::max(max_px, chunk_px);
+        max_gray = std::max(max_gray, gray);
+    }
+    starts.push_back(n);
+    const int n_chunks = (int)starts.size() - 1;
+    const int n_slots = std::min(3, n_chunks);
+    for (int s = 0; s < n_slots; ++s) {
+        CB_TRY(ensure_ws(ctx->ws_parent[s], (size_t)max_px * 4));
+        CB_TRY(ensure_ws(ctx->ws_list[s], 64 + (size_t)max_px * 4));
+        if (bpp == 3) CB_TRY(ensure_ws(ctx->dev_in[s], (size_t)max_gray));
+    }
+    if (n_slots == 1) return run_ragged_chunk(ctx, ctx->stream, 0, fr, n, lo, hi, bpp == 3);
+    // the same three stream slots and fork / join as batch_device_impl
+    CB_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+    for (int s = 0; s < n_slots; ++s) CB_CUDA(cudaStreamWaitEvent(ctx->side[s], ctx->ev_fork, 0));
+    for (int c = 0; c < n_chunks; ++c) {
+        const int s = c % n_slots;
+        CB_TRY(run_ragged_chunk(ctx, ctx->side[s], s, fr + starts[(size_t)c], starts[(size_t)c + 1] - starts[(size_t)c], lo, hi, bpp == 3));
+    }
+    for (int s = 0; s < n_slots; ++s) {
+        CB_CUDA(cudaEventRecord(ctx->ev_join[s], ctx->side[s]));
+        CB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[s], 0));
+    }
+    return B200_OK;
+}
+
+int b200_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val) {
+    return frames_device_impl(ctx, frames, n_frames, sigma, min_val, max_val, 1);
+}
+
+int b200_canny_frames_device_bgr(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val) {
+    return frames_device_impl(ctx, frames, n_frames, sigma, min_val, max_val, 3);
 }
 
 // Host buffers in, host buffers out: frames -> 0 / 255 edge maps, as bytes (edges8) or as the reference's int16 (edges16).

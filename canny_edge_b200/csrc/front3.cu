@@ -23,6 +23,9 @@
 // Used for compile-time radii without spill planes; everything else (run-time radius, `steps` planes, sigma so small that sums
 // approach the subnormal range) stays on front.cu's kernel.  B200_CANNY_FRONT=2 selects front2.cu's kernel for A/B runs.
 #include <cuda.h>
+#include <string.h>
+
+#include <algorithm>
 
 #include "canny_math.h"
 #include "exact_math.cuh"
@@ -125,7 +128,12 @@ __device__ __forceinline__ void red_or_shared_if(bool on, uint32_t* ptr, uint32_
 // (b200_canny_batch_device_strided; layout_pitched()).  Dense layouts (the batch and host paths) keep the dense addressing, whose
 // class and union-find offsets are one and the same, so their instruction stream and register allocation are those of the
 // dense-only kernel.
-template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false, bool PITCHED = false>
+// RAGGED: frames of different sizes in one launch (b200_canny_frames_device).  A 1-D grid over work items (p.ritems): the item names
+// the frame, the strip and the row band, and the frame's descriptor (p.rframes) replaces in / in_pitch / width / height / cls /
+// cls_pitch / cls_words and the slot base, with the pitched addressing.  Frames are whole images (in_row0 = plane_row0 = 0), so
+// every border rule keys off the frame's own H and W.  TMA staging reads the frame's tensor map from the chunk's table in global
+// memory.  Gray input, DIV 5 only.
+template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false, bool PITCHED = false, bool RAGGED = false>
 #ifndef F3_MAXREG
 #define F3_MAXREG 96
 #endif
@@ -143,6 +151,7 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
     constexpr SmemLayout L = smem_layout(R, SLAB, BGR);
     constexpr int in_pitch = in_pitch_for(R);
     static_assert(!BGR || (USE_TMA && 3 * in_pitch == kVuPitch * 4 && R <= 9), "BGR staging: one TMA box row per VU row, 160 staged columns");
+    static_assert(!RAGGED || (!BGR && !PITCHED && DIV == 5), "ragged launches: gray input, their own pitched addressing, DIV 5");
     constexpr int T0 = 2 * R + 2;  // temp buffer row of the first row of the current slab
 
     unsigned char* s_in = smem + L.in_off;
@@ -170,13 +179,19 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
 #endif
 
     // ---- which strip / band / frame ----
-    const int strip = blockIdx.x, band = blockIdx.y, frame = blockIdx.z;
-    const int x0 = strip * kTW;
+    RaggedItem item{};
+    RaggedFrame fd{};
+    if (RAGGED) {
+        item = p.ritems[blockIdx.x];
+        fd = p.rframes[item.frame];
+    }
+    const int strip = blockIdx.x, band = blockIdx.y, frame = RAGGED ? item.frame : blockIdx.z;
+    const int x0 = RAGGED ? item.x0 : strip * kTW;
     const int rows_per_band = (p.out_rows + p.tiles_y - 1) / p.tiles_y;
-    const int yb = p.out_row0 + band * rows_per_band;
-    const int ye = min(p.out_row0 + p.out_rows, yb + rows_per_band);
+    const int yb = RAGGED ? item.yb : p.out_row0 + band * rows_per_band;
+    const int ye = RAGGED ? item.ye : min(p.out_row0 + p.out_rows, yb + rows_per_band);
     if (yb >= ye) return;
-    const int W = p.width, H = p.height;
+    const int W = RAGGED ? fd.width : p.width, H = RAGGED ? fd.height : p.height;
     const int n_slabs = (ye - yb + 2 * R + 4 + kSlab - 1) / kSlab;
     const int in_y0 = yb - 2 - R;                 // global row of slab 0, line 0
     const int lead = (x0 - 2 - R) & 15;           // bytes between the 16 B aligned box origin and the first needed column
@@ -193,6 +208,9 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
         mbar_init(bar0 + 8, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        // a tensor map in global memory, written by a host copy: acquire it for the tensor-map proxy before its first use (CUDA
+        // programming guide, "Using TMA to transfer multi-dimensional arrays": scope .sys after a cudaMemcpy from the host)
+        if (RAGGED) asm volatile("fence.proxy.tensormap::generic.acquire.sys [%0], 128;" ::"l"(p.rtmaps + frame) : "memory");
     }
     __syncthreads();
 
@@ -209,7 +227,7 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
     // strips that contain image column -1 or W need the virtual Sobel columns patched in (see the patch pass)
     const bool x_edge = (x0 - 2 < 0) || (x0 - 2 + kTC - 1 >= W);
 
-    const uint8_t* in_frame = p.in + (long long)frame * p.in_frame_stride;
+    const uint8_t* in_frame = RAGGED ? fd.in : p.in + (long long)frame * p.in_frame_stride;
     constexpr uint32_t slab_bytes = (uint32_t)(kSlab * in_pitch);
 
     constexpr int kInBufs = BGR ? 1 : in_bufs_for(R);
@@ -220,7 +238,8 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
             if (tid == 0) {
                 const uint32_t bar = bar0 + 8 * (k % kInBufs);
                 mbar_expect_tx(bar, slab_bytes);
-                tma_load_3d(smem_u32(dst), &tmap, bar, in_x0, gy - p.in_row0, frame);
+                if (RAGGED) tma_load_3d(smem_u32(dst), p.rtmaps + frame, bar, in_x0, gy, 0);
+                else tma_load_3d(smem_u32(dst), &tmap, bar, in_x0, gy - p.in_row0, frame);
             }
         } else {
             // generic staging (image pitch not a multiple of 16 B): byte loads, zero outside the image / buffer
@@ -229,7 +248,8 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 const int y = gy + r, x = in_x0 + c;
                 const int by = y - p.in_row0;
                 unsigned char v = 0;
-                if (y >= 0 && y < H && by >= 0 && by < p.in_rows && x >= 0 && x < W) v = in_frame[(long long)by * (PITCHED ? p.in_pitch : (long long)W) + x];
+                if (y >= 0 && y < H && by >= 0 && by < (RAGGED ? H : p.in_rows) && x >= 0 && x < W)
+                    v = in_frame[(long long)by * (RAGGED ? fd.in_pitch : PITCHED ? p.in_pitch : (long long)W) + x];
                 dst[i] = v;
             }
         }
@@ -548,17 +568,18 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 }
                 const uint32_t zero_word = 0x01010101u * (uint32_t)p.cls_zero;
                 // dense layouts: base aligned (layout_pitched), so word stores need a width that is a multiple of 4
-                const bool words = PITCHED ? p.cls_words != 0 : ((W & 3) == 0);
+                const bool words = RAGGED ? fd.cls_words != 0 : PITCHED ? p.cls_words != 0 : ((W & 3) == 0);
                 const bool word_ok = words && lane < kTW / 4 && (x0 + 4 * lane + 3 < W);  // the aligned 32-bit store applies
                 const bool tail_ok = !word_ok && lane < kTW / 4 && (x0 + 4 * lane < W);            // ragged right edge: byte stores
                 const unsigned lt_mask = (1u << lane) - 1u;
                 int q = cq_lo + ((warp - cq_lo) & 7);         // first class row of this warp (rows q = warp mod 8)
                 const int32_t* vrow = s_vu + q * kVuPitch + 4 * lane;
                 float* nrow = s_np + q * kNpPitch + 4 * lane;
-                uint8_t* o = PITCHED ? p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * p.cls_pitch + (x0 + 4 * lane)
+                uint8_t* o = RAGGED ? fd.cls + (long long)(y_base + q - 1) * fd.cls_pitch + (x0 + 4 * lane)
+                           : PITCHED ? p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * p.cls_pitch + (x0 + 4 * lane)
                                      : p.cls + (long long)frame * p.out_frame_stride + (long long)(y_base + q - 1 - p.plane_row0) * W + (x0 + 4 * lane);
                 int ent = ((q - 1) << 6) | (lane << 1);
-                const long long o_step = 8LL * (PITCHED ? p.cls_pitch : (long long)W);
+                const long long o_step = 8LL * (RAGGED ? fd.cls_pitch : PITCHED ? p.cls_pitch : (long long)W);
                 // two copies of the loop so the store form is decided once, not per row: the aligned 32-bit store (every strip of
                 // a class map whose base, pitch and frame stride are multiples of 4, except a ragged last strip) or byte stores
                 auto class_row_nq = [&](const float4 nq, float* nr, int e16) {
@@ -619,9 +640,14 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
         // per SM this phase is bound by those chains, not by issue slots.
         {
             // PITCHED: the class byte is addressed through the caller's pitches; the union-find slot and the list index stay dense
-            const long long out_off = (long long)frame * p.out_frame_stride + (long long)(y_base - p.plane_row0) * W + (x0 - 2) + 1;
-            uint8_t* out_base = PITCHED ? p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base - p.plane_row0) * p.cls_pitch + (x0 - 2) + 1
+            const long long out_off = RAGGED ? (long long)fd.base + (long long)y_base * W + (x0 - 2) + 1
+                                             : (long long)frame * p.out_frame_stride + (long long)(y_base - p.plane_row0) * W + (x0 - 2) + 1;
+            uint8_t* out_base = RAGGED ? fd.cls + (long long)y_base * fd.cls_pitch + (x0 - 2) + 1
+                              : PITCHED ? p.cls + (long long)frame * p.cls_frame_stride + (long long)(y_base - p.plane_row0) * p.cls_pitch + (x0 - 2) + 1
                                         : p.cls + out_off;
+            // ragged launches always hand over the list, also when minVal <= 0 makes every suppressed pixel weak (class cls_zero = 1):
+            // then every class pixel that is not kept as strong is listed
+            const bool zero_weak = RAGGED && p.cls_zero == 1;
             int32_t* par_base = p.parent + out_off;                           // only dereferenced when `sparse`
             const int idx_base = (int)out_off;                                // launch-relative pixel index of (class row 0, column j = 1)
             for (int i = lane; i < my_count; i += 64) {
@@ -640,7 +666,8 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 for (int u = 0; u < 2; ++u) {
                     const int rr = ent[u] >> 6, c0 = 2 * (ent[u] & 63);        // pixels j = c0 + 1 and c0 + 2 of class row rr
                     rel[u] = rr * W + c0;                                      // < 2^31: rr < 64, W < 2^24
-                    orow[u] = PITCHED ? out_base + ((long long)rr * p.cls_pitch + c0) : out_base + (unsigned)rel[u];
+                    orow[u] = RAGGED ? out_base + ((long long)rr * fd.cls_pitch + c0)
+                            : PITCHED ? out_base + ((long long)rr * p.cls_pitch + c0) : out_base + (unsigned)rel[u];
                     prow[u] = par_base + (unsigned)rel[u];
                     const int32_t* vrow = s_vu + (rr + 1) * kVuPitch + c0;     // VU words j-1 .. j+2 = c0 .. c0+3
                     const uint2 qa = *reinterpret_cast<const uint2*>(vrow);
@@ -693,7 +720,7 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                         // hand-over to the list-driven hysteresis kernels: only WEAK pixels need any work there (a strong pixel is
                         // final; its neighbours find it through the class map).  The weak pixel gets its union-find slot (itself)
                         // and a bit in the slab's bitmap, from which the list entries are made once the slab is finished
-                        const bool weak = sparse && keep && !strong;
+                        const bool weak = RAGGED ? sparse && (keep ? !strong : (pass[u][e] && zero_weak)) : sparse && keep && !strong;
                         st_u32_if(weak, prow[u] + e, (uint32_t)(idx_base + rel[u] + e));
                         red_or_shared_if(weak, bits[u][e], mask[u][e]);
                     }
@@ -724,7 +751,8 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
                 asm volatile("atom.global.add.u32 %0, [%1], %2;" : "=r"(pend_base) : "l"(p.kept_count + threadIdx.z), "r"((unsigned int)total) : "memory");
             pend_off = incl - cnt;
             // word tid <-> class row rr = tid >> 2, columns 32*(tid & 3) .. of the strip
-            pend_g0 = (int)((long long)frame * p.out_frame_stride + (long long)(y_base + (tid >> 2) - p.plane_row0) * W + x0 + 32 * (tid & 3));
+            pend_g0 = RAGGED ? (int)((long long)fd.base + (long long)(y_base + (tid >> 2)) * W + x0 + 32 * (tid & 3))
+                             : (int)((long long)frame * p.out_frame_stride + (long long)(y_base + (tid >> 2) - p.plane_row0) * W + x0 + 32 * (tid & 3));
         }
         // VU rows 64,65 (blurred-row neighbours of the next slab's first class rows) -> rows 0,1
         if (!BGR) {
@@ -752,18 +780,18 @@ front3_kernel(const FrontParams p, const __grid_constant__ CUtensorMap tmap) {
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false, bool PITCHED = false>
+template <int R, bool USE_TMA, int DIV, int SLAB, bool BGR = false, bool PITCHED = false, bool RAGGED = false>
 static int launch_one3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CUtensorMap& tmap, dim3 grid) {
     const f3::SmemLayout L = f3::smem_layout(R, SLAB, BGR);
     static bool configured[64] = {false};  // per instantiation, per device
     if (!configured[ctx->device & 63]) {
-        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
-        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED, RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, L.total));
+        CB_CUDA(cudaFuncSetAttribute(f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED, RAGGED>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
         configured[ctx->device & 63] = true;
     }
     {
         ProfScope ps(ctx, st, 0);
-        f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED><<<grid, f3::kThreads, L.total, st>>>(p, tmap);
+        f3::front3_kernel<R, USE_TMA, DIV, SLAB, BGR, PITCHED, RAGGED><<<grid, f3::kThreads, L.total, st>>>(p, tmap);
     }
     CB_CUDA(cudaGetLastError());
     ctx->launches++;
@@ -840,6 +868,84 @@ static int choose_bands3(const b200_ctx* ctx, int out_rows, int strips, int fram
         if (cost < best_cost * 0.999) { best_cost = cost; best = b; }
     }
     return best;
+}
+
+// ---- ragged chunks ----
+// Band policy: one class-row band height T for the whole chunk, every frame cut into ceil(H / T) equal bands, so every CTA marches
+// about the same rows (T plus the 2R+4 warm-up rows) whatever its frame's size: large frames get more bands and the CTAs of a chunk
+// take similar times.  T is chosen from the heights that fill whole 64-row slabs (64k - 2R - 4) by the list-scheduling estimate
+// of the chunk's time: slab-steps of all CTAs over the 2 x SMs CTA slots, plus the longest CTA (the last wave's tail); the largest
+// T within 0.1 % of the best wins, since more bands cost warm-up rows.  Measured with this policy on one B200 (1000 W), 2000 frames of
+// 320x240 .. 1920x1080 (tools/ragged_probe.py, profiles/r04_ragged_probe.jsonl): 113 Gpix/s for the C call on "shapes" content
+// against 281 Gpix/s for the same pixels as uniform 4K frames and 21 Gpix/s for one call per frame; other policies not measured.
+int ragged_band_rows3(const b200_ctx* ctx, const int* heights, const int* widths, int n, int radius) {
+    const long long slots = 2LL * (ctx->sm_count > 0 ? ctx->sm_count : 148);
+    const int warm = 2 * radius + 4, slab = 64;
+    int max_h = 0;
+    for (int i = 0; i < n; ++i) max_h = std::max(max_h, heights[i]);
+    int best = max_h;
+    double best_cost = 1e300;
+    for (int k = (max_h + warm + slab - 1) / slab; k >= 1; --k) {
+        const int t = std::min(max_h, std::max(16, slab * k - warm));
+        long long steps = 0;
+        int longest = 0;
+        for (int i = 0; i < n; ++i) {
+            const int bands = (heights[i] + t - 1) / t;
+            const int rows = (heights[i] + bands - 1) / bands;
+            const int slabs = (rows + warm + slab - 1) / slab;
+            steps += (long long)slabs * bands * ((widths[i] + f3::kTW - 1) / f3::kTW);
+            longest = std::max(longest, slabs);
+        }
+        const double cost = (double)steps / (double)slots + longest;
+        if (cost < best_cost * 0.999) { best_cost = cost; best = t; }
+    }
+    return best;
+}
+
+void ragged_items3(int frame, int height, int width, int band_rows, std::vector<RaggedItem>& items) {
+    const int bands = (height + band_rows - 1) / band_rows;
+    const int rows = (height + bands - 1) / bands;
+    for (int b = 0; b < bands; ++b) {
+        const int yb = b * rows, ye = std::min(height, yb + rows);
+        if (yb >= ye) break;
+        for (int x0 = 0; x0 < width; x0 += f3::kTW) items.push_back(RaggedItem{frame, x0, yb, ye});
+    }
+}
+
+// The tensor map of one ragged frame (3-D like the uniform maps, one frame deep); *use_tma is false when its base or pitch is not a
+// multiple of 16 bytes (the frame then takes the byte-load staging)
+int ragged_tensor_map3(const uint8_t* in, long long pitch, int height, int width, int radius, CUtensorMap_st* tmap, bool* use_tma) {
+    FrontParams p;
+    memset(&p, 0, sizeof(p));
+    p.in = in; p.in_pitch = pitch; p.in_frame_stride = (long long)height * pitch; p.in_rows = height; p.width = width; p.n_frames = 1;
+    return make_input_tensor_map(p, f3::in_pitch_for(radius), 64, tmap, use_tma);
+}
+
+template <int R>
+static int launch_r3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CUtensorMap& tmap, dim3 grid, bool use_tma) {
+    return use_tma ? launch_one3<R, true, 5, 64, false, false, true>(ctx, st, p, tmap, grid)
+                   : launch_one3<R, false, 5, 64, false, false, true>(ctx, st, p, tmap, grid);
+}
+
+int launch_front3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, int n_items, bool use_tma) {
+    if (n_items <= 0) return B200_OK;
+    FrontParams p = p_in;
+    p.div_c = ctx->gauss.div_c;
+    CUtensorMap tmap;   // unused: every frame's map is in the chunk's table
+    memset(&tmap, 0, sizeof(tmap));
+    const dim3 grid(n_items);
+    ctx->front_fast++;
+    switch (p.radius) {
+        case 2: return launch_r3_ragged<2>(ctx, st, p, tmap, grid, use_tma);
+        case 3: return launch_r3_ragged<3>(ctx, st, p, tmap, grid, use_tma);
+        case 5: return launch_r3_ragged<5>(ctx, st, p, tmap, grid, use_tma);
+        case 6: return launch_r3_ragged<6>(ctx, st, p, tmap, grid, use_tma);
+        case 9: return launch_r3_ragged<9>(ctx, st, p, tmap, grid, use_tma);
+        case 15: return launch_r3_ragged<15>(ctx, st, p, tmap, grid, use_tma);
+        default: break;
+    }
+    set_error("front3 kernel not built for radius %d", p.radius);
+    return B200_ERR_UNSUPPORTED;
 }
 
 int launch_front3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in) {

@@ -19,12 +19,17 @@
 //     ccl_sparse_link     one thread per weak pixel: strong neighbour -> SUPER, unions with its forward weak neighbours; the
 //                         last block applies the one-way link and retires the list's counters (HystParams::ctr)
 //     ccl_sparse_resolve  every weak pixel chases its root and becomes 0 or 255
+//     ragged chunks (frames of different sizes, b200_canny_frames_device) always take the list-driven pair, in a form that finds
+//     each entry's frame in the chunk's table (ccl_ragged_link / ccl_ragged_resolve); the tile-based family below serves uniform
+//     batches only
 //   tile-based (stage API, minVal <= 0, maps with more than 1/8 weak pixels):
 //     ccl_local   one CTA per 64x64 tile: union-find in shared memory (atomicMin links, row-run seeding
 //                 with warp ballots), then writes each candidate's parent (its tile root, or SUPER).
 //     ccl_merge   one thread per pixel on a tile boundary: lock-free atomicMin unions in global memory.
 //     ccl_final   every weak pixel chases its root; rewrites the class map to 0 / 255 in place.
 #include <string.h>
+
+#include <algorithm>
 
 #include "ccl.cuh"
 #include "internal.h"
@@ -488,6 +493,106 @@ int launch_ccl_resolve(b200_ctx* ctx, cudaStream_t st, const HystParams& p_in) {
 int launch_hysteresis(b200_ctx* ctx, cudaStream_t st, const HystParams& p) {
     CB_TRY(launch_ccl_label(ctx, st, p));
     return launch_ccl_resolve(ctx, st, p);
+}
+
+// ---------------------------------------------------------------------------------------------
+// ragged chunks: the list-driven kernels over frames of different sizes (b200_canny_frames_device)
+// ---------------------------------------------------------------------------------------------
+// A list entry g is a launch-relative slot; its frame is the last one whose base is <= g (binary search in the dense base table,
+// which stays in L1), and the frame gives W, H and the class-byte address.  Same unions, same neighbour rules, per frame.  Ragged
+// chunks always take these kernels, never the tile-based ones: the list holds every weak pixel at any density (every pixel at
+// worst, which also covers minVal <= 0), so they are correct everywhere, and the uniform path's density state is left alone.
+__device__ __forceinline__ int ragged_frame_of(const RaggedHystParams& p, unsigned int g) {
+    int lo = 0, hi = p.n_frames - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(p.bases + mid) <= g) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(256)
+ccl_ragged_link_kernel(const RaggedHystParams p) {
+    const unsigned int n = p.ctr[0];
+    for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const unsigned int g = p.list[i];
+        const RaggedFrame fd = p.frames[ragged_frame_of(p, g)];
+        const int W = fd.width, Hh = fd.height;
+        const unsigned int rel = g - (unsigned int)fd.base;
+        const int y = (int)(rel / (unsigned int)W), x = (int)(rel - (unsigned int)y * (unsigned int)W);
+        const long long cp = fd.cls_pitch;
+        const uint8_t* c = fd.cls + ((long long)y * cp + x);
+        const bool has_n = y > 0, has_s = y + 1 < Hh, has_w = x > 0, has_e = x + 1 < W;
+        const bool q01 = (y == 0) && (x == 1);   // (0,1): its SW neighbour (1,0) is off limits
+        const bool q10 = (y == 1) && (x == 0);   // (1,0): its NE neighbour (0,1) is off limits
+        const int c_nw = (has_n && has_w) ? c[-cp - 1] : 0;
+        const int c_n = has_n ? c[-cp] : 0;
+        const int c_ne = (has_n && has_e && !q10) ? c[-cp + 1] : 0;
+        const int c_w = has_w ? c[-1] : 0;
+        const int c_e = has_e ? c[1] : 0;
+        const int c_sw = (has_s && has_w && !q01) ? c[cp - 1] : 0;
+        const int c_s = has_s ? c[cp] : 0;
+        const int c_se = (has_s && has_e) ? c[cp + 1] : 0;
+        if (((c_nw | c_n | c_ne | c_w | c_e | c_sw | c_s | c_se) & 0x80) != 0) g_union_halve(p.parent, (int)g, kSuper);
+        if (c_e == 1) g_union_halve(p.parent, (int)g, (int)g + 1);
+        if (c_s == 1) {
+            g_union_halve(p.parent, (int)g, (int)g + W);
+        } else {
+            if (c_sw == 1) g_union_halve(p.parent, (int)g, (int)g + W - 1);
+            if (c_se == 1) g_union_halve(p.parent, (int)g, (int)g + W + 1);
+        }
+    }
+    // the last block applies the reference's one-way link (0,1) -> (1,0) of every frame (see ccl_sparse_link_kernel)
+    __shared__ bool s_last;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        s_last = atomicAdd(p.ctr + 1, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    for (int f = threadIdx.x; f < p.n_frames; f += blockDim.x) {
+        const RaggedFrame fd = p.frames[f];
+        const int c01 = fd.cls[1], c10 = fd.cls[fd.cls_pitch];
+        if (c10 == 1 && (c01 == 255 || (c01 == 1 && g_find_halve(p.parent, fd.base + 1) == kSuper)))
+            g_union_halve(p.parent, fd.base + fd.width, kSuper);
+    }
+    if (threadIdx.x == 0) {
+        p.ctr[2] = n;
+        p.ctr[0] = 0;
+        p.ctr[1] = 0;
+    }
+}
+
+__global__ void __launch_bounds__(256)
+ccl_ragged_resolve_kernel(const RaggedHystParams p) {
+    const unsigned int n = p.ctr[2];
+    for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const unsigned int g = p.list[i];
+        const RaggedFrame fd = p.frames[ragged_frame_of(p, g)];
+        const unsigned int rel = g - (unsigned int)fd.base;
+        const unsigned int y = rel / (unsigned int)fd.width, x = rel - y * (unsigned int)fd.width;
+        fd.cls[(long long)y * fd.cls_pitch + x] = (g_find_halve(p.parent, (int)g) == kSuper) ? 255 : 0;
+    }
+}
+
+int launch_hysteresis_ragged(b200_ctx* ctx, cudaStream_t st, const RaggedHystParams& p) {
+    const long long cap = 8LL * (ctx->sm_count > 0 ? ctx->sm_count : 148);
+    const int grid = (int)std::min(cap, std::max(32LL, p.px / 16384));   // as sparse_grid()
+    {
+        ProfScope ps(ctx, st, 1);
+        ccl_ragged_link_kernel<<<grid, 256, 0, st>>>(p);
+    }
+    CB_CUDA(cudaGetLastError());
+    ctx->launches++;
+    {
+        ProfScope ps(ctx, st, 3);
+        ccl_ragged_resolve_kernel<<<grid, 256, 0, st>>>(p);
+    }
+    CB_CUDA(cudaGetLastError());
+    ctx->launches++;
+    return B200_OK;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -89,6 +89,44 @@ struct FrontParams {
                             // frame*out_frame_stride + (y - plane_row0)*width + x (strong pixels need no slot: they are final)
     uint32_t* kept_list;    // launch-relative indices of all weak pixels, in no particular order
     unsigned int* kept_count;  // number of entries: word 0 of the list's counter block (see HystParams::ctr); zero at launch
+    // ragged launches (front3's RAGGED variant, b200_canny_frames_device): the chunk's device table.  Work item blockIdx.x names a
+    // frame, a strip and a row band; the frame's descriptor replaces in / in_pitch / width / height / cls / cls_pitch / cls_words
+    // and the slot base, and its tensor map (TMA staging) replaces the `tmap` parameter.
+    const struct RaggedFrame* rframes;
+    const struct RaggedItem* ritems;
+    const CUtensorMap_st* rtmaps;
+};
+
+// ---- ragged chunks: frames of different sizes in one launch --------------------------------------
+// One frame of a chunk as the kernels see it.  Frames are whole images (row 0 is the image's row 0).  Union-find slots and list
+// indices stay dense and launch-relative: pixel (y, x) of the frame is slot base + y*width + x, base being the sum of h*w over
+// the frames before it in the chunk (ascending, below 2^31).
+struct RaggedFrame {
+    const uint8_t* in;      // gray input (a scratch plane for B,G,R lists)
+    long long in_pitch;
+    uint8_t* cls;           // the caller's output: class map, then 0 / 255
+    long long cls_pitch;
+    int height, width;
+    int base;
+    int cls_words;          // cls and cls_pitch are multiples of 4 (aligned 32-bit class stores)
+};
+struct RaggedItem { int frame, x0, yb, ye; };   // one front CTA: strip at column x0, class rows [yb, ye) of the frame
+// B,G,R -> gray of one frame of a ragged chunk: rows [row0, row0 + height) of the chunk's row space
+struct RaggedGrayJob {
+    const uint8_t* bgr;
+    long long bgr_pitch;
+    uint8_t* gray;
+    long long gray_pitch;
+    int row0, width;
+};
+struct RaggedHystParams {
+    const RaggedFrame* frames;
+    const uint32_t* bases;  // frames[i].base, a dense copy for the per-entry binary search (stays in L1)
+    int n_frames;
+    int32_t* parent;
+    const uint32_t* list;
+    unsigned int* ctr;      // the list's counter block (HystParams::ctr); h_kept is never written by ragged launches
+    long long px;           // pixels of the chunk (sizes the grid)
 };
 
 // The input layout a TMA tensor map can describe: base, row pitch and frame stride on 16-byte boundaries, frames that do not
@@ -210,6 +248,11 @@ struct b200_ctx {
     unsigned int* d_kept = nullptr;       // device-side address of h_kept
     bool list_dirty[4] = {false, false, false, false};   // a launch on this slot failed between front and link: re-zero its counters
     long long kept_px[4] = {0, 0, 0, 0};
+    // ragged chunks (b200_canny_frames_device): the chunk's table (descriptors, tensor maps, work items) is built in pinned
+    // staging per slot and sent up with one copy; the host rewrites the staging only after ev_ragged[slot] (recorded behind it)
+    cb::Workspace ws_ragged[3], host_ragged[3];
+    cudaEvent_t ev_ragged[3] = {nullptr, nullptr, nullptr};
+    bool ragged_busy[3] = {false, false, false};
 };
 
 namespace cb {
@@ -246,12 +289,19 @@ int launch_front2(b200_ctx* ctx, cudaStream_t st, const FrontParams& p);
 bool front3_supports(int radius);
 bool front3_bgr_supports(const FrontParams& p);   // p.in / width / in_frame_stride / radius allow the fused BGR -> gray staging
 int launch_front3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p);
+// ragged chunks: class-row band height shared by the chunk's frames (the policy is described at its definition), the work items
+// of one frame, and the launch over n_items items of p.ritems (all TMA-staged or all byte-staged)
+int ragged_band_rows3(const b200_ctx* ctx, const int* heights, const int* widths, int n, int radius);
+void ragged_items3(int frame, int height, int width, int band_rows, std::vector<RaggedItem>& items);
+int ragged_tensor_map3(const uint8_t* in, long long pitch, int height, int width, int radius, CUtensorMap_st* tmap, bool* use_tma);
+int launch_front3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, bool use_tma);
 // selftest.cu
 int check_div_mode_device(b200_ctx* ctx, float b, float y, float* c, int* mode);
 // hysteresis.cu
 int launch_hysteresis(b200_ctx* ctx, cudaStream_t st, const HystParams& p);   // label + resolve
 int launch_ccl_label(b200_ctx* ctx, cudaStream_t st, const HystParams& p);    // tile-local forest + tile-boundary unions
 int launch_ccl_resolve(b200_ctx* ctx, cudaStream_t st, const HystParams& p);  // weak pixels -> 0/255 in place
+int launch_hysteresis_ragged(b200_ctx* ctx, cudaStream_t st, const RaggedHystParams& p);   // list-driven link + resolve
 int launch_classify_i16(b200_ctx* ctx, cudaStream_t st, const int16_t* nms, uint8_t* cls, size_t n,
                         int lo, int hi);
 int launch_expand_u8_to_i16(b200_ctx* ctx, cudaStream_t st, const uint8_t* cls, int16_t* out, size_t n);
@@ -267,6 +317,8 @@ int launch_bgr_to_gray(b200_ctx* ctx, cudaStream_t st, const uint8_t* bgr, uint8
 // n_frames x h rows of w pixels from a pitched B,G,R source into a dense n_frames*h*w gray plane
 int launch_bgr_to_gray_strided(b200_ctx* ctx, cudaStream_t st, const uint8_t* bgr, long long pitch, long long frame_stride,
                                int n_frames, int h, int w, uint8_t* gray);
+// the frames of a ragged chunk (jobs: device table, ascending row0) into their gray scratch frames; rows: total rows
+int launch_bgr_to_gray_ragged(b200_ctx* ctx, cudaStream_t st, const RaggedGrayJob* jobs, int n_jobs, long long rows);
 // band.cu: one row band's local stages in pieces
 struct BandGeom {
     const uint8_t* d_rows;   // global row (row0 - above) of the band buffer

@@ -188,4 +188,31 @@ int launch_bgr_to_gray_strided(b200_ctx* ctx, cudaStream_t st, const uint8_t* bg
     return B200_OK;
 }
 
+// The same conversion for the frames of a ragged chunk, driven by the chunk's job table: block-rows walk the chunk's row space,
+// and row r belongs to the last job whose row0 is <= r (binary search).
+__global__ void bgr_to_gray_ragged_kernel(const RaggedGrayJob* __restrict__ jobs, int n_jobs, long long rows) {
+    for (long long r = blockIdx.x; r < rows; r += gridDim.x) {
+        int lo = 0, hi = n_jobs - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (jobs[mid].row0 <= r) lo = mid; else hi = mid - 1;
+        }
+        const RaggedGrayJob j = jobs[lo];
+        const long long y = r - j.row0;
+        const uint8_t* src = j.bgr + y * j.bgr_pitch;
+        uint8_t* dst = j.gray + y * j.gray_pitch;
+        for (int x = threadIdx.x; x < j.width; x += blockDim.x)
+            dst[x] = (uint8_t)gray_of(__ldcs(src + 3 * x), __ldcs(src + 3 * x + 1), __ldcs(src + 3 * x + 2));
+    }
+}
+
+int launch_bgr_to_gray_ragged(b200_ctx* ctx, cudaStream_t st, const RaggedGrayJob* jobs, int n_jobs, long long rows) {
+    const long long cap = 32LL * (ctx->sm_count > 0 ? ctx->sm_count : 148);
+    const int blocks = (int)std::max<long long>(1, std::min(rows, cap));
+    bgr_to_gray_ragged_kernel<<<blocks, 256, 0, st>>>(jobs, n_jobs, rows);
+    CB_CUDA(cudaGetLastError());
+    ctx->launches++;
+    return B200_OK;
+}
+
 }  // namespace cb

@@ -3,7 +3,8 @@
 Any view whose rows are contiguous goes straight to the kernels with its strides — a crop `x[:, y0:y1, x0:x1]`, one channel of an
 `(N, C, H, W)` tensor, frames padded for alignment — through b200_canny_batch_device_strided; nothing is copied.  Layouts the
 kernels cannot address (rows that are not unit-stride, frames that overlap, broadcast frames) raise ValueError rather than being
-copied behind the caller's back.
+copied behind the caller's back.  canny_list / canny_bgr_list take a list of frames of different sizes in one call
+(b200_canny_frames_device).
 
 Work is issued on torch.cuda.current_stream(frames.device): the context is pointed at that stream on every call, so results are
 ordered with the caller's other torch work like any torch op.  When consecutive calls come from different streams, the later
@@ -14,7 +15,7 @@ from __future__ import annotations
 import threading
 from typing import Dict, Optional, Tuple
 
-from .api import Context, canny_batch_device_bgr_strided_ptr, canny_batch_device_strided_ptr
+from .api import Context, canny_batch_device_bgr_strided_ptr, canny_batch_device_strided_ptr, canny_frames_device_ptr
 
 _contexts: Dict[int, Context] = {}
 _contexts_lock = threading.Lock()
@@ -116,3 +117,60 @@ def canny_bgr(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx
     """canny() for interleaved B,G,R frames (cv2 / cv::Mat layout): (H, W, 3) or (N, H, W, 3), each pixel's 3 bytes contiguous,
     rows and frames with any stride.  The gray conversion is OpenCV's COLOR_BGR2GRAY, bit for bit.  Returns (H, W) or (N, H, W)."""
     return _run(frames, sigma, min_val, max_val, out, ctx, bgr=True)
+
+
+def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool):
+    import torch
+
+    frames = list(frames)
+    if not frames:
+        raise ValueError("empty frame list")
+    single = 3 if bgr else 2   # one frame per element: (H, W) gray, (H, W, 3) B,G,R
+    descs = []
+    for i, f in enumerate(frames):
+        if isinstance(f, torch.Tensor) and f.dim() != single:
+            raise ValueError(f"frame {i}: expected one {'(H, W, 3) B,G,R' if bgr else '(H, W) gray'} frame, got shape {tuple(f.shape)}")
+        _, h, w, pitch, _ = frame_layout(f, bgr)
+        descs.append([f.data_ptr(), pitch, 0, 0, h, w])
+    if out is not None:
+        out = list(out)
+        if len(out) != len(frames):
+            raise ValueError(f"out has {len(out)} tensors for {len(frames)} frames")
+        for i, (o, d) in enumerate(zip(out, descs)):
+            if not isinstance(o, torch.Tensor) or tuple(o.shape) != (d[4], d[5]):
+                raise ValueError(f"out[{i}] has shape {tuple(getattr(o, 'shape', ()))}, expected {(d[4], d[5])}")
+    device = frames[0].device
+    for i, t in enumerate(frames + (out or [])):
+        name = f"frame {i}" if i < len(frames) else f"out[{i - len(frames)}]"
+        if not t.is_cuda:
+            raise ValueError(f"{name} must be a CUDA tensor (got device {t.device})")
+        if t.device != device:
+            raise ValueError(f"{name} is on {t.device}, frame 0 on {device}: all tensors must be on one device")
+    if out is None:
+        out = [torch.empty((d[4], d[5]), dtype=torch.uint8, device=device) for d in descs]
+    for d, o in zip(descs, out):
+        _, _, _, d[3], _ = frame_layout(o, False)
+        d[2] = o.data_ptr()
+    dev = device.index if device.index is not None else torch.cuda.current_device()
+    if ctx is None:
+        ctx = _context(dev)
+    elif ctx.device != dev:
+        raise ValueError(f"context is on cuda:{ctx.device}, frames on cuda:{dev}")
+    with _call_lock, torch.cuda.device(dev):
+        ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)
+        canny_frames_device_ptr(ctx, descs, sigma, min_val, max_val, bgr=bgr)
+    return out
+
+
+def canny_list(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx: Optional[Context] = None):
+    """Canny edge maps of a list of gray frames of different sizes, in one call (b200_canny_frames_device): each element a CUDA
+    uint8 (H, W) view whose rows are contiguous, any row pitch.  Returns a list of uint8 (H, W) tensors holding 0 / 255 (`out` when
+    given: a list of views of the same shapes, e.g. regions of one mosaic; only their elements are written).  Every map equals
+    canny() of that frame alone.  Asynchronous on torch.cuda.current_stream(device); ctx defaults to the cached Context."""
+    return _run_list(frames, sigma, min_val, max_val, out, ctx, bgr=False)
+
+
+def canny_bgr_list(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx: Optional[Context] = None):
+    """canny_list() for interleaved B,G,R frames: each element an (H, W, 3) view with each pixel's 3 bytes contiguous.  The gray
+    conversion is OpenCV's COLOR_BGR2GRAY, bit for bit.  Returns a list of (H, W) maps."""
+    return _run_list(frames, sigma, min_val, max_val, out, ctx, bgr=True)

@@ -213,6 +213,29 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
                                         int n_frames, int height, int width, float sigma, int min_val, int max_val,
                                         uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
 
+/* A list of frames of DIFFERENT sizes and layouts in one call: dataset images, camera streams of several resolutions, crops of
+ * detections, a list of cv::cuda::GpuMat.  Each frame has its own size, input pointer and row pitch and its own output pointer
+ * and row pitch; sigma and the thresholds are shared.  Frame i's map is the one b200_canny_batch_device_strided gives for that
+ * frame alone, bit for bit.
+ *   pixel (y, x) of frame i is read from in + y*in_row_pitch + x (gray) or from the 3 bytes at in + y*in_row_pitch + 3*x
+ *   (B, G, R), and its 0 / 255 result is written to out + y*out_row_pitch + x.  No other output byte is written, so the outputs
+ *   may be regions of one larger image (a mosaic whose tiles sit in rows of their own: extents may not overlap, see below).
+ * `frames` is host memory, read only during the call.  Work is asynchronous on the context's stream.  The list is cut, in call
+ * order, into chunks of about 75 Mpix (b200_ctx_set_chunk_frames caps the frames per chunk); a larger frame has a chunk of its own.
+ * B200_ERR_INVALID_ARG, before any device work: a null `frames`, `in` or `out`; n_frames <= 0; a frame smaller than 2 x 2; a
+ * negative pitch or one below a row (width, 3*width for BGR); an extent ((height-1)*pitch + row bytes) above 2^48 bytes; an
+ * output extent that overlaps any input extent or any other output extent.  Inputs may overlap each other (the same frame may be
+ * listed twice).  A frame of 2^31 pixels or more: B200_ERR_UNSUPPORTED. */
+typedef struct b200_frame {
+    const uint8_t* in;        /* device; gray: 1 byte per pixel, BGR: 3 (B,G,R) */
+    int64_t in_row_pitch;     /* bytes */
+    uint8_t* out;             /* device; 0 / 255 bytes */
+    int64_t out_row_pitch;    /* bytes */
+    int32_t height, width;
+} b200_frame;
+int b200_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val);
+int b200_canny_frames_device_bgr(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val);
+
 /* The packed form of an edge map — 1 bit per pixel, bit i of byte k <-> pixel 8k+i, ceil(n_px/32)*4 bytes — is what
  * b200_canny_batch_host moves over PCIe.  Both halves are exported for callers that store or ship maps in that form:
  *   b200_pack_edges_device   0 / 255 bytes in DEVICE memory -> packed words in DEVICE memory, asynchronous on the context's

@@ -223,6 +223,17 @@ def canny_batch_device_bgr_strided_ptr(ctx: Optional[Context], d_bgr: int, in_ro
                                                      int(out_row_pitch), int(out_frame_stride)))
 
 
+def cv_canny_device_strided_ptr(ctx: Optional[Context], d_in: int, in_row_pitch: int, in_frame_stride: int, n: int, h: int, w: int,
+                                channels: int, threshold1: float, threshold2: float, l2_gradient: bool, d_edges: int,
+                                out_row_pitch: int, out_frame_stride: int) -> None:
+    """cv2.Canny(frame, threshold1, threshold2, L2gradient=l2_gradient) of every frame, bit for bit (b200_cv_canny_device_strided):
+    1 or 3 interleaved channels, pixel (f, y, x) read at d_in + f*in_frame_stride + y*in_row_pitch + channels*x, its 0 / 255
+    result written at d_edges + f*out_frame_stride + y*out_row_pitch + x.  Asynchronous on the context's stream."""
+    check(load().b200_cv_canny_device_strided(_h(ctx), C.c_void_p(d_in), int(in_row_pitch), int(in_frame_stride), n, h, w,
+                                              int(channels), C.c_double(threshold1), C.c_double(threshold2), int(bool(l2_gradient)),
+                                              C.c_void_p(d_edges), int(out_row_pitch), int(out_frame_stride)))
+
+
 def frame_list(descs) -> C.Array:
     """(in_ptr, in_pitch, out_ptr, out_pitch, h, w) tuples -> the ctypes array of b200_frame that b200_canny_frames_device takes."""
     descs = list(descs)

@@ -303,9 +303,10 @@ static int resolve_ctx(b200_ctx*& ctx) {
     return B200_OK;
 }
 
-static int check_image(const void* in, const void* out, int h, int w) {
+// min_side: 2 for the reference's semantics, 1 for the OpenCV-compatible path (cv::Canny takes any image of at least one pixel)
+static int check_image(const void* in, const void* out, int h, int w, int min_side = 2) {
     if (!in || !out) { set_error("null image pointer"); return B200_ERR_INVALID_ARG; }
-    if (h < 2 || w < 2) { set_error("height and width must be >= 2 (got %dx%d)", h, w); return B200_ERR_INVALID_ARG; }
+    if (h < min_side || w < min_side) { set_error("height and width must be >= %d (got %dx%d)", min_side, h, w); return B200_ERR_INVALID_ARG; }
     if ((long long)h * w >= (1LL << 31)) { set_error("image of %dx%d pixels exceeds int indexing", h, w); return B200_ERR_UNSUPPORTED; }
     return B200_OK;
 }
@@ -390,6 +391,48 @@ static bool bgr_fused_ok(const b200_ctx* ctx, const uint8_t* d_bgr, int n, int h
     fp.in = d_bgr; fp.in_pitch = pitch; fp.in_frame_stride = frame_stride; fp.n_frames = n; fp.in_rows = h; fp.width = w;
     fp.radius = ctx->gauss.radius;
     return force == 0 && !ctx->gauss.tiny && front3_bgr_supports(fp);
+}
+
+// The OpenCV-compatible path (b200_cv_canny_device_strided): cv::Canny's thresholds as integers in magnitude space (swapped,
+// clamped and squared for L2, floored) and the input's channel count
+struct CvSpec {
+    int lo, hi;
+    int channels;
+    bool l2;
+};
+
+// Front + hysteresis with cv::Canny's semantics on frames [f0, f0+nf) of slot `slot` (run_frames_device's counterpart): the
+// OpenCV front kernel, then always the list-driven hysteresis kernels with plain 8-connectivity.  The uniform path's density state
+// (h_kept, kept_px) is neither read nor written.
+static int run_frames_cv(b200_ctx* ctx, cudaStream_t st, int slot, const uint8_t* d_in, uint8_t* d_out, int nf, int h, int w,
+                         const CvSpec& cv, const FrameLayout& lay) {
+    const long long px = (long long)h * w;
+    FrontParams fp;
+    memset(&fp, 0, sizeof(fp));
+    fp.in = d_in; fp.in_pitch = lay.in_pitch; fp.in_frame_stride = lay.in_frame_stride; fp.in_bgr = 0;
+    fp.in_rows = h; fp.width = w; fp.height = h; fp.out_rows = h; fp.n_frames = nf; fp.out_frame_stride = px;
+    fp.cls = d_out; fp.cls_pitch = lay.out_pitch; fp.cls_frame_stride = lay.out_frame_stride;
+    fp.lo = cv.lo; fp.hi = cv.hi;
+    fp.parent = reinterpret_cast<int32_t*>(ctx->ws_parent[slot].ptr);
+    fp.kept_count = reinterpret_cast<unsigned int*>(ctx->ws_list[slot].ptr);
+    fp.kept_list = reinterpret_cast<uint32_t*>(ctx->ws_list[slot].ptr) + 16;
+    // the list's counter block is zero here (see run_frames_device)
+    if (ctx->list_dirty[slot]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
+    ctx->list_dirty[slot] = true;
+    CB_TRY(launch_front_cv(ctx, st, fp, cv.channels, cv.l2));
+    HystParams hp;
+    memset(&hp, 0, sizeof(hp));
+    hp.cls = d_out; hp.cls_pitch = lay.out_pitch; hp.cls_frame_stride = lay.out_frame_stride;
+    hp.list = fp.kept_list; hp.ctr = fp.kept_count;
+    hp.parent = fp.parent;
+    hp.frame_stride = px; hp.rows = h; hp.width = w; hp.row0 = 0; hp.n_frames = nf;
+    hp.opencv = 1;
+    static const int pdl_env = [] { const char* e = getenv("B200_CANNY_PDL"); return e ? atoi(e) : -1; }();
+    hp.pdl = pdl_env >= 0 ? pdl_env : ((long long)nf * px <= (4LL << 20) ? 1 : 0);   // as run_frames_device
+    if (ctx->prof.on) hp.pdl = 0;
+    CB_TRY(launch_hysteresis(ctx, st, hp));
+    ctx->list_dirty[slot] = false;
+    return B200_OK;
 }
 
 // bytes of the weak-pixel list for nf frames of h x w: a counter block + one 32-bit entry per pixel (worst case: all weak)
@@ -815,8 +858,8 @@ int b200_canny_bgr(b200_ctx* ctx, const uint8_t* bgr, float sigma, int lo, int h
 // ---- batched --------------------------------------------------------------------------------------------
 // Argument checks of a strided device batch; all of them run before any device work.  bpp: bytes per input pixel.
 static int check_strided(const uint8_t* in, long long in_pitch, long long in_fs, int n, int h, int w, const uint8_t* out,
-                         long long out_pitch, long long out_fs, int bpp) {
-    CB_TRY(check_image(in, out, h, w));
+                         long long out_pitch, long long out_fs, int bpp, int min_side = 2) {
+    CB_TRY(check_image(in, out, h, w, min_side));
     if (n <= 0) { set_error("n_frames must be positive"); return B200_ERR_INVALID_ARG; }
     if (in_pitch < 0 || in_fs < 0 || out_pitch < 0 || out_fs < 0) {
         set_error("negative stride (in: pitch %lld, frame %lld; out: pitch %lld, frame %lld)", in_pitch, in_fs, out_pitch, out_fs);
@@ -845,12 +888,15 @@ static int check_strided(const uint8_t* in, long long in_pitch, long long in_fs,
 // bpp: bytes per input pixel — 1 gray, 3 interleaved B,G,R (converted by the front kernel while staging when it can, else chunk by
 // chunk into a gray scratch plane first).  Strides in bytes (b200_canny_batch_device_strided); the dense entry points pass
 // pitch = bpp*width and frame stride = height*pitch.
+// cv: the OpenCV-compatible path (b200_cv_canny_device_strided; its thresholds are checked by the caller, sigma, lo and hi are
+// unused): the same chunks, slots and workspace, each chunk through run_frames_cv.  Null: the reference's semantics.
 static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, long long in_pitch, long long in_fs, int n_frames, int h, int w,
-                             float sigma, int lo, int hi, uint8_t* d_edges, long long out_pitch, long long out_fs, int bpp) {
-    CB_TRY(check_strided(d_frames, in_pitch, in_fs, n_frames, h, w, d_edges, out_pitch, out_fs, bpp));
-    CB_TRY(check_thresholds(lo, hi));
+                             float sigma, int lo, int hi, uint8_t* d_edges, long long out_pitch, long long out_fs, int bpp,
+                             const CvSpec* cv = nullptr) {
+    CB_TRY(check_strided(d_frames, in_pitch, in_fs, n_frames, h, w, d_edges, out_pitch, out_fs, bpp, cv ? 1 : 2));
+    if (!cv) CB_TRY(check_thresholds(lo, hi));
     CB_TRY(resolve_ctx(ctx));
-    CB_TRY(prepare_gauss(ctx, sigma));
+    if (!cv) CB_TRY(prepare_gauss(ctx, sigma));
     // a single frame's stride is never used: make it the one that keeps the tensor map and the word stores eligible
     if (n_frames == 1) { in_fs = (long long)h * in_pitch; out_fs = (long long)h * out_pitch; }
     const FrameLayout lay = {in_pitch, in_fs, out_pitch, out_fs};
@@ -862,7 +908,7 @@ static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, long long i
     // waiting (same slot) for those hysteresis kernels (226 against 219 Gpix/s with two slots; running the hysteresis kernels on
     // high-priority streams on top of that measured 222)
     const int n_slots = std::min(3, n_chunks);
-    const bool bgr = bpp == 3;
+    const bool bgr = bpp == 3 && !cv;   // the OpenCV kernel reads 3-channel frames itself
     const bool fused = bgr && bgr_fused_ok(ctx, d_frames, std::min(chunk, n_frames), h, w, in_pitch, in_fs);
     const bool bgr_dense = in_pitch == 3LL * w && in_fs == 3 * px;
     for (int s = 0; s < n_slots; ++s) {
@@ -872,6 +918,7 @@ static int batch_device_impl(b200_ctx* ctx, const uint8_t* d_frames, long long i
     }
     auto run_chunk = [&](cudaStream_t st, int s, int f0, int nf) -> int {
         const uint8_t* src = d_frames + (long long)f0 * in_fs;
+        if (cv) return run_frames_cv(ctx, st, s, src, d_edges + (long long)f0 * out_fs, nf, h, w, *cv, lay);
         FrameLayout cl = lay;
         if (bgr && !fused) {
             // the gray scratch plane is dense whatever the B,G,R frames' strides
@@ -931,6 +978,43 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
                                         int64_t out_row_pitch, int64_t out_frame_stride) {
     return batch_device_impl(ctx, d_bgr, in_row_pitch, in_frame_stride, n_frames, h, w, sigma, lo, hi, d_edges, out_row_pitch,
                              out_frame_stride, 3);
+}
+
+// ---- cv::Canny semantics ----------------------------------------------------------------------------------
+// Thresholds as cv::Canny uses them (imgproc/src/canny.cpp): swapped when low > high; for L2 clamped to 32767 and squared when
+// positive; floored.  NaN / inf: B200_ERR_INVALID_ARG.  A floor outside int32: B200_ERR_UNSUPPORTED (OpenCV's cvFloor overflows
+// there and its result is not the comparison the thresholds describe).
+constexpr int kCvMaxHeight = 65535 * 64;   // the OpenCV front kernel's grid: one row of CTAs per 64 rows, gridDim.y <= 65535
+
+static int cv_thresholds(double t1, double t2, bool l2, int* lo, int* hi) {
+    if (!isfinite(t1) || !isfinite(t2)) { set_error("thresholds must be finite (got %g, %g)", t1, t2); return B200_ERR_INVALID_ARG; }
+    double a = std::min(t1, t2), b = std::max(t1, t2);
+    if (l2) {
+        a = std::min(32767.0, a); b = std::min(32767.0, b);
+        if (a > 0) a *= a;
+        if (b > 0) b *= b;
+    }
+    a = floor(a); b = floor(b);
+    const double kMin = -2147483648.0, kMax = 2147483647.0;
+    if (a < kMin || a > kMax || b < kMin || b > kMax) {
+        set_error("thresholds %g, %g: their floor does not fit in int32", t1, t2);
+        return B200_ERR_UNSUPPORTED;
+    }
+    *lo = (int)a; *hi = (int)b;
+    return B200_OK;
+}
+
+int b200_cv_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride, int n_frames,
+                                 int height, int width, int channels, double threshold1, double threshold2, int l2_gradient,
+                                 uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride) {
+    if (channels != 1 && channels != 3) { set_error("channels must be 1 or 3 (got %d)", channels); return B200_ERR_UNSUPPORTED; }
+    if (height > kCvMaxHeight) { set_error("height %d: at most %d rows (65535 tiles of 64)", height, kCvMaxHeight); return B200_ERR_UNSUPPORTED; }
+    CvSpec cv;
+    cv.channels = channels;
+    cv.l2 = l2_gradient != 0;
+    CB_TRY(cv_thresholds(threshold1, threshold2, cv.l2, &cv.lo, &cv.hi));
+    return batch_device_impl(ctx, d_in, in_row_pitch, in_frame_stride, n_frames, height, width, 0.f, 0, 0, d_edges, out_row_pitch,
+                             out_frame_stride, channels, &cv);
 }
 
 // ---- ragged lists: frames of different sizes in one call ------------------------------------------------

@@ -22,7 +22,9 @@
 //     ragged chunks (frames of different sizes, b200_canny_frames_device) always take the list-driven pair, in a form that finds
 //     each entry's frame in the chunk's table (ccl_ragged_link / ccl_ragged_resolve); the tile-based family below serves uniform
 //     batches only
-//   tile-based (stage API, minVal <= 0, maps with more than 1/8 weak pixels):
+//     launches of the OpenCV-compatible path (HystParams::opencv) take the list-driven pair too, with plain 8-connectivity: no pair
+//     is left out and no one-way link is applied
+//   tile-based (stage API, minVal <= 0, maps with more than 1/8 weak pixels; reference semantics only):
 //     ccl_local   one CTA per 64x64 tile: union-find in shared memory (atomicMin links, row-run seeding
 //                 with warp ballots), then writes each candidate's parent (its tile root, or SUPER).
 //     ccl_merge   one thread per pixel on a tile boundary: lock-free atomicMin unions in global memory.
@@ -304,6 +306,9 @@ __device__ __forceinline__ long long cls_index(const HystParams& p, unsigned int
     return (long long)f * p.cls_frame_stride + (long long)y * p.cls_pitch + x;
 }
 
+// OPENCV: cv::Canny's plain 8-connectivity (b200_cv_canny_device_strided) — the pair (0,1)-(1,0) is linked like any other and the
+// last block applies no one-way link; it only retires the counters.
+template <bool OPENCV>
 __global__ void __launch_bounds__(256)
 ccl_sparse_link_kernel(const HystParams p) {
     pdl_launch_dependents();
@@ -320,7 +325,7 @@ ccl_sparse_link_kernel(const HystParams p) {
         const int y = (int)(rel / (unsigned int)W), x = (int)(rel - (unsigned int)y * (unsigned int)W);
         const uint8_t* c = p.cls + ((long long)f * p.cls_frame_stride + y * cp + x);
         const bool has_n = y > 0, has_s = y + 1 < Hh, has_w = x > 0, has_e = x + 1 < W;
-        const bool top_rows = (p.row0 + y) <= 1;
+        const bool top_rows = !OPENCV && (p.row0 + y) <= 1;
         const bool q01 = top_rows && (p.row0 + y == 0) && (x == 1);   // this pixel is (0,1): its SW neighbour (1,0) is off limits
         const bool q10 = top_rows && (p.row0 + y == 1) && (x == 0);   // this pixel is (1,0): its NE neighbour (0,1) is off limits
         const int c_nw = (has_n && has_w) ? c[-cp - 1] : 0;
@@ -353,7 +358,7 @@ ccl_sparse_link_kernel(const HystParams p) {
     __syncthreads();
     if (!s_last) return;
     __threadfence();
-    if (p.row0 == 0 && Hh >= 2 && W >= 2) {
+    if (!OPENCV && p.row0 == 0 && Hh >= 2 && W >= 2) {
         for (int f = threadIdx.x; f < p.n_frames; f += blockDim.x) {
             const unsigned int f0 = (unsigned int)f * fs;
             const uint8_t* cf = p.cls + (long long)f * p.cls_frame_stride;
@@ -430,11 +435,12 @@ int launch_ccl_label(b200_ctx* ctx, cudaStream_t st, const HystParams& p_in) {
     CB_TRY(check_hyst_params(p));
     if (p.list) {
         ProfScope ps(ctx, st, 1);
-        CB_CUDA(launch_list_kernel(ccl_sparse_link_kernel, sparse_grid(ctx, p), st, p));
+        CB_CUDA(launch_list_kernel(p.opencv ? ccl_sparse_link_kernel<true> : ccl_sparse_link_kernel<false>, sparse_grid(ctx, p), st, p));
         CB_CUDA(cudaGetLastError());
         ctx->launches++;
         return B200_OK;
     }
+    if (p.opencv) { set_error("internal: OpenCV hysteresis runs on the weak-pixel list only"); return B200_ERR_INVALID_ARG; }
     if (p.ctr) {
         list_retire_kernel<<<1, 1, 0, st>>>(p.ctr, p.h_kept, p.kept_prev, p.kept_thresh);
         ctx->launches++;

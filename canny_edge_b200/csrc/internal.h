@@ -186,6 +186,8 @@ struct HystParams {
     unsigned int kept_prev, kept_thresh;   // ... but only when it moves across the threshold: the host's last view of it and the
                                            // "tile-based labelling above this many weak pixels" bound (a write to host memory at the
                                            // end of every launch measured 1 % of the batch throughput)
+    int opencv;                  // 1: cv::Canny's plain 8-connectivity, without the reference's one-way (0,1)/(1,0) link (list-driven
+                                 // kernels only; b200_cv_canny_device_strided)
 };
 
 struct HostPool;  // api.cu
@@ -295,6 +297,9 @@ int ragged_band_rows3(const b200_ctx* ctx, const int* heights, const int* widths
 void ragged_items3(int frame, int height, int width, int band_rows, std::vector<RaggedItem>& items);
 int ragged_tensor_map3(const uint8_t* in, long long pitch, int height, int width, int radius, CUtensorMap_st* tmap, bool* use_tma);
 int launch_front3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, bool use_tma);
+// front_cv.cu (cv::Canny semantics, b200_cv_canny_device_strided): class map + weak-pixel list of p's frames, channels 1 or 3
+// interleaved, L1 or L2 magnitude against p.lo / p.hi (already floored and, for L2, squared)
+int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int channels, bool l2);
 // selftest.cu
 int check_div_mode_device(b200_ctx* ctx, float b, float y, float* c, int* mode);
 // hysteresis.cu

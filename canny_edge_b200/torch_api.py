@@ -4,7 +4,8 @@ Any view whose rows are contiguous goes straight to the kernels with its strides
 `(N, C, H, W)` tensor, frames padded for alignment — through b200_canny_batch_device_strided; nothing is copied.  Layouts the
 kernels cannot address (rows that are not unit-stride, frames that overlap, broadcast frames) raise ValueError rather than being
 copied behind the caller's back.  canny_list / canny_bgr_list take a list of frames of different sizes in one call
-(b200_canny_frames_device).
+(b200_canny_frames_device).  cv_canny / cv_canny_color compute cv2.Canny's maps instead of the reference's
+(b200_cv_canny_device_strided), from the same kinds of views.
 
 Work is issued on torch.cuda.current_stream(frames.device): the context is pointed at that stream on every call, so results are
 ordered with the caller's other torch work like any torch op.  When consecutive calls come from different streams, the later
@@ -15,7 +16,8 @@ from __future__ import annotations
 import threading
 from typing import Dict, Optional, Tuple
 
-from .api import Context, canny_batch_device_bgr_strided_ptr, canny_batch_device_strided_ptr, canny_frames_device_ptr
+from .api import (Context, canny_batch_device_bgr_strided_ptr, canny_batch_device_strided_ptr, canny_frames_device_ptr,
+                  cv_canny_device_strided_ptr)
 
 _contexts: Dict[int, Context] = {}
 _contexts_lock = threading.Lock()
@@ -25,10 +27,11 @@ _CUDA_STREAM_LEGACY = 0x1   # cudaStreamLegacy (driver_types.h)
 _CONTIGUOUS_HINT = "pass a view whose rows are contiguous (e.g. call .contiguous() first)"
 
 
-def frame_layout(t, bgr: bool = False) -> Tuple[int, int, int, int, int]:
+def frame_layout(t, bgr: bool = False, min_side: int = 2) -> Tuple[int, int, int, int, int]:
     """(n_frames, height, width, row pitch, frame stride) of a uint8 tensor as the strided C calls take them, strides in bytes.
 
-    Gray: (H, W) or (N, H, W).  BGR: (H, W, 3) or (N, H, W, 3).  Raises ValueError for a layout the kernels cannot address."""
+    Gray: (H, W) or (N, H, W).  BGR: (H, W, 3) or (N, H, W, 3).  Raises ValueError for a layout the kernels cannot address, or for
+    frames smaller than min_side x min_side (2 for the reference's semantics, 1 for the OpenCV-compatible calls)."""
     import torch
 
     if not isinstance(t, torch.Tensor):
@@ -52,8 +55,8 @@ def frame_layout(t, bgr: bool = False) -> Tuple[int, int, int, int, int]:
     h, w = shape[-2], shape[-1]
     pitch = stride[-2]
     n = shape[0] if len(shape) == 3 else 1
-    if h < 2 or w < 2:
-        raise ValueError(f"frames must be at least 2 x 2 pixels (got {h} x {w})")
+    if h < min_side or w < min_side:
+        raise ValueError(f"frames must be at least {min_side} x {min_side} pixels (got {h} x {w})")
     if n < 1:
         raise ValueError("no frames")
     if pitch < row_bytes:
@@ -76,10 +79,13 @@ def _context(device_index: int) -> Context:
         return ctx
 
 
-def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool):
+def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool, cv_l2=None):
+    """cv_l2 None: the reference's Canny (sigma, min_val, max_val); False / True: cv2.Canny with L1 / L2 magnitude, min_val and
+    max_val being threshold1 and threshold2."""
     import torch
 
-    n, h, w, in_pitch, in_fs = frame_layout(frames, bgr)
+    min_side = 2 if cv_l2 is None else 1
+    n, h, w, in_pitch, in_fs = frame_layout(frames, bgr, min_side)
     out_shape = tuple(frames.shape[:-1]) if bgr else tuple(frames.shape)
     if not frames.is_cuda:
         raise ValueError(f"frames must be a CUDA tensor (got device {frames.device})")
@@ -90,7 +96,7 @@ def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Co
             raise ValueError(f"out has shape {tuple(out.shape)}, expected {out_shape}")
         if out.device != frames.device:
             raise ValueError(f"out is on {out.device}, frames on {frames.device}")
-    _, _, _, out_pitch, out_fs = frame_layout(out, False)
+    _, _, _, out_pitch, out_fs = frame_layout(out, False, min_side)
     dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
     if ctx is None:
         ctx = _context(dev)
@@ -100,8 +106,12 @@ def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Co
         # torch's default stream has the handle 0, which the library reads as "the context's own stream": name the legacy default
         # stream (cudaStreamLegacy) instead, so the work is ordered with the caller's
         ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)
-        call = canny_batch_device_bgr_strided_ptr if bgr else canny_batch_device_strided_ptr
-        call(ctx, frames.data_ptr(), in_pitch, in_fs, n, h, w, sigma, min_val, max_val, out.data_ptr(), out_pitch, out_fs)
+        if cv_l2 is not None:
+            cv_canny_device_strided_ptr(ctx, frames.data_ptr(), in_pitch, in_fs, n, h, w, 3 if bgr else 1, min_val, max_val, cv_l2,
+                                        out.data_ptr(), out_pitch, out_fs)
+        else:
+            call = canny_batch_device_bgr_strided_ptr if bgr else canny_batch_device_strided_ptr
+            call(ctx, frames.data_ptr(), in_pitch, in_fs, n, h, w, sigma, min_val, max_val, out.data_ptr(), out_pitch, out_fs)
     return out
 
 
@@ -117,6 +127,26 @@ def canny_bgr(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx
     """canny() for interleaved B,G,R frames (cv2 / cv::Mat layout): (H, W, 3) or (N, H, W, 3), each pixel's 3 bytes contiguous,
     rows and frames with any stride.  The gray conversion is OpenCV's COLOR_BGR2GRAY, bit for bit.  Returns (H, W) or (N, H, W)."""
     return _run(frames, sigma, min_val, max_val, out, ctx, bgr=True)
+
+
+def cv_canny(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None, ctx: Optional[Context] = None):
+    """cv2.Canny(frame, threshold1, threshold2, L2gradient=L2gradient) (apertureSize 3) of gray frames, bit for bit: a CUDA uint8
+    tensor of shape (H, W) or (N, H, W), any strides with contiguous rows, frames of at least 1 x 1.
+
+    No blur, Sobel with replicated borders, L1 (or L2) magnitude, OpenCV's direction test and non-maximum suppression, `> low` /
+    `> high` thresholds (swapped when threshold1 > threshold2), plain 8-connected hysteresis.  Returns a uint8 tensor of the same
+    shape holding 0 / 255 (`out` when given, which may be a strided view).  Asynchronous on torch.cuda.current_stream(frames.device);
+    ctx defaults to one cached Context per device."""
+    return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=False, cv_l2=bool(L2gradient))
+
+
+def cv_canny_color(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None,
+                   ctx: Optional[Context] = None):
+    """cv2.Canny of 3-channel frames, bit for bit: (H, W, 3) or (N, H, W, 3), each pixel's 3 bytes contiguous, rows and frames with
+    any stride.  As cv2.Canny on a 3-channel image: the gradient of every channel, per pixel the channel of largest magnitude.  The
+    channel order does not matter (B,G,R or R,G,B give the same map except where two channels tie, when the first wins).
+    Returns (H, W) or (N, H, W)."""
+    return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient))
 
 
 def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool):

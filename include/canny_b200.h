@@ -213,6 +213,35 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
                                         int n_frames, int height, int width, float sigma, int min_val, int max_val,
                                         uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
 
+/* OpenCV semantics: the edge maps of cv::Canny(image, edges, threshold1, threshold2, 3, l2_gradient) (OpenCV 4.x), bit for bit,
+ * for 8-bit frames with 1 channel or 3 interleaved channels (in any order: B,G,R as cv::Mat holds them, R,G,B, ...), any size of at
+ * least 1 x 1.  The entry points above compute the reference's Canny instead; the differences:
+ *   blur            reference: Gaussian from sigma, renormalised at borders      here: none
+ *   gradient        reference: Sobel, replicate for gx, drop for gy                here: Sobel 3x3, BORDER_REPLICATE for both
+ *   magnitude       reference: floor(sqrt(gx^2 + gy^2))                            here: |dx| + |dy|, or dx^2 + dy^2 against squared
+ *                                                                                        thresholds when l2_gradient != 0
+ *   direction, NMS  reference: atan2 bins, `>` on both sides                       here: fixed-point tan 22.5 deg (13573 / 2^15),
+ *                                                                                        `>` on one side and `>=` on the other, `>`
+ *                                                                                        on both along the diagonals
+ *   thresholds      reference: `>= minVal`, `>= maxVal`, ints                      here: `> low`, `> high`, doubles: swapped when
+ *                                                                                        threshold1 > threshold2; for L2 clamped to
+ *                                                                                        32767 and squared when positive; floored
+ *   hysteresis      reference: 8-connected minus its one-way (1,0)->(0,1) link     here: plain 8-connected
+ *   colour          reference: BGR -> gray first                                   here: Sobel on every channel, per pixel the
+ *                                                                                        channel of largest magnitude (the first
+ *                                                                                        in memory on ties)
+ * Strides in BYTES as b200_canny_batch_device_strided: pixel (f, y, x) is the `channels` bytes at d_in + f*in_frame_stride +
+ * y*in_row_pitch + channels*x, and its 0 / 255 result is written to d_edges + f*out_frame_stride + y*out_row_pitch + x; no other
+ * byte of d_edges is written.  Chunks, stream slots and b200_ctx_set_chunk_frames as the batch calls.  Asynchronous on the
+ * context's stream.
+ * Before any device work: B200_ERR_UNSUPPORTED for channels other than 1 and 3 or a height above 4 194 240 (65535 x 64) rows;
+ * B200_ERR_INVALID_ARG for a NaN or infinite threshold; B200_ERR_UNSUPPORTED for a threshold whose floor (after the L2 squaring)
+ * does not fit in int32, where OpenCV's own conversion overflows; then the layout checks of b200_canny_batch_device_strided (in_row_pitch >= channels*width), except that
+ * frames of 1 pixel per side are accepted. */
+int b200_cv_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride, int n_frames,
+                                 int height, int width, int channels, double threshold1, double threshold2, int l2_gradient,
+                                 uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
+
 /* A list of frames of DIFFERENT sizes and layouts in one call: dataset images, camera streams of several resolutions, crops of
  * detections, a list of cv::cuda::GpuMat.  Each frame has its own size, input pointer and row pitch and its own output pointer
  * and row pitch; sigma and the thresholds are shared.  Frame i's map is the one b200_canny_batch_device_strided gives for that

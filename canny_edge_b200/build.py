@@ -15,7 +15,7 @@ from pathlib import Path
 PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 LIB_PATH = PKG_DIR / "libcanny_b200.so"
-SOURCES = ["front.cu", "front2.cu", "front3.cu", "front_cv.cu", "hysteresis.cu", "stages.cu", "synth.cu", "band.cu", "bands_mgpu.cu", "selftest.cu", "api.cu"]
+SOURCES = ["front.cu", "front3.cu", "front_cv.cu", "hysteresis.cu", "stages.cu", "synth.cu", "band.cu", "bands_mgpu.cu", "selftest.cu", "api.cu"]
 HEADERS = sorted(p.name for p in CSRC.glob("*.h")) + sorted(p.name for p in CSRC.glob("*.cuh")) + ["../../include/canny_b200.h"]
 
 NVCC_FLAGS = [

@@ -385,12 +385,10 @@ static int run_frames_device(b200_ctx* ctx, cudaStream_t st, int slot, const uin
 
 // whether launch_front takes these interleaved B,G,R frames directly (fused conversion) under the context's current sigma
 static bool bgr_fused_ok(const b200_ctx* ctx, const uint8_t* d_bgr, int n, int h, int w, long long pitch, long long frame_stride) {
-    static const int force = [] { const char* e = getenv("B200_CANNY_FRONT"); return e ? atoi(e) : 0; }();
     FrontParams fp;
     memset(&fp, 0, sizeof(fp));
     fp.in = d_bgr; fp.in_pitch = pitch; fp.in_frame_stride = frame_stride; fp.n_frames = n; fp.in_rows = h; fp.width = w;
-    fp.radius = ctx->gauss.radius;
-    return force == 0 && !ctx->gauss.tiny && front3_bgr_supports(fp);
+    return front3_bgr_supports(ctx->gauss, fp);
 }
 
 // The OpenCV-compatible path (b200_cv_canny_device_strided): cv::Canny's thresholds as integers in magnitude space (swapped,
@@ -1182,9 +1180,8 @@ static int frames_device_impl(b200_ctx* ctx, const b200_frame* fr, int n, float 
     CB_TRY(check_thresholds(lo, hi));
     CB_TRY(resolve_ctx(ctx));
     CB_TRY(prepare_gauss(ctx, sigma));
-    static const int force = [] { const char* e = getenv("B200_CANNY_FRONT"); return e ? atoi(e) : 0; }();
-    if (force != 0 || ctx->gauss.tiny || !front3_supports(ctx->gauss.radius)) {
-        // no ragged kernel for this sigma (or a front kernel forced for A/B runs): each frame through the strided path
+    if (!front3_supports(ctx->gauss)) {
+        // no ragged kernel for this sigma: each frame through the strided path
         for (int i = 0; i < n; ++i) {
             const b200_frame& f = fr[i];
             CB_TRY(batch_device_impl(ctx, f.in, f.in_row_pitch, f.height * f.in_row_pitch, 1, f.height, f.width, sigma, lo, hi, f.out,

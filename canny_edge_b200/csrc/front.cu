@@ -1,7 +1,7 @@
 // front.cu — fused stages 1-3 of the Canny hot path for sm_100a, GENERAL variant:
 //   u8 gray  --row blur-->  f32  --column blur + truncate-->  i16 blur  --Sobel-->  (gx,gy)
 //            --magnitude / direction / non-max suppression / double threshold-->  u8 class map
-// It serves what the lean kernel of front2.cu does not: run-time radii (sigma outside the compiled set), the int16 spill planes
+// It serves what the lean kernel of front3.cu does not: run-time radii (sigma outside the compiled set), the int16 spill planes
 // of the stage API / `steps` (blur, magnitude, angle, nms), and sigma so small that sums approach the subnormal range.  The
 // dispatcher launch_front() at the end of this file picks between the two; both are parity-tested against the oracle.
 //
@@ -567,9 +567,8 @@ static int launch_front_v1(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_
     }
 }
 
-// Dispatcher: the lean kernel (front2.cu) for the hot configuration — compile-time radius, no spill planes,
-// ordinary sigma: front3.cu's kernel (front2.cu's with B200_CANNY_FRONT=2); front_kernel above for everything else
-// (B200_CANNY_FRONT=1 forces it: A/B runs).
+// Dispatcher: front3.cu's kernel for the hot configuration — no spill planes and a sigma it takes (front3_supports);
+// front_kernel above for everything else.
 int launch_front(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, bool* sparse_out) {
     FrontParams p = p_in;
     if (sparse_out) *sparse_out = false;
@@ -584,14 +583,12 @@ int launch_front(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, bool* 
         set_error("gaussian radius %d outside [1,%d]", radius, B200_MAX_RADIUS);
         return B200_ERR_UNSUPPORTED;
     }
-    static const int force = [] { const char* e = getenv("B200_CANNY_FRONT"); return e ? atoi(e) : 0; }();
-    const bool force_v1 = force == 1;
     const bool spill = p.blur || p.mag || p.ang || p.nms;
-    if (p.in_bgr && (force_v1 || force == 2 || spill || ctx->gauss.tiny || !front3_bgr_supports(p))) {
+    if (p.in_bgr && (spill || !front3_bgr_supports(ctx->gauss, p))) {
         set_error("interleaved B,G,R input is only taken by the fused front kernel (callers check front3_bgr_supports)");
         return B200_ERR_UNSUPPORTED;
     }
-    if (!force_v1 && !spill && !ctx->gauss.tiny && front2_supports(radius)) {
+    if (!spill && front3_supports(ctx->gauss)) {
         // the sparse hand-over lists KEPT pixels; with minVal <= 0 suppressed pixels are candidates too (src/utils.cpp:328), so the
         // whole-plane labelling has to run
         const bool sparse = p.parent != nullptr && p.kept_list != nullptr && p.kept_count != nullptr && p.cls_zero == 0 &&
@@ -599,13 +596,12 @@ int launch_front(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, bool* 
         if (!sparse) { p.parent = nullptr; p.kept_list = nullptr; p.kept_count = nullptr; }
         if (sparse_out) *sparse_out = sparse;
         ctx->front_fast++;
-        if (force != 2 && front3_supports(radius)) return launch_front3(ctx, st, p);
-        return launch_front2(ctx, st, p);
+        return launch_front3(ctx, st, p);
     }
     // The generic kernel is 3-4x slower than the lean ones.  It is the right one for spill planes (stage API, `steps`); for a plain
     // map it means sigma's half-window is not in the compiled set {2,3,5,6,9,15}: say so once per context instead of silently
     // running at a quarter of the speed (b200_ctx_front_kernel_stats counts both kinds).
-    if (!spill && !force_v1 && ctx->front_generic == 0 && getenv("B200_CANNY_QUIET") == nullptr)
+    if (!spill && ctx->front_generic == 0 && getenv("B200_CANNY_QUIET") == nullptr)
         fprintf(stderr, "libcanny_b200: gaussian half-window %d (sigma %g) has no specialised front kernel (built: 2, 3, 5, 6, 9, 15)%s; "
                         "using the generic kernel (about 4x slower). Set B200_CANNY_QUIET=1 to silence.\n",
                 radius, (double)ctx->gauss.sigma, ctx->gauss.tiny ? " and its weights reach the subnormal range" : "");

@@ -1,5 +1,5 @@
-// front_common.cuh — pieces shared by the two front kernels (front.cu: generic / spilling variant,
-// front2.cu: the lean fused variant): mbarrier + TMA wrappers, u8->f32 conversion, the blur core.
+// front_common.cuh — pieces of the front kernels (front.cu: generic / spilling variant, front3.cu: the lean fused variant):
+// mbarrier + TMA wrappers, the scalar blur core.
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -39,18 +39,6 @@ static __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorM
         "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
         ::"r"(dst), "l"(map), "r"(bar), "r"(x), "r"(y), "r"(z)
         : "memory");
-}
-
-// u8 -> f32 without the conversion pipe: drop the byte into the mantissa of 2^23 and subtract 2^23.
-template <int BYTE>
-static __device__ __forceinline__ float byte_to_float(uint32_t word) {
-    uint32_t bits = __byte_perm(word, 0x4B000000u, 0x7650 + BYTE);  // {b, 0x00, 0x00, 0x4B}
-    return __fsub_rn(__uint_as_float(bits), 8388608.0f);
-}
-static __device__ __forceinline__ float byte_to_float_dyn(const uint32_t* words, int i) {
-    uint32_t word = words[i >> 2];
-    uint32_t bits = __byte_perm(word, 0x4B000000u, 0x7650 + (i & 3));
-    return __fsub_rn(__uint_as_float(bits), 8388608.0f);
 }
 
 // The shared blur core.  S consecutive outputs o = 0..S-1; output o is

@@ -47,7 +47,8 @@ static __device__ __forceinline__ void blur_run2(const u64 (&ws2)[R + 1], Fetch 
     }
 }
 
-// RN(a / b) for the interior count on pairs (same forms, same device-side proof as div_const: check_div_mode_device).
+// RN(a / b) for the interior count on pairs.  The 1- and 3-instruction forms are only used when the host has checked on the
+// device, for this very b and every float mantissa, that they give the IEEE quotient (check_div_mode_device).
 // nb2 = {-b, -b}, y2 = {RN(1/b)} x 2, c2 = {RN(1/b - 1)} x 2
 template <int DIV>
 __device__ __forceinline__ u64 div_const2(u64 a, u64 nb2, u64 y2, u64 c2) {

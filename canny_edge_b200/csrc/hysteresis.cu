@@ -15,7 +15,7 @@
 // component is strong, (1,0)'s becomes strong; not the other way round.
 //
 // Two kernel families, identical results:
-//   list-driven (the default after front2.cu, which hands over a list of the WEAK pixels and their union-find slots):
+//   list-driven (the default after the lean front kernels, which hand over a list of the WEAK pixels and their union-find slots):
 //     ccl_sparse_link     one thread per weak pixel: strong neighbour -> SUPER, unions with its forward weak neighbours; the
 //                         last block applies the one-way link and retires the list's counters (HystParams::ctr)
 //     ccl_sparse_resolve  every weak pixel chases its root and becomes 0 or 255
@@ -282,10 +282,10 @@ ccl_final_kernel(const HystParams p) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// sparse variants: driven by the weak-pixel list front2.cu writes (work ~ number of weak pixels, not pixels)
+// sparse variants: driven by the weak-pixel list front3 (uniform and ragged) and front_cv write (work ~ weak pixels, not pixels)
 // ---------------------------------------------------------------------------------------------
-// Only weak pixels (class 1) need anything: a strong pixel is final.  front2 has initialised parent[] of every weak pixel to its
-// own launch-relative index.  One thread per weak pixel: the eight neighbours' class bytes are fetched together; any strong
+// Only weak pixels (class 1) need anything: a strong pixel is final.  The front kernel has initialised parent[] of every weak pixel
+// to its own launch-relative index.  One thread per weak pixel: the eight neighbours' class bytes are fetched together; any strong
 // neighbour hangs the pixel's component under SUPER; weak "forward" neighbours E, S (or SW / SE when S is not weak: with S weak
 // the two diagonals reach the pixel through S's own links) are united with it, so every weak-weak pair is visited exactly once,
 // from its earlier endpoint in raster order.  The pair (0,1)-(1,0) of the GLOBAL image is skipped in both directions (see the

@@ -81,10 +81,10 @@ struct FrontParams {
     int lo2, hi2;           // thresholds in squared-magnitude space (see front.cu)
     int lo, hi;             // raw thresholds (spill / zero-class decisions)
     int cls_zero;           // class of a suppressed pixel (value 0): nonzero only when lo <= 0
-    float div_c;            // front2: c of the one-instruction interior division (GaussTables::div_c)
+    float div_c;            // front3: c of the one-instruction interior division (GaussTables::div_c)
     int ieee_div;           // 1: weights so small that sums can fall below 2^-100 -> use IEEE division instead of div_exact
     int tiles_x, tiles_y;
-    // sparse hand-over to the hysteresis kernels (front2.cu only; both null -> not produced):
+    // sparse hand-over to the hysteresis kernels (front3.cu and front_cv.cu only; both null -> not produced):
     int32_t* parent;        // union-find slots, dense: every WEAK pixel is initialised to its own launch-relative index
                             // frame*out_frame_stride + (y - plane_row0)*width + x (strong pixels need no slot: they are final)
     uint32_t* kept_list;    // launch-relative indices of all weak pixels, in no particular order
@@ -171,12 +171,12 @@ struct HystParams {
     int row0;              // global row of plane row 0 (the missing-link quirk lives at global (1,0)->(0,1))
     int n_frames;
     int tiles_x, tiles_y;
-    const uint32_t* list;        // weak-pixel list written by front2 (null -> tile-based labelling over the whole plane);
+    const uint32_t* list;        // weak-pixel list written by the front kernel (null -> tile-based labelling over the whole plane);
                                  // the list-driven kernels keep LAUNCH-relative indices (frame*frame_stride + pixel) in parent[]
     // Counter block of the list (null when the front kernel did not produce one).  It is zeroed ONCE, when the workspace is
     // allocated, and then kept consistent by the kernels themselves, so a launch needs neither a memset before the front kernel
     // nor a copy after it:
-    //   ctr[0]  live entry count (front2's atomicAdd)        ctr[1]  link-kernel blocks that have finished
+    //   ctr[0]  live entry count (the front kernel's atomicAdd)   ctr[1]  link-kernel blocks that have finished
     //   ctr[2]  entry count of the finished launch: written, with h_kept, by the last block of the link kernel (or by
     //           list_retire_kernel on the tile-based path), which also zeroes ctr[0] and ctr[1] for the next launch
     unsigned int* ctr;
@@ -235,7 +235,7 @@ struct b200_ctx {
     cb::Workspace ws_band_aux;            // boundary roots of the resident band + the cross-band forest
     int chunk_frames = 0;
     long long launches = 0;
-    long long front_fast = 0, front_generic = 0;   // front-kernel launches on the lean kernels (front3 / front2) and on front.cu's generic one
+    long long front_fast = 0, front_generic = 0;   // front-kernel launches on the lean kernels (front3 / front_cv) and on front.cu's generic one
     unsigned long long h2d_bytes = 0, d2h_bytes = 0;  // PCIe bytes moved by b200_canny_batch_host so far
     cb::Profiler prof;
     // band state (row-band sharding)
@@ -284,12 +284,10 @@ int host_window(float sigma);
 int launch_front(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, bool* sparse_out = nullptr);
 int make_input_tensor_map(const FrontParams& p, int box_cols, int box_rows, CUtensorMap_st* tmap, bool* use_tma);
 int make_bgr_tensor_map(const FrontParams& p, int box_words, int box_rows, CUtensorMap_st* tmap);   // 32-bit elements over 3*width-byte rows
-// front2.cu
-bool front2_supports(int radius);
-int launch_front2(b200_ctx* ctx, cudaStream_t st, const FrontParams& p);
 // front3.cu (packed-FP32 blur, half-precision Sobel; the default for the radii it is built for)
-bool front3_supports(int radius);
-bool front3_bgr_supports(const FrontParams& p);   // p.in / width / in_frame_stride / radius allow the fused BGR -> gray staging
+bool front3_supports(const GaussTables& g);   // front3 takes this sigma: its half-window is compiled and its weights are not tiny
+// ... and these interleaved B,G,R frames: p.in / width / in_pitch / in_frame_stride allow the fused BGR -> gray staging
+bool front3_bgr_supports(const GaussTables& g, const FrontParams& p);
 int launch_front3(b200_ctx* ctx, cudaStream_t st, const FrontParams& p);
 // ragged chunks: class-row band height shared by the chunk's frames (the policy is described at its definition), the work items
 // of one frame, and the launch over n_items items of p.ritems (all TMA-staged or all byte-staged)

@@ -28,8 +28,7 @@
 // magnitude^2 plane 33 KB (it can no longer alias the temp rows: they are being refilled), candidate lists 8 KB: 176 KB, one CTA per
 // SM, <= 96 registers x 640 threads.
 //
-// Used for compile-time radii without spill planes; everything else stays on front.cu's kernel.  B200_CANNY_FRONT=3 / 2 select
-// front3.cu's / front2.cu's kernel for A/B runs.
+// Used for compile-time radii without spill planes; everything else stays on front.cu's kernel.
 #include <cuda.h>
 
 #include "canny_math.h"

@@ -1,9 +1,9 @@
 """SASS evidence for the front kernels (run on the CPU box; needs cuobjdump):
   * TMA (cp.async.bulk.tensor) shows up as UTMALDG, its mbarrier as SYNCS;
-  * the blur's products and sums are separate FMUL / FADD — the only FFMAs are the Markstein division steps
-    (and, in front2, none are FFMA2: packed FP32 is not used);
-  * opcode histogram of the hot instantiation.
-    python tools/sass_check.py > profiles/r01_front2_sass_summary.txt
+  * the blur's products and sums are separate multiplies and adds (FMUL2.FTZ / FADD2) — FFMA / FFMA2 only where written: the
+    Markstein division steps and the exact-integer vertical Sobel;
+  * opcode histogram of one instantiation, by default front3's bench kernel <R=5, TMA, DIV=1, SLAB=64, gray, dense, uniform>:
+    python tools/sass_check.py > profiles/r02_front3_sass_summary.txt
 """
 import collections
 import re
@@ -13,7 +13,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[1]
 lib = ROOT / "canny_edge_b200" / "libcanny_b200.so"
-want = sys.argv[1] if len(sys.argv) > 1 else "front2_kernelILi5ELb1ELb1"
+want = sys.argv[1] if len(sys.argv) > 1 else "front3_kernelILi5ELb1ELi1ELi64ELb0ELb0ELb0E"
 sass = subprocess.run(["cuobjdump", "-sass", str(lib)], capture_output=True, text=True).stdout
 cur, keep = None, []
 for line in sass.splitlines():

@@ -12,7 +12,7 @@ Layout:
 from ._lib import CannyB200Error, LIB_PATH, load  # noqa: F401
 from .api import (  # noqa: F401
     EDGE, NOEDGE, PI, Context, calculateXYGradient, canny_batch_device_bgr_ptr, canny_batch_device_bgr_strided_ptr, canny_batch_device_ptr,
-    canny_batch_device_strided_ptr, canny_batch_host, canny_frames_device_ptr, createGaussianKernel, cv_canny_device_strided_ptr, cuda_canny, cuda_canny_bgr, cuda_gaussian, cuda_hysteresis,
+    canny_batch_device_strided_ptr, canny_batch_host, canny_frames_device_ptr, createGaussianKernel, cv_canny_device_strided_ptr, cv_canny_frames_device_ptr, cuda_canny, cuda_canny_bgr, cuda_gaussian, cuda_hysteresis,
     cuda_nonmaixmal_suppression, cuda_sobel, synth_host, synth_rows_host,
 )
 from . import torch_api  # noqa: F401  (torch is imported inside its functions)

@@ -252,6 +252,17 @@ def canny_frames_device_ptr(ctx: Optional[Context], descs, sigma: float, min_val
     check(fn(_h(ctx), frame_list(descs), len(descs), C.c_float(sigma), int(min_val), int(max_val)))
 
 
+def cv_canny_frames_device_ptr(ctx: Optional[Context], descs, channels: int, threshold1: float, threshold2: float,
+                               l2_gradient: bool) -> None:
+    """cv2.Canny(frame, threshold1, threshold2, L2gradient=l2_gradient) of frames of different sizes in one call, bit for bit
+    (b200_cv_canny_frames_device).  descs as canny_frames_device_ptr: pixel (y, x) of a frame is the `channels` bytes (1 or 3
+    interleaved) at in_ptr + y*in_pitch + channels*x, its 0 / 255 result written at out_ptr + y*out_pitch + x; frames from 1 x 1.
+    Asynchronous on the context's stream."""
+    descs = list(descs)
+    check(load().b200_cv_canny_frames_device(_h(ctx), frame_list(descs), len(descs), int(channels), C.c_double(threshold1),
+                                             C.c_double(threshold2), int(bool(l2_gradient))))
+
+
 def synth_host(n: int, h: int, w: int, kind: int = 0, seed: int = 1234, first_frame: int = 0) -> np.ndarray:
     out = np.empty((n, h, w), np.uint8)
     check(load().b200_synth_host(_ptr(out), n, h, w, kind, C.c_uint64(seed), first_frame))

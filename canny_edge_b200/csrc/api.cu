@@ -12,6 +12,7 @@
 #include <algorithm>
 #include <condition_variable>
 #include <fstream>
+#include <functional>
 #include <sstream>
 #include <mutex>
 #include <thread>
@@ -1016,9 +1017,10 @@ int b200_cv_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_
 }
 
 // ---- ragged lists: frames of different sizes in one call ------------------------------------------------
-// Argument checks of b200_canny_frames_device[_bgr]; all of them run before any device work.  Overlaps are found by sorting the
-// extents (a list can hold thousands of frames): the outputs among themselves, then every output against the merged inputs.
-static int check_frames(const b200_frame* fr, int n, int bpp) {
+// Argument checks of b200_canny_frames_device[_bgr] and b200_cv_canny_frames_device; all of them run before any device work.  Overlaps
+// are found by sorting the extents (a list can hold thousands of frames): the outputs among themselves, then every output against
+// the merged inputs.  bpp: bytes per input pixel; min_side as check_image.
+static int check_frames(const b200_frame* fr, int n, int bpp, int min_side = 2) {
     if (!fr) { set_error("null frame list"); return B200_ERR_INVALID_ARG; }
     if (n <= 0) { set_error("n_frames must be positive"); return B200_ERR_INVALID_ARG; }
     typedef __int128 i128;
@@ -1027,7 +1029,10 @@ static int check_frames(const b200_frame* fr, int n, int bpp) {
     for (int i = 0; i < n; ++i) {
         const b200_frame& f = fr[i];
         if (!f.in || !f.out) { set_error("frame %d: null image pointer", i); return B200_ERR_INVALID_ARG; }
-        if (f.height < 2 || f.width < 2) { set_error("frame %d: height and width must be >= 2 (got %dx%d)", i, f.height, f.width); return B200_ERR_INVALID_ARG; }
+        if (f.height < min_side || f.width < min_side) {
+            set_error("frame %d: height and width must be >= %d (got %dx%d)", i, min_side, f.height, f.width);
+            return B200_ERR_INVALID_ARG;
+        }
         if (f.in_row_pitch < 0 || f.out_row_pitch < 0) {
             set_error("frame %d: negative row pitch (in %lld, out %lld)", i, (long long)f.in_row_pitch, (long long)f.out_row_pitch);
             return B200_ERR_INVALID_ARG;
@@ -1068,6 +1073,41 @@ static int check_frames(const b200_frame* fr, int n, int bpp) {
 constexpr long long kRaggedChunkPx = 75LL << 20;   // the uniform path's chunk budget (auto_chunk_frames): a chunk's class map fits L2
 
 static size_t align16(size_t v) { return (v + 15) & ~(size_t)15; }
+
+// A ragged chunk's table is built on the host in the slot's pinned staging and sent up with one copy.  The staging is rewritten only
+// once the copy out of it (previous chunk or call on this slot) has completed: this waits for ev_ragged[s], lets fill(h) write the
+// `bytes` bytes at h, copies them to the slot's device table (*d) and records ev_ragged[s] behind the copy.
+static int upload_ragged_table(b200_ctx* ctx, cudaStream_t st, int s, size_t bytes, const std::function<void(uint8_t*)>& fill,
+                               uint8_t** d) {
+    if (ctx->ragged_busy[s]) { CB_CUDA(cudaEventSynchronize(ctx->ev_ragged[s])); ctx->ragged_busy[s] = false; }
+    CB_TRY(ensure_ws(ctx->host_ragged[s], bytes, /*pinned_host=*/true));
+    CB_TRY(ensure_ws(ctx->ws_ragged[s], bytes));
+    uint8_t* h = reinterpret_cast<uint8_t*>(ctx->host_ragged[s].ptr);
+    *d = reinterpret_cast<uint8_t*>(ctx->ws_ragged[s].ptr);
+    fill(h);
+    CB_CUDA(cudaMemcpyAsync(*d, h, bytes, cudaMemcpyHostToDevice, st));
+    CB_CUDA(cudaEventRecord(ctx->ev_ragged[s], st));
+    ctx->ragged_busy[s] = true;
+    return B200_OK;
+}
+
+// The frame descriptors and dense slot bases of a chunk.  src / src_pitch: what each frame's front kernel reads (null: the caller's
+// frames themselves).
+static void fill_ragged_frames(const b200_frame* fr, int nf, const uint8_t* const* src, const long long* src_pitch, RaggedFrame* hf,
+                               uint32_t* hb) {
+    long long base = 0;
+    for (int i = 0; i < nf; ++i) {
+        const b200_frame& f = fr[i];
+        RaggedFrame& r = hf[i];
+        r.in = src ? src[i] : f.in; r.in_pitch = src_pitch ? src_pitch[i] : f.in_row_pitch;
+        r.cls = f.out; r.cls_pitch = f.out_row_pitch;
+        r.height = f.height; r.width = f.width;
+        r.base = (int)base;
+        r.cls_words = ((reinterpret_cast<uintptr_t>(f.out) | (uintptr_t)f.out_row_pitch) & 3) == 0;
+        hb[i] = (uint32_t)base;
+        base += (long long)f.height * f.width;
+    }
+}
 
 // One chunk of a ragged list on slot s / stream st: table (descriptors, tensor maps, work items, B,G,R jobs) built on the host into
 // the slot's pinned staging and sent up with one copy; then [B,G,R -> gray], the front kernel (one launch per staging form, both
@@ -1112,37 +1152,21 @@ static int run_ragged_chunk(b200_ctx* ctx, cudaStream_t st, int s, const b200_fr
     const size_t off_items = align16(off_bases + (size_t)nf * sizeof(uint32_t));
     const size_t off_jobs = align16(off_items + n_items * sizeof(RaggedItem));
     const size_t bytes = off_jobs + (bgr ? (size_t)nf * sizeof(RaggedGrayJob) : 0);
-    // the staging of this slot is rewritten only once the copy out of it (previous chunk or call on this slot) has completed
-    if (ctx->ragged_busy[s]) { CB_CUDA(cudaEventSynchronize(ctx->ev_ragged[s])); ctx->ragged_busy[s] = false; }
-    CB_TRY(ensure_ws(ctx->host_ragged[s], bytes, /*pinned_host=*/true));
-    CB_TRY(ensure_ws(ctx->ws_ragged[s], bytes));
-    uint8_t* h = reinterpret_cast<uint8_t*>(ctx->host_ragged[s].ptr);
-    uint8_t* d = reinterpret_cast<uint8_t*>(ctx->ws_ragged[s].ptr);
-    memcpy(h, maps.data(), off_frames);
-    RaggedFrame* hf = reinterpret_cast<RaggedFrame*>(h + off_frames);
-    uint32_t* hb = reinterpret_cast<uint32_t*>(h + off_bases);
-    RaggedGrayJob* hj = reinterpret_cast<RaggedGrayJob*>(h + off_jobs);
-    long long base = 0, row0 = 0;
-    for (int i = 0; i < nf; ++i) {
-        const b200_frame& f = fr[i];
-        RaggedFrame& r = hf[i];
-        r.in = src[(size_t)i]; r.in_pitch = src_pitch[(size_t)i];
-        r.cls = f.out; r.cls_pitch = f.out_row_pitch;
-        r.height = f.height; r.width = f.width;
-        r.base = (int)base;
-        r.cls_words = ((reinterpret_cast<uintptr_t>(f.out) | (uintptr_t)f.out_row_pitch) & 3) == 0;
-        hb[i] = (uint32_t)base;
-        base += (long long)f.height * f.width;
-        if (bgr) {
+    long long row0 = 0;
+    uint8_t* d = nullptr;
+    CB_TRY(upload_ragged_table(ctx, st, s, bytes, [&](uint8_t* h) {
+        memcpy(h, maps.data(), off_frames);
+        fill_ragged_frames(fr, nf, src.data(), src_pitch.data(), reinterpret_cast<RaggedFrame*>(h + off_frames),
+                           reinterpret_cast<uint32_t*>(h + off_bases));
+        RaggedGrayJob* hj = reinterpret_cast<RaggedGrayJob*>(h + off_jobs);
+        for (int i = 0; bgr && i < nf; ++i) {
+            const b200_frame& f = fr[i];
             hj[i] = RaggedGrayJob{f.in, f.in_row_pitch, const_cast<uint8_t*>(src[(size_t)i]), src_pitch[(size_t)i], (int)row0, f.width};
             row0 += f.height;
         }
-    }
-    memcpy(h + off_items, items_tma.data(), items_tma.size() * sizeof(RaggedItem));
-    memcpy(h + off_items + items_tma.size() * sizeof(RaggedItem), items_byte.data(), items_byte.size() * sizeof(RaggedItem));
-    CB_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, st));
-    CB_CUDA(cudaEventRecord(ctx->ev_ragged[s], st));
-    ctx->ragged_busy[s] = true;
+        memcpy(h + off_items, items_tma.data(), items_tma.size() * sizeof(RaggedItem));
+        memcpy(h + off_items + items_tma.size() * sizeof(RaggedItem), items_byte.data(), items_byte.size() * sizeof(RaggedItem));
+    }, &d));
     if (bgr) CB_TRY(launch_bgr_to_gray_ragged(ctx, st, reinterpret_cast<const RaggedGrayJob*>(d + off_jobs), nf, row0));
 
     FrontParams fp;
@@ -1175,19 +1199,71 @@ static int run_ragged_chunk(b200_ctx* ctx, cudaStream_t st, int s, const b200_fr
     return B200_OK;
 }
 
-static int frames_device_impl(b200_ctx* ctx, const b200_frame* fr, int n, float sigma, int lo, int hi, int bpp) {
-    CB_TRY(check_frames(fr, n, bpp));
-    CB_TRY(check_thresholds(lo, hi));
+// One chunk of an OpenCV-compatible list (b200_cv_canny_frames_device) on slot s / stream st: table (frame descriptors | bases | tile
+// items) sent up as run_ragged_chunk's, then the OpenCV front kernel over every frame's 128 x 64 tiles and the list-driven hysteresis
+// kernels with plain 8-connectivity.  No Gaussian tables, tensor maps, band height or B,G,R jobs: the kernel stages the caller's 1 or
+// 3 interleaved bytes per pixel itself, 16-byte loads where a chunk of a row is aligned and byte loads elsewhere.  As run_frames_cv,
+// the uniform path's density state (h_kept, kept_px) is neither read nor written.
+static int run_ragged_cv_chunk(b200_ctx* ctx, cudaStream_t st, int s, const b200_frame* fr, int nf, const CvSpec& cv) {
+    std::vector<RaggedItem> items;
+    long long px = 0;
+    for (int i = 0; i < nf; ++i) {
+        ragged_items_cv(i, fr[i].height, fr[i].width, items);
+        px += (long long)fr[i].height * fr[i].width;
+    }
+    const size_t off_bases = align16((size_t)nf * sizeof(RaggedFrame));
+    const size_t off_items = align16(off_bases + (size_t)nf * sizeof(uint32_t));
+    const size_t bytes = off_items + items.size() * sizeof(RaggedItem);
+    uint8_t* d = nullptr;
+    CB_TRY(upload_ragged_table(ctx, st, s, bytes, [&](uint8_t* h) {
+        fill_ragged_frames(fr, nf, nullptr, nullptr, reinterpret_cast<RaggedFrame*>(h), reinterpret_cast<uint32_t*>(h + off_bases));
+        memcpy(h + off_items, items.data(), items.size() * sizeof(RaggedItem));
+    }, &d));
+
+    FrontParams fp;
+    memset(&fp, 0, sizeof(fp));
+    fp.lo = cv.lo; fp.hi = cv.hi;
+    fp.parent = reinterpret_cast<int32_t*>(ctx->ws_parent[s].ptr);
+    fp.kept_count = reinterpret_cast<unsigned int*>(ctx->ws_list[s].ptr);
+    fp.kept_list = reinterpret_cast<uint32_t*>(ctx->ws_list[s].ptr) + 16;
+    fp.rframes = reinterpret_cast<const RaggedFrame*>(d);
+    fp.ritems = reinterpret_cast<const RaggedItem*>(d + off_items);
+    // the list's counter block is zero here (see run_frames_device)
+    if (ctx->list_dirty[s]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
+    ctx->list_dirty[s] = true;
+    CB_TRY(launch_front_cv_ragged(ctx, st, fp, (int)items.size(), cv.channels, cv.l2));
+    RaggedHystParams hp;
+    memset(&hp, 0, sizeof(hp));
+    hp.frames = fp.rframes;
+    hp.bases = reinterpret_cast<const uint32_t*>(d + off_bases);
+    hp.n_frames = nf;
+    hp.parent = fp.parent; hp.list = fp.kept_list; hp.ctr = fp.kept_count;
+    hp.px = px;
+    hp.opencv = 1;
+    CB_TRY(launch_hysteresis_ragged(ctx, st, hp));
+    ctx->list_dirty[s] = false;
+    return B200_OK;
+}
+
+// cv: an OpenCV-compatible list (b200_cv_canny_frames_device; its channel count and thresholds are checked by the caller, sigma, lo
+// and hi are unused): the same checks (frames from 1 x 1), chunks, slots and workspace, each chunk through run_ragged_cv_chunk.  It
+// needs no sigma, so it never prepares Gaussian tables and never takes the per-frame fallback.  Null: the reference's semantics.
+static int frames_device_impl(b200_ctx* ctx, const b200_frame* fr, int n, float sigma, int lo, int hi, int bpp,
+                              const CvSpec* cv = nullptr) {
+    CB_TRY(check_frames(fr, n, bpp, cv ? 1 : 2));
+    if (!cv) CB_TRY(check_thresholds(lo, hi));
     CB_TRY(resolve_ctx(ctx));
-    CB_TRY(prepare_gauss(ctx, sigma));
-    if (!front3_supports(ctx->gauss)) {
-        // no ragged kernel for this sigma: each frame through the strided path
-        for (int i = 0; i < n; ++i) {
-            const b200_frame& f = fr[i];
-            CB_TRY(batch_device_impl(ctx, f.in, f.in_row_pitch, f.height * f.in_row_pitch, 1, f.height, f.width, sigma, lo, hi, f.out,
-                                     f.out_row_pitch, f.height * f.out_row_pitch, bpp));
+    if (!cv) {
+        CB_TRY(prepare_gauss(ctx, sigma));
+        if (!front3_supports(ctx->gauss)) {
+            // no ragged kernel for this sigma: each frame through the strided path
+            for (int i = 0; i < n; ++i) {
+                const b200_frame& f = fr[i];
+                CB_TRY(batch_device_impl(ctx, f.in, f.in_row_pitch, f.height * f.in_row_pitch, 1, f.height, f.width, sigma, lo, hi, f.out,
+                                         f.out_row_pitch, f.height * f.out_row_pitch, bpp));
+            }
+            return B200_OK;
         }
-        return B200_OK;
     }
     // chunks in call order: about the uniform path's pixel budget each, at most chunk_frames (b200_ctx_set_chunk_frames) frames;
     // a frame above the budget has a chunk of its own
@@ -1209,19 +1285,22 @@ static int frames_device_impl(b200_ctx* ctx, const b200_frame* fr, int n, float 
     starts.push_back(n);
     const int n_chunks = (int)starts.size() - 1;
     const int n_slots = std::min(3, n_chunks);
+    const bool gray_scratch = bpp == 3 && !cv;   // the OpenCV kernel reads 3-channel frames itself
     for (int s = 0; s < n_slots; ++s) {
         CB_TRY(ensure_ws(ctx->ws_parent[s], (size_t)max_px * 4));
         CB_TRY(ensure_ws(ctx->ws_list[s], 64 + (size_t)max_px * 4));
-        if (bpp == 3) CB_TRY(ensure_ws(ctx->dev_in[s], (size_t)max_gray));
+        if (gray_scratch) CB_TRY(ensure_ws(ctx->dev_in[s], (size_t)max_gray));
     }
-    if (n_slots == 1) return run_ragged_chunk(ctx, ctx->stream, 0, fr, n, lo, hi, bpp == 3);
+    auto run_chunk = [&](cudaStream_t st, int s, int c) -> int {
+        const b200_frame* f = fr + starts[(size_t)c];
+        const int nf = starts[(size_t)c + 1] - starts[(size_t)c];
+        return cv ? run_ragged_cv_chunk(ctx, st, s, f, nf, *cv) : run_ragged_chunk(ctx, st, s, f, nf, lo, hi, bpp == 3);
+    };
+    if (n_slots == 1) return run_chunk(ctx->stream, 0, 0);
     // the same three stream slots and fork / join as batch_device_impl
     CB_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
     for (int s = 0; s < n_slots; ++s) CB_CUDA(cudaStreamWaitEvent(ctx->side[s], ctx->ev_fork, 0));
-    for (int c = 0; c < n_chunks; ++c) {
-        const int s = c % n_slots;
-        CB_TRY(run_ragged_chunk(ctx, ctx->side[s], s, fr + starts[(size_t)c], starts[(size_t)c + 1] - starts[(size_t)c], lo, hi, bpp == 3));
-    }
+    for (int c = 0; c < n_chunks; ++c) CB_TRY(run_chunk(ctx->side[c % n_slots], c % n_slots, c));
     for (int s = 0; s < n_slots; ++s) {
         CB_CUDA(cudaEventRecord(ctx->ev_join[s], ctx->side[s]));
         CB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join[s], 0));
@@ -1235,6 +1314,16 @@ int b200_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_fram
 
 int b200_canny_frames_device_bgr(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val) {
     return frames_device_impl(ctx, frames, n_frames, sigma, min_val, max_val, 3);
+}
+
+int b200_cv_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
+                                double threshold2, int l2_gradient) {
+    if (channels != 1 && channels != 3) { set_error("channels must be 1 or 3 (got %d)", channels); return B200_ERR_UNSUPPORTED; }
+    CvSpec cv;
+    cv.channels = channels;
+    cv.l2 = l2_gradient != 0;
+    CB_TRY(cv_thresholds(threshold1, threshold2, cv.l2, &cv.lo, &cv.hi));
+    return frames_device_impl(ctx, frames, n_frames, 0.f, 0, 0, channels, &cv);
 }
 
 // Host buffers in, host buffers out: frames -> 0 / 255 edge maps, as bytes (edges8) or as the reference's int16 (edges16).

@@ -1,4 +1,5 @@
-// front_cv.cu — the front kernel of the OpenCV-compatible path (b200_cv_canny_device_strided): 1- or 3-channel u8 frames -> class
+// front_cv.cu — the front kernel of the OpenCV-compatible path (b200_cv_canny_device_strided, and b200_cv_canny_frames_device through
+// the RAGGED variant below): 1- or 3-channel u8 frames -> class
 // map (0 / 1 weak / 255 strong) plus the weak-pixel hand-over of the list-driven hysteresis kernels, with cv::Canny's arithmetic
 // (apertureSize 3) bit for bit.  No blur: Sobel 3x3 on the input, BORDER_REPLICATE for both derivatives.
 //
@@ -16,10 +17,18 @@
 //   4. hand-over: each thread's 32 pixels fit one bitmask of weak pixels; one atomicAdd per CTA reserves room in the list, and
 //      every weak pixel gets its union-find slot (its own dense launch-relative index) and its list entry.
 //
+// RAGGED (b200_cv_canny_frames_device): frames of different sizes in one launch.  A 1-D grid over work items (p.ritems), each naming a
+// frame and one 128 x 64 tile of it (RaggedItem: x0, yb; ye is not read, rows past the frame's height are clipped as in a uniform
+// launch); the frame's descriptor (p.rframes) replaces in / in_pitch / width / height / cls / cls_pitch / cls_words and its slot
+// base replaces frame * out_frame_stride.  Staging is per frame as above: 16-byte loads where the chunk is aligned, byte loads
+// elsewhere.
+//
 // Integer bounds: |dx|, |dy| <= 4 * 255 = 1020; L1 m <= 2040; L2 m <= 2 * 1020^2 = 2 080 800, so m << 2 | code < 2^23.  In the
 // direction test x = |dx| <= 1020: x * TG22 <= 13 844 460 and x << 16 <= 66 846 720, their sum and |dy| << 15 <= 33 423 360 fit in
 // int32.
 #include <string.h>
+
+#include <algorithm>
 
 #include "internal.h"
 
@@ -45,7 +54,7 @@ struct Smem {
     static constexpr int total = sum_off + 16 * 4;
 };
 
-template <int C, bool L2>
+template <int C, bool L2, bool RAGGED = false>
 __global__ void __launch_bounds__(kThreads)
 front_cv_kernel(const FrontParams p) {
     extern __shared__ __align__(16) unsigned char smem[];
@@ -57,9 +66,16 @@ front_cv_kernel(const FrontParams p) {
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int x0 = blockIdx.x * kTW, y0 = blockIdx.y * kTH, frame = blockIdx.z;
-    const int W = p.width, H = p.height;
-    const uint8_t* in_f = p.in + (long long)frame * p.in_frame_stride;
+    RaggedItem item;
+    RaggedFrame fd;
+    if (RAGGED) {
+        item = p.ritems[blockIdx.x];
+        fd = p.rframes[item.frame];
+    }
+    const int x0 = RAGGED ? item.x0 : blockIdx.x * kTW, y0 = RAGGED ? item.yb : blockIdx.y * kTH, frame = RAGGED ? 0 : blockIdx.z;
+    const int W = RAGGED ? fd.width : p.width, H = RAGGED ? fd.height : p.height;
+    const uint8_t* in_f = RAGGED ? fd.in : p.in + (long long)frame * p.in_frame_stride;
+    const long long in_pitch = RAGGED ? fd.in_pitch : p.in_pitch;
 
     // ---- 1. staging, clamped coordinates ----
     {
@@ -69,7 +85,7 @@ front_cv_kernel(const FrontParams p) {
         for (int i = tid; i < kSH * kChunks; i += kThreads) {
             const int r = i / kChunks, q = i - r * kChunks;
             const int y = min(max(y0 - 2 + r, 0), H - 1);
-            const uint8_t* row = in_f + (long long)y * p.in_pitch;
+            const uint8_t* row = in_f + (long long)y * in_pitch;
             const long long b0 = xb + 16 * q;
             uint4 v;
             if (b0 >= 0 && b0 + 16 <= row_bytes && ((reinterpret_cast<uintptr_t>(row + b0) & 15) == 0)) {
@@ -139,8 +155,9 @@ front_cv_kernel(const FrontParams p) {
     uint32_t weak_mask = 0;                                      // bit 4k + e: pixel e of this lane's quad in row warp + 8k
     if (warp < 8) {
         const int xq = x0 + 4 * lane;
-        uint8_t* cls_f = p.cls + (long long)frame * p.cls_frame_stride;
-        const bool words = p.cls_words && xq + 3 < W;
+        uint8_t* cls_f = RAGGED ? fd.cls : p.cls + (long long)frame * p.cls_frame_stride;
+        const long long cls_pitch = RAGGED ? fd.cls_pitch : p.cls_pitch;
+        const bool words = (RAGGED ? fd.cls_words : p.cls_words) && xq + 3 < W;
 #pragma unroll 1
         for (int k = 0; k < kTH / 8; ++k) {
             const int r = warp + 8 * k, y = y0 + r;
@@ -180,7 +197,7 @@ front_cv_kernel(const FrontParams p) {
                 weak_mask |= (uint32_t)weak << (4 * k + e);
             }
             if (y < H) {
-                uint8_t* o = cls_f + (long long)y * p.cls_pitch + xq;
+                uint8_t* o = cls_f + (long long)y * cls_pitch + xq;
                 if (words) {
                     *reinterpret_cast<uint32_t*>(o) = word;
                 } else {
@@ -208,7 +225,7 @@ front_cv_kernel(const FrontParams p) {
     __syncthreads();
     if (weak_mask) {
         uint32_t* dst = p.kept_list + s_sum[15] + s_sum[warp] + (unsigned int)(incl - cnt);
-        const long long g0 = (long long)frame * p.out_frame_stride + (long long)y0 * W + x0 + 4 * lane;
+        const long long g0 = (RAGGED ? (long long)fd.base : (long long)frame * p.out_frame_stride) + (long long)y0 * W + x0 + 4 * lane;
         uint32_t m = weak_mask;
         while (m) {
             const int bit = __ffs(m) - 1;
@@ -220,16 +237,16 @@ front_cv_kernel(const FrontParams p) {
     }
 }
 
-template <int C, bool L2>
+template <int C, bool L2, bool RAGGED = false>
 static int launch_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, dim3 grid) {
     static bool configured[64] = {false};  // per instantiation, per device
     if (!configured[ctx->device & 63]) {
-        CB_CUDA(cudaFuncSetAttribute(front_cv_kernel<C, L2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<C>::total));
+        CB_CUDA(cudaFuncSetAttribute(front_cv_kernel<C, L2, RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<C>::total));
         configured[ctx->device & 63] = true;
     }
     {
         ProfScope ps(ctx, st, 0);
-        front_cv_kernel<C, L2><<<grid, kThreads, Smem<C>::total, st>>>(p);
+        front_cv_kernel<C, L2, RAGGED><<<grid, kThreads, Smem<C>::total, st>>>(p);
     }
     CB_CUDA(cudaGetLastError());
     ctx->launches++;
@@ -247,6 +264,25 @@ int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, int
     ctx->front_fast++;
     if (channels == 1) return l2 ? fcv::launch_cv<1, true>(ctx, st, p, grid) : fcv::launch_cv<1, false>(ctx, st, p, grid);
     if (channels == 3) return l2 ? fcv::launch_cv<3, true>(ctx, st, p, grid) : fcv::launch_cv<3, false>(ctx, st, p, grid);
+    set_error("OpenCV front kernel: %d channels (1 or 3 are supported)", channels);
+    return B200_ERR_UNSUPPORTED;
+}
+
+void ragged_items_cv(int frame, int height, int width, std::vector<RaggedItem>& items) {
+    for (int y0 = 0; y0 < height; y0 += fcv::kTH)
+        for (int x0 = 0; x0 < width; x0 += fcv::kTW) items.push_back(RaggedItem{frame, x0, y0, std::min(height, y0 + fcv::kTH)});
+}
+
+int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, int channels, bool l2) {
+    if (!p.parent || !p.kept_list || !p.kept_count || !p.rframes || !p.ritems) {
+        set_error("internal: ragged OpenCV front kernel without its table or weak-pixel list");
+        return B200_ERR_INVALID_ARG;
+    }
+    if (n_items <= 0) return B200_OK;
+    const dim3 grid(n_items);
+    ctx->front_fast++;
+    if (channels == 1) return l2 ? fcv::launch_cv<1, true, true>(ctx, st, p, grid) : fcv::launch_cv<1, false, true>(ctx, st, p, grid);
+    if (channels == 3) return l2 ? fcv::launch_cv<3, true, true>(ctx, st, p, grid) : fcv::launch_cv<3, false, true>(ctx, st, p, grid);
     set_error("OpenCV front kernel: %d channels (1 or 3 are supported)", channels);
     return B200_ERR_UNSUPPORTED;
 }

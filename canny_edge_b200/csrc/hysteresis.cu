@@ -19,9 +19,9 @@
 //     ccl_sparse_link     one thread per weak pixel: strong neighbour -> SUPER, unions with its forward weak neighbours; the
 //                         last block applies the one-way link and retires the list's counters (HystParams::ctr)
 //     ccl_sparse_resolve  every weak pixel chases its root and becomes 0 or 255
-//     ragged chunks (frames of different sizes, b200_canny_frames_device) always take the list-driven pair, in a form that finds
-//     each entry's frame in the chunk's table (ccl_ragged_link / ccl_ragged_resolve); the tile-based family below serves uniform
-//     batches only
+//     ragged chunks (frames of different sizes, b200_canny_frames_device and b200_cv_canny_frames_device) always take the list-driven
+//     pair, in a form that finds each entry's frame in the chunk's table (ccl_ragged_link / ccl_ragged_resolve; the link kernel
+//     has the same OpenCV switch, RaggedHystParams::opencv); the tile-based family below serves uniform batches only
 //     launches of the OpenCV-compatible path (HystParams::opencv) take the list-driven pair too, with plain 8-connectivity: no pair
 //     is left out and no one-way link is applied
 //   tile-based (stage API, minVal <= 0, maps with more than 1/8 weak pixels; reference semantics only):
@@ -517,6 +517,10 @@ __device__ __forceinline__ int ragged_frame_of(const RaggedHystParams& p, unsign
     return lo;
 }
 
+// OPENCV: cv::Canny's plain 8-connectivity (b200_cv_canny_frames_device), as in ccl_sparse_link_kernel: no pair is left out and the
+// last block only retires the counters.  It must not run the one-way fix-up anyway: that reads cls[1] and cls[cls_pitch], which a
+// 1-wide or 1-tall frame (accepted on that path) does not have.
+template <bool OPENCV>
 __global__ void __launch_bounds__(256)
 ccl_ragged_link_kernel(const RaggedHystParams p) {
     const unsigned int n = p.ctr[0];
@@ -529,8 +533,8 @@ ccl_ragged_link_kernel(const RaggedHystParams p) {
         const long long cp = fd.cls_pitch;
         const uint8_t* c = fd.cls + ((long long)y * cp + x);
         const bool has_n = y > 0, has_s = y + 1 < Hh, has_w = x > 0, has_e = x + 1 < W;
-        const bool q01 = (y == 0) && (x == 1);   // (0,1): its SW neighbour (1,0) is off limits
-        const bool q10 = (y == 1) && (x == 0);   // (1,0): its NE neighbour (0,1) is off limits
+        const bool q01 = !OPENCV && (y == 0) && (x == 1);   // (0,1): its SW neighbour (1,0) is off limits
+        const bool q10 = !OPENCV && (y == 1) && (x == 0);   // (1,0): its NE neighbour (0,1) is off limits
         const int c_nw = (has_n && has_w) ? c[-cp - 1] : 0;
         const int c_n = has_n ? c[-cp] : 0;
         const int c_ne = (has_n && has_e && !q10) ? c[-cp + 1] : 0;
@@ -558,7 +562,7 @@ ccl_ragged_link_kernel(const RaggedHystParams p) {
     __syncthreads();
     if (!s_last) return;
     __threadfence();
-    for (int f = threadIdx.x; f < p.n_frames; f += blockDim.x) {
+    for (int f = threadIdx.x; !OPENCV && f < p.n_frames; f += blockDim.x) {
         const RaggedFrame fd = p.frames[f];
         const int c01 = fd.cls[1], c10 = fd.cls[fd.cls_pitch];
         if (c10 == 1 && (c01 == 255 || (c01 == 1 && g_find_halve(p.parent, fd.base + 1) == kSuper)))
@@ -588,7 +592,7 @@ int launch_hysteresis_ragged(b200_ctx* ctx, cudaStream_t st, const RaggedHystPar
     const int grid = (int)std::min(cap, std::max(32LL, p.px / 16384));   // as sparse_grid()
     {
         ProfScope ps(ctx, st, 1);
-        ccl_ragged_link_kernel<<<grid, 256, 0, st>>>(p);
+        (p.opencv ? ccl_ragged_link_kernel<true> : ccl_ragged_link_kernel<false>)<<<grid, 256, 0, st>>>(p);
     }
     CB_CUDA(cudaGetLastError());
     ctx->launches++;

@@ -89,9 +89,10 @@ struct FrontParams {
                             // frame*out_frame_stride + (y - plane_row0)*width + x (strong pixels need no slot: they are final)
     uint32_t* kept_list;    // launch-relative indices of all weak pixels, in no particular order
     unsigned int* kept_count;  // number of entries: word 0 of the list's counter block (see HystParams::ctr); zero at launch
-    // ragged launches (front3's RAGGED variant, b200_canny_frames_device): the chunk's device table.  Work item blockIdx.x names a
-    // frame, a strip and a row band; the frame's descriptor replaces in / in_pitch / width / height / cls / cls_pitch / cls_words
-    // and the slot base, and its tensor map (TMA staging) replaces the `tmap` parameter.
+    // ragged launches (front3's RAGGED variant, b200_canny_frames_device; front_cv's, b200_cv_canny_frames_device): the chunk's device
+    // table.  Work item blockIdx.x names a frame, a strip and a row band (front_cv: one 128 x 64 tile); the frame's descriptor replaces
+    // in / in_pitch / width / height / cls / cls_pitch / cls_words and the slot base, and for front3 its tensor map (TMA staging)
+    // replaces the `tmap` parameter.
     const struct RaggedFrame* rframes;
     const struct RaggedItem* ritems;
     const CUtensorMap_st* rtmaps;
@@ -102,7 +103,8 @@ struct FrontParams {
 // indices stay dense and launch-relative: pixel (y, x) of the frame is slot base + y*width + x, base being the sum of h*w over
 // the frames before it in the chunk (ascending, below 2^31).
 struct RaggedFrame {
-    const uint8_t* in;      // gray input (a scratch plane for B,G,R lists)
+    const uint8_t* in;      // gray input (a scratch plane for B,G,R lists); for OpenCV-compatible lists (b200_cv_canny_frames_device)
+                            // the caller's frame itself, 1 or 3 interleaved bytes per pixel
     long long in_pitch;
     uint8_t* cls;           // the caller's output: class map, then 0 / 255
     long long cls_pitch;
@@ -127,6 +129,8 @@ struct RaggedHystParams {
     const uint32_t* list;
     unsigned int* ctr;      // the list's counter block (HystParams::ctr); h_kept is never written by ragged launches
     long long px;           // pixels of the chunk (sizes the grid)
+    int opencv;             // 1: cv::Canny's plain 8-connectivity, without the reference's one-way (0,1)/(1,0) link (as HystParams::opencv;
+                            // b200_cv_canny_frames_device)
 };
 
 // The input layout a TMA tensor map can describe: base, row pitch and frame stride on 16-byte boundaries, frames that do not
@@ -298,6 +302,10 @@ int launch_front3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, i
 // front_cv.cu (cv::Canny semantics, b200_cv_canny_device_strided): class map + weak-pixel list of p's frames, channels 1 or 3
 // interleaved, L1 or L2 magnitude against p.lo / p.hi (already floored and, for L2, squared)
 int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int channels, bool l2);
+// ragged chunks (b200_cv_canny_frames_device): the work items of one frame (its 128 x 64 tiles), and the launch over n_items items of
+// p.ritems with the frames of p.rframes
+void ragged_items_cv(int frame, int height, int width, std::vector<RaggedItem>& items);
+int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, int channels, bool l2);
 // selftest.cu
 int check_div_mode_device(b200_ctx* ctx, float b, float y, float* c, int* mode);
 // hysteresis.cu

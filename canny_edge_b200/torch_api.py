@@ -5,7 +5,8 @@ Any view whose rows are contiguous goes straight to the kernels with its strides
 kernels cannot address (rows that are not unit-stride, frames that overlap, broadcast frames) raise ValueError rather than being
 copied behind the caller's back.  canny_list / canny_bgr_list take a list of frames of different sizes in one call
 (b200_canny_frames_device).  cv_canny / cv_canny_color compute cv2.Canny's maps instead of the reference's
-(b200_cv_canny_device_strided), from the same kinds of views.
+(b200_cv_canny_device_strided), from the same kinds of views; cv_canny_list / cv_canny_color_list do so for lists of frames of
+different sizes (b200_cv_canny_frames_device).
 
 Work is issued on torch.cuda.current_stream(frames.device): the context is pointed at that stream on every call, so results are
 ordered with the caller's other torch work like any torch op.  When consecutive calls come from different streams, the later
@@ -17,7 +18,7 @@ import threading
 from typing import Dict, Optional, Tuple
 
 from .api import (Context, canny_batch_device_bgr_strided_ptr, canny_batch_device_strided_ptr, canny_frames_device_ptr,
-                  cv_canny_device_strided_ptr)
+                  cv_canny_device_strided_ptr, cv_canny_frames_device_ptr)
 
 _contexts: Dict[int, Context] = {}
 _contexts_lock = threading.Lock()
@@ -149,9 +150,11 @@ def cv_canny_color(frames, threshold1: float, threshold2: float, *, L2gradient: 
     return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient))
 
 
-def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool):
+def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool, cv_l2=None):
+    """cv_l2 as _run: None for the reference's Canny, False / True for cv2.Canny with L1 / L2 magnitude."""
     import torch
 
+    min_side = 2 if cv_l2 is None else 1
     frames = list(frames)
     if not frames:
         raise ValueError("empty frame list")
@@ -160,7 +163,7 @@ def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Option
     for i, f in enumerate(frames):
         if isinstance(f, torch.Tensor) and f.dim() != single:
             raise ValueError(f"frame {i}: expected one {'(H, W, 3) B,G,R' if bgr else '(H, W) gray'} frame, got shape {tuple(f.shape)}")
-        _, h, w, pitch, _ = frame_layout(f, bgr)
+        _, h, w, pitch, _ = frame_layout(f, bgr, min_side)
         descs.append([f.data_ptr(), pitch, 0, 0, h, w])
     if out is not None:
         out = list(out)
@@ -179,7 +182,7 @@ def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Option
     if out is None:
         out = [torch.empty((d[4], d[5]), dtype=torch.uint8, device=device) for d in descs]
     for d, o in zip(descs, out):
-        _, _, _, d[3], _ = frame_layout(o, False)
+        _, _, _, d[3], _ = frame_layout(o, False, min_side)
         d[2] = o.data_ptr()
     dev = device.index if device.index is not None else torch.cuda.current_device()
     if ctx is None:
@@ -188,7 +191,10 @@ def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Option
         raise ValueError(f"context is on cuda:{ctx.device}, frames on cuda:{dev}")
     with _call_lock, torch.cuda.device(dev):
         ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)
-        canny_frames_device_ptr(ctx, descs, sigma, min_val, max_val, bgr=bgr)
+        if cv_l2 is not None:
+            cv_canny_frames_device_ptr(ctx, descs, 3 if bgr else 1, min_val, max_val, cv_l2)
+        else:
+            canny_frames_device_ptr(ctx, descs, sigma, min_val, max_val, bgr=bgr)
     return out
 
 
@@ -204,3 +210,19 @@ def canny_bgr_list(frames, sigma: float, min_val: int, max_val: int, *, out=None
     """canny_list() for interleaved B,G,R frames: each element an (H, W, 3) view with each pixel's 3 bytes contiguous.  The gray
     conversion is OpenCV's COLOR_BGR2GRAY, bit for bit.  Returns a list of (H, W) maps."""
     return _run_list(frames, sigma, min_val, max_val, out, ctx, bgr=True)
+
+
+def cv_canny_list(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None, ctx: Optional[Context] = None):
+    """cv2.Canny(frame, threshold1, threshold2, L2gradient=L2gradient) (apertureSize 3) of a list of gray frames of different sizes,
+    in one call (b200_cv_canny_frames_device): each element a CUDA uint8 (H, W) view whose rows are contiguous, any row pitch, at
+    least 1 x 1.  Returns a list of uint8 (H, W) tensors holding 0 / 255 (`out` when given: a list of views of the same shapes, e.g.
+    tiles of one mosaic; only their elements are written).  Every map equals cv_canny() of that frame alone.  Asynchronous on
+    torch.cuda.current_stream(device); ctx defaults to the cached Context."""
+    return _run_list(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=False, cv_l2=bool(L2gradient))
+
+
+def cv_canny_color_list(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None,
+                        ctx: Optional[Context] = None):
+    """cv_canny_list() for 3-channel frames: each element an (H, W, 3) view with each pixel's 3 bytes contiguous.  Every map equals
+    cv_canny_color() of that frame alone.  Returns a list of (H, W) maps."""
+    return _run_list(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient))

@@ -237,7 +237,8 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
  * Before any device work: B200_ERR_UNSUPPORTED for channels other than 1 and 3 or a height above 4 194 240 (65535 x 64) rows;
  * B200_ERR_INVALID_ARG for a NaN or infinite threshold; B200_ERR_UNSUPPORTED for a threshold whose floor (after the L2 squaring)
  * does not fit in int32, where OpenCV's own conversion overflows; then the layout checks of b200_canny_batch_device_strided (in_row_pitch >= channels*width), except that
- * frames of 1 pixel per side are accepted. */
+ * frames of 1 pixel per side are accepted.
+ * Frames of different sizes in one call: b200_cv_canny_frames_device, below b200_frame. */
 int b200_cv_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride, int n_frames,
                                  int height, int width, int channels, double threshold1, double threshold2, int l2_gradient,
                                  uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
@@ -264,6 +265,22 @@ typedef struct b200_frame {
 } b200_frame;
 int b200_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val);
 int b200_canny_frames_device_bgr(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val);
+
+/* cv2.Canny(frame_i, threshold1, threshold2, apertureSize=3, L2gradient=l2_gradient) of a list of frames of different sizes in one
+ * call: b200_cv_canny_device_strided's semantics with b200_canny_frames_device's lists (a dataset of photos of many sizes, prepared
+ * for an edge-conditioned model).  Frame i's map is bit for bit the one b200_cv_canny_device_strided gives for that frame alone.
+ *   pixel (y, x) of frame i is the `channels` bytes (1 or 3 interleaved) at in + y*in_row_pitch + channels*x, and its 0 / 255 result
+ *   is written to out + y*out_row_pitch + x.  No other output byte is written.
+ * Frames of any size from 1 x 1 up; no limit on the height beyond the 2^31 pixels below.  `frames` is host memory, read only during
+ * the call.  Chunks (about 75 Mpix, b200_ctx_set_chunk_frames), stream slots and asynchrony as b200_canny_frames_device.
+ * Before any device work, in this order: B200_ERR_UNSUPPORTED for channels other than 1 and 3; the threshold checks of
+ * b200_cv_canny_device_strided (B200_ERR_INVALID_ARG for NaN or inf, B200_ERR_UNSUPPORTED for a floor outside int32); then the list
+ * checks of b200_canny_frames_device with `channels` bytes per input pixel and frames from 1 x 1: B200_ERR_INVALID_ARG for a null
+ * `frames`, `in` or `out`, n_frames <= 0, an empty frame, a negative pitch or one below a row (channels*width input bytes, width
+ * output bytes), an extent above 2^48 bytes, an output extent that overlaps any input extent or any other output extent (inputs may
+ * overlap); B200_ERR_UNSUPPORTED for a frame of 2^31 pixels or more. */
+int b200_cv_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
+                                double threshold2, int l2_gradient);
 
 /* The packed form of an edge map — 1 bit per pixel, bit i of byte k <-> pixel 8k+i, ceil(n_px/32)*4 bytes — is what
  * b200_canny_batch_host moves over PCIe.  Both halves are exported for callers that store or ship maps in that form:

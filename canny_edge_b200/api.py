@@ -225,13 +225,15 @@ def canny_batch_device_bgr_strided_ptr(ctx: Optional[Context], d_bgr: int, in_ro
 
 def cv_canny_device_strided_ptr(ctx: Optional[Context], d_in: int, in_row_pitch: int, in_frame_stride: int, n: int, h: int, w: int,
                                 channels: int, threshold1: float, threshold2: float, l2_gradient: bool, d_edges: int,
-                                out_row_pitch: int, out_frame_stride: int) -> None:
-    """cv2.Canny(frame, threshold1, threshold2, L2gradient=l2_gradient) of every frame, bit for bit (b200_cv_canny_device_strided):
-    1 or 3 interleaved channels, pixel (f, y, x) read at d_in + f*in_frame_stride + y*in_row_pitch + channels*x, its 0 / 255
-    result written at d_edges + f*out_frame_stride + y*out_row_pitch + x.  Asynchronous on the context's stream."""
-    check(load().b200_cv_canny_device_strided(_h(ctx), C.c_void_p(d_in), int(in_row_pitch), int(in_frame_stride), n, h, w,
-                                              int(channels), C.c_double(threshold1), C.c_double(threshold2), int(bool(l2_gradient)),
-                                              C.c_void_p(d_edges), int(out_row_pitch), int(out_frame_stride)))
+                                out_row_pitch: int, out_frame_stride: int, aperture_size: int = 3) -> None:
+    """cv2.Canny(frame, threshold1, threshold2, apertureSize=aperture_size, L2gradient=l2_gradient) of every frame, bit for bit
+    (b200_cv_canny_aperture_device_strided; aperture_size 3, 5 or 7): 1 or 3 interleaved channels, pixel (f, y, x) read at
+    d_in + f*in_frame_stride + y*in_row_pitch + channels*x, its 0 / 255 result written at d_edges + f*out_frame_stride +
+    y*out_row_pitch + x.  Asynchronous on the context's stream."""
+    check(load().b200_cv_canny_aperture_device_strided(_h(ctx), C.c_void_p(d_in), int(in_row_pitch), int(in_frame_stride), n, h, w,
+                                                       int(channels), C.c_double(threshold1), C.c_double(threshold2),
+                                                       int(aperture_size), int(bool(l2_gradient)), C.c_void_p(d_edges),
+                                                       int(out_row_pitch), int(out_frame_stride)))
 
 
 def frame_list(descs) -> C.Array:
@@ -253,14 +255,14 @@ def canny_frames_device_ptr(ctx: Optional[Context], descs, sigma: float, min_val
 
 
 def cv_canny_frames_device_ptr(ctx: Optional[Context], descs, channels: int, threshold1: float, threshold2: float,
-                               l2_gradient: bool) -> None:
-    """cv2.Canny(frame, threshold1, threshold2, L2gradient=l2_gradient) of frames of different sizes in one call, bit for bit
-    (b200_cv_canny_frames_device).  descs as canny_frames_device_ptr: pixel (y, x) of a frame is the `channels` bytes (1 or 3
-    interleaved) at in_ptr + y*in_pitch + channels*x, its 0 / 255 result written at out_ptr + y*out_pitch + x; frames from 1 x 1.
-    Asynchronous on the context's stream."""
+                               l2_gradient: bool, aperture_size: int = 3) -> None:
+    """cv2.Canny(frame, threshold1, threshold2, apertureSize=aperture_size, L2gradient=l2_gradient) of frames of different sizes in
+    one call, bit for bit (b200_cv_canny_aperture_frames_device; aperture_size 3, 5 or 7).  descs as canny_frames_device_ptr: pixel
+    (y, x) of a frame is the `channels` bytes (1 or 3 interleaved) at in_ptr + y*in_pitch + channels*x, its 0 / 255 result written
+    at out_ptr + y*out_pitch + x; frames from 1 x 1.  Asynchronous on the context's stream."""
     descs = list(descs)
-    check(load().b200_cv_canny_frames_device(_h(ctx), frame_list(descs), len(descs), int(channels), C.c_double(threshold1),
-                                             C.c_double(threshold2), int(bool(l2_gradient))))
+    check(load().b200_cv_canny_aperture_frames_device(_h(ctx), frame_list(descs), len(descs), int(channels), C.c_double(threshold1),
+                                                      C.c_double(threshold2), int(aperture_size), int(bool(l2_gradient))))
 
 
 def synth_host(n: int, h: int, w: int, kind: int = 0, seed: int = 1234, first_frame: int = 0) -> np.ndarray:

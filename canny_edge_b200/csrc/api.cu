@@ -1,5 +1,6 @@
 // api.cu — the extern "C" boundary (include/canny_b200.h): context, workspace pool, Gaussian tables,
 // stage entry points on host buffers, batched device/host pipelines.
+#include <limits.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -392,12 +393,13 @@ static bool bgr_fused_ok(const b200_ctx* ctx, const uint8_t* d_bgr, int n, int h
     return front3_bgr_supports(ctx->gauss, fp);
 }
 
-// The OpenCV-compatible path (b200_cv_canny_device_strided): cv::Canny's thresholds as integers in magnitude space (swapped,
-// clamped and squared for L2, floored) and the input's channel count
+// The OpenCV-compatible path (b200_cv_canny_aperture_device_strided): cv::Canny's thresholds as integers in magnitude space
+// (divided by 16 for aperture 7, swapped, clamped and squared for L2, floored), the input's channel count and the Sobel aperture
 struct CvSpec {
     int lo, hi;
     int channels;
     bool l2;
+    int aperture;   // 3, 5 or 7
 };
 
 // Front + hysteresis with cv::Canny's semantics on frames [f0, f0+nf) of slot `slot` (run_frames_device's counterpart): the
@@ -418,7 +420,7 @@ static int run_frames_cv(b200_ctx* ctx, cudaStream_t st, int slot, const uint8_t
     // the list's counter block is zero here (see run_frames_device)
     if (ctx->list_dirty[slot]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
     ctx->list_dirty[slot] = true;
-    CB_TRY(launch_front_cv(ctx, st, fp, cv.channels, cv.l2));
+    CB_TRY(launch_front_cv(ctx, st, fp, cv.channels, cv.l2, cv.aperture));
     HystParams hp;
     memset(&hp, 0, sizeof(hp));
     hp.cls = d_out; hp.cls_pitch = lay.out_pitch; hp.cls_frame_stride = lay.out_frame_stride;
@@ -980,13 +982,15 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
 }
 
 // ---- cv::Canny semantics ----------------------------------------------------------------------------------
-// Thresholds as cv::Canny uses them (imgproc/src/canny.cpp): swapped when low > high; for L2 clamped to 32767 and squared when
-// positive; floored.  NaN / inf: B200_ERR_INVALID_ARG.  A floor outside int32: B200_ERR_UNSUPPORTED (OpenCV's cvFloor overflows
-// there and its result is not the comparison the thresholds describe).
+// Thresholds as cv::Canny uses them (imgproc/src/canny.cpp): divided by 16 for aperture 7 (whose derivatives are scaled by 1/16)
+// before anything else; swapped when low > high; for L2 clamped to 32767 and squared when positive; floored.  NaN / inf:
+// B200_ERR_INVALID_ARG.  A floor outside int32: B200_ERR_UNSUPPORTED (OpenCV's cvFloor overflows there and its result is not the
+// comparison the thresholds describe).
 constexpr int kCvMaxHeight = 65535 * 64;   // the OpenCV front kernel's grid: one row of CTAs per 64 rows, gridDim.y <= 65535
 
-static int cv_thresholds(double t1, double t2, bool l2, int* lo, int* hi) {
+static int cv_thresholds(double t1, double t2, bool l2, int aperture, int* lo, int* hi) {
     if (!isfinite(t1) || !isfinite(t2)) { set_error("thresholds must be finite (got %g, %g)", t1, t2); return B200_ERR_INVALID_ARG; }
+    if (aperture == 7) { t1 /= 16; t2 /= 16; }
     double a = std::min(t1, t2), b = std::max(t1, t2);
     if (l2) {
         a = std::min(32767.0, a); b = std::min(32767.0, b);
@@ -1003,17 +1007,36 @@ static int cv_thresholds(double t1, double t2, bool l2, int* lo, int* hi) {
     return B200_OK;
 }
 
+// The checks of the OpenCV calls that come before the layout's: channel count (UNSUPPORTED), aperture (INVALID_ARG, as cv::Canny
+// rejects it), the uniform call's height (max_height; UNSUPPORTED), thresholds
+static int cv_spec(int channels, int aperture, int height, int max_height, double t1, double t2, int l2_gradient, CvSpec* cv) {
+    if (channels != 1 && channels != 3) { set_error("channels must be 1 or 3 (got %d)", channels); return B200_ERR_UNSUPPORTED; }
+    if (aperture != 3 && aperture != 5 && aperture != 7) {
+        set_error("aperture size must be 3, 5 or 7 (got %d)", aperture);
+        return B200_ERR_INVALID_ARG;
+    }
+    if (height > max_height) { set_error("height %d: at most %d rows (65535 tiles of 64)", height, max_height); return B200_ERR_UNSUPPORTED; }
+    cv->channels = channels;
+    cv->l2 = l2_gradient != 0;
+    cv->aperture = aperture;
+    return cv_thresholds(t1, t2, cv->l2, aperture, &cv->lo, &cv->hi);
+}
+
+int b200_cv_canny_aperture_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride,
+                                          int n_frames, int height, int width, int channels, double threshold1, double threshold2,
+                                          int aperture_size, int l2_gradient, uint8_t* d_edges, int64_t out_row_pitch,
+                                          int64_t out_frame_stride) {
+    CvSpec cv;
+    CB_TRY(cv_spec(channels, aperture_size, height, kCvMaxHeight, threshold1, threshold2, l2_gradient, &cv));
+    return batch_device_impl(ctx, d_in, in_row_pitch, in_frame_stride, n_frames, height, width, 0.f, 0, 0, d_edges, out_row_pitch,
+                             out_frame_stride, channels, &cv);
+}
+
 int b200_cv_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride, int n_frames,
                                  int height, int width, int channels, double threshold1, double threshold2, int l2_gradient,
                                  uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride) {
-    if (channels != 1 && channels != 3) { set_error("channels must be 1 or 3 (got %d)", channels); return B200_ERR_UNSUPPORTED; }
-    if (height > kCvMaxHeight) { set_error("height %d: at most %d rows (65535 tiles of 64)", height, kCvMaxHeight); return B200_ERR_UNSUPPORTED; }
-    CvSpec cv;
-    cv.channels = channels;
-    cv.l2 = l2_gradient != 0;
-    CB_TRY(cv_thresholds(threshold1, threshold2, cv.l2, &cv.lo, &cv.hi));
-    return batch_device_impl(ctx, d_in, in_row_pitch, in_frame_stride, n_frames, height, width, 0.f, 0, 0, d_edges, out_row_pitch,
-                             out_frame_stride, channels, &cv);
+    return b200_cv_canny_aperture_device_strided(ctx, d_in, in_row_pitch, in_frame_stride, n_frames, height, width, channels, threshold1,
+                                                 threshold2, 3, l2_gradient, d_edges, out_row_pitch, out_frame_stride);
 }
 
 // ---- ragged lists: frames of different sizes in one call ------------------------------------------------
@@ -1231,7 +1254,7 @@ static int run_ragged_cv_chunk(b200_ctx* ctx, cudaStream_t st, int s, const b200
     // the list's counter block is zero here (see run_frames_device)
     if (ctx->list_dirty[s]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
     ctx->list_dirty[s] = true;
-    CB_TRY(launch_front_cv_ragged(ctx, st, fp, (int)items.size(), cv.channels, cv.l2));
+    CB_TRY(launch_front_cv_ragged(ctx, st, fp, (int)items.size(), cv.channels, cv.l2, cv.aperture));
     RaggedHystParams hp;
     memset(&hp, 0, sizeof(hp));
     hp.frames = fp.rframes;
@@ -1316,14 +1339,17 @@ int b200_canny_frames_device_bgr(b200_ctx* ctx, const b200_frame* frames, int n_
     return frames_device_impl(ctx, frames, n_frames, sigma, min_val, max_val, 3);
 }
 
+int b200_cv_canny_aperture_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
+                                         double threshold2, int aperture_size, int l2_gradient) {
+    CvSpec cv;
+    // a list's 1-D grid has no height limit
+    CB_TRY(cv_spec(channels, aperture_size, 0, INT_MAX, threshold1, threshold2, l2_gradient, &cv));
+    return frames_device_impl(ctx, frames, n_frames, 0.f, 0, 0, channels, &cv);
+}
+
 int b200_cv_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
                                 double threshold2, int l2_gradient) {
-    if (channels != 1 && channels != 3) { set_error("channels must be 1 or 3 (got %d)", channels); return B200_ERR_UNSUPPORTED; }
-    CvSpec cv;
-    cv.channels = channels;
-    cv.l2 = l2_gradient != 0;
-    CB_TRY(cv_thresholds(threshold1, threshold2, cv.l2, &cv.lo, &cv.hi));
-    return frames_device_impl(ctx, frames, n_frames, 0.f, 0, 0, channels, &cv);
+    return b200_cv_canny_aperture_frames_device(ctx, frames, n_frames, channels, threshold1, threshold2, 3, l2_gradient);
 }
 
 // Host buffers in, host buffers out: frames -> 0 / 255 edge maps, as bytes (edges8) or as the reference's int16 (edges16).

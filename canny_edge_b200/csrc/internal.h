@@ -299,13 +299,14 @@ int ragged_band_rows3(const b200_ctx* ctx, const int* heights, const int* widths
 void ragged_items3(int frame, int height, int width, int band_rows, std::vector<RaggedItem>& items);
 int ragged_tensor_map3(const uint8_t* in, long long pitch, int height, int width, int radius, CUtensorMap_st* tmap, bool* use_tma);
 int launch_front3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, bool use_tma);
-// front_cv.cu (cv::Canny semantics, b200_cv_canny_device_strided): class map + weak-pixel list of p's frames, channels 1 or 3
-// interleaved, L1 or L2 magnitude against p.lo / p.hi (already floored and, for L2, squared)
-int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int channels, bool l2);
-// ragged chunks (b200_cv_canny_frames_device): the work items of one frame (its 128 x 64 tiles), and the launch over n_items items of
+// front_cv.cu (cv::Canny semantics, b200_cv_canny_aperture_device_strided): class map + weak-pixel list of p's frames, channels 1 or
+// 3 interleaved, Sobel aperture 3, 5 or 7, L1 or L2 magnitude against p.lo / p.hi (already divided for aperture 7, floored and, for
+// L2, squared)
+int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int channels, bool l2, int aperture);
+// ragged chunks (b200_cv_canny_aperture_frames_device): the work items of one frame (its 128 x 64 tiles), and the launch over n_items items of
 // p.ritems with the frames of p.rframes
 void ragged_items_cv(int frame, int height, int width, std::vector<RaggedItem>& items);
-int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, int channels, bool l2);
+int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, int channels, bool l2, int aperture);
 // selftest.cu
 int check_div_mode_device(b200_ctx* ctx, float b, float y, float* c, int* mode);
 // hysteresis.cu

@@ -5,8 +5,8 @@ Any view whose rows are contiguous goes straight to the kernels with its strides
 kernels cannot address (rows that are not unit-stride, frames that overlap, broadcast frames) raise ValueError rather than being
 copied behind the caller's back.  canny_list / canny_bgr_list take a list of frames of different sizes in one call
 (b200_canny_frames_device).  cv_canny / cv_canny_color compute cv2.Canny's maps instead of the reference's
-(b200_cv_canny_device_strided), from the same kinds of views; cv_canny_list / cv_canny_color_list do so for lists of frames of
-different sizes (b200_cv_canny_frames_device).
+(b200_cv_canny_aperture_device_strided; apertureSize 3, 5 or 7), from the same kinds of views; cv_canny_list / cv_canny_color_list
+do so for lists of frames of different sizes (b200_cv_canny_aperture_frames_device).
 
 Work is issued on torch.cuda.current_stream(frames.device): the context is pointed at that stream on every call, so results are
 ordered with the caller's other torch work like any torch op.  When consecutive calls come from different streams, the later
@@ -80,9 +80,9 @@ def _context(device_index: int) -> Context:
         return ctx
 
 
-def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool, cv_l2=None):
-    """cv_l2 None: the reference's Canny (sigma, min_val, max_val); False / True: cv2.Canny with L1 / L2 magnitude, min_val and
-    max_val being threshold1 and threshold2."""
+def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool, cv_l2=None, aperture: int = 3):
+    """cv_l2 None: the reference's Canny (sigma, min_val, max_val); False / True: cv2.Canny with L1 / L2 magnitude and Sobel
+    aperture `aperture`, min_val and max_val being threshold1 and threshold2."""
     import torch
 
     min_side = 2 if cv_l2 is None else 1
@@ -109,7 +109,7 @@ def _run(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Co
         ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)
         if cv_l2 is not None:
             cv_canny_device_strided_ptr(ctx, frames.data_ptr(), in_pitch, in_fs, n, h, w, 3 if bgr else 1, min_val, max_val, cv_l2,
-                                        out.data_ptr(), out_pitch, out_fs)
+                                        out.data_ptr(), out_pitch, out_fs, aperture)
         else:
             call = canny_batch_device_bgr_strided_ptr if bgr else canny_batch_device_strided_ptr
             call(ctx, frames.data_ptr(), in_pitch, in_fs, n, h, w, sigma, min_val, max_val, out.data_ptr(), out_pitch, out_fs)
@@ -130,28 +130,33 @@ def canny_bgr(frames, sigma: float, min_val: int, max_val: int, *, out=None, ctx
     return _run(frames, sigma, min_val, max_val, out, ctx, bgr=True)
 
 
-def cv_canny(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None, ctx: Optional[Context] = None):
-    """cv2.Canny(frame, threshold1, threshold2, L2gradient=L2gradient) (apertureSize 3) of gray frames, bit for bit: a CUDA uint8
-    tensor of shape (H, W) or (N, H, W), any strides with contiguous rows, frames of at least 1 x 1.
+def cv_canny(frames, threshold1: float, threshold2: float, *, apertureSize: int = 3, L2gradient: bool = False, out=None,
+             ctx: Optional[Context] = None):
+    """cv2.Canny(frame, threshold1, threshold2, apertureSize=apertureSize, L2gradient=L2gradient) of gray frames, bit for bit: a
+    CUDA uint8 tensor of shape (H, W) or (N, H, W), any strides with contiguous rows, frames of at least 1 x 1.
 
-    No blur, Sobel with replicated borders, L1 (or L2) magnitude, OpenCV's direction test and non-maximum suppression, `> low` /
-    `> high` thresholds (swapped when threshold1 > threshold2), plain 8-connected hysteresis.  Returns a uint8 tensor of the same
-    shape holding 0 / 255 (`out` when given, which may be a strided view).  Asynchronous on torch.cuda.current_stream(frames.device);
-    ctx defaults to one cached Context per device."""
-    return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=False, cv_l2=bool(L2gradient))
+    No blur, Sobel of apertureSize 3, 5 or 7 with replicated borders (7: derivatives and thresholds scaled by 1/16, as cv2 does),
+    L1 (or L2) magnitude, OpenCV's direction test and non-maximum suppression, `> low` / `> high` thresholds (swapped when
+    threshold1 > threshold2), plain 8-connected hysteresis.  Any other apertureSize raises CannyB200Error, as cv2 rejects it.
+    Returns a uint8 tensor of the same shape holding 0 / 255 (`out` when given, which may be a strided view).  Asynchronous on
+    torch.cuda.current_stream(frames.device); ctx defaults to one cached Context per device."""
+    return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=False, cv_l2=bool(L2gradient),
+                aperture=int(apertureSize))
 
 
-def cv_canny_color(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None,
+def cv_canny_color(frames, threshold1: float, threshold2: float, *, apertureSize: int = 3, L2gradient: bool = False, out=None,
                    ctx: Optional[Context] = None):
     """cv2.Canny of 3-channel frames, bit for bit: (H, W, 3) or (N, H, W, 3), each pixel's 3 bytes contiguous, rows and frames with
-    any stride.  As cv2.Canny on a 3-channel image: the gradient of every channel, per pixel the channel of largest magnitude.  The
-    channel order does not matter (B,G,R or R,G,B give the same map except where two channels tie, when the first wins).
-    Returns (H, W) or (N, H, W)."""
-    return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient))
+    any stride; apertureSize 3, 5 or 7.  As cv2.Canny on a 3-channel image: the gradient of every channel, per pixel the channel
+    of largest magnitude.  The channel order does not matter (B,G,R or R,G,B give the same map except where two channels tie,
+    when the first wins).  Returns (H, W) or (N, H, W)."""
+    return _run(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient),
+                aperture=int(apertureSize))
 
 
-def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool, cv_l2=None):
-    """cv_l2 as _run: None for the reference's Canny, False / True for cv2.Canny with L1 / L2 magnitude."""
+def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Optional[Context], bgr: bool, cv_l2=None,
+              aperture: int = 3):
+    """cv_l2 and aperture as _run: cv_l2 None for the reference's Canny, False / True for cv2.Canny with L1 / L2 magnitude."""
     import torch
 
     min_side = 2 if cv_l2 is None else 1
@@ -192,7 +197,7 @@ def _run_list(frames, sigma: float, min_val: int, max_val: int, out, ctx: Option
     with _call_lock, torch.cuda.device(dev):
         ctx.set_stream(torch.cuda.current_stream(dev).cuda_stream or _CUDA_STREAM_LEGACY)
         if cv_l2 is not None:
-            cv_canny_frames_device_ptr(ctx, descs, 3 if bgr else 1, min_val, max_val, cv_l2)
+            cv_canny_frames_device_ptr(ctx, descs, 3 if bgr else 1, min_val, max_val, cv_l2, aperture)
         else:
             canny_frames_device_ptr(ctx, descs, sigma, min_val, max_val, bgr=bgr)
     return out
@@ -212,17 +217,20 @@ def canny_bgr_list(frames, sigma: float, min_val: int, max_val: int, *, out=None
     return _run_list(frames, sigma, min_val, max_val, out, ctx, bgr=True)
 
 
-def cv_canny_list(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None, ctx: Optional[Context] = None):
-    """cv2.Canny(frame, threshold1, threshold2, L2gradient=L2gradient) (apertureSize 3) of a list of gray frames of different sizes,
-    in one call (b200_cv_canny_frames_device): each element a CUDA uint8 (H, W) view whose rows are contiguous, any row pitch, at
-    least 1 x 1.  Returns a list of uint8 (H, W) tensors holding 0 / 255 (`out` when given: a list of views of the same shapes, e.g.
+def cv_canny_list(frames, threshold1: float, threshold2: float, *, apertureSize: int = 3, L2gradient: bool = False, out=None,
+                  ctx: Optional[Context] = None):
+    """cv2.Canny(frame, threshold1, threshold2, apertureSize=apertureSize, L2gradient=L2gradient) of a list of gray frames of
+    different sizes, in one call (b200_cv_canny_aperture_frames_device; apertureSize 3, 5 or 7, anything else raises
+    CannyB200Error): each element a CUDA uint8 (H, W) view whose rows are contiguous, any row pitch, at least 1 x 1.  Returns a list of uint8 (H, W) tensors holding 0 / 255 (`out` when given: a list of views of the same shapes, e.g.
     tiles of one mosaic; only their elements are written).  Every map equals cv_canny() of that frame alone.  Asynchronous on
     torch.cuda.current_stream(device); ctx defaults to the cached Context."""
-    return _run_list(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=False, cv_l2=bool(L2gradient))
+    return _run_list(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=False, cv_l2=bool(L2gradient),
+                     aperture=int(apertureSize))
 
 
-def cv_canny_color_list(frames, threshold1: float, threshold2: float, *, L2gradient: bool = False, out=None,
-                        ctx: Optional[Context] = None):
-    """cv_canny_list() for 3-channel frames: each element an (H, W, 3) view with each pixel's 3 bytes contiguous.  Every map equals
-    cv_canny_color() of that frame alone.  Returns a list of (H, W) maps."""
-    return _run_list(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient))
+def cv_canny_color_list(frames, threshold1: float, threshold2: float, *, apertureSize: int = 3, L2gradient: bool = False,
+                        out=None, ctx: Optional[Context] = None):
+    """cv_canny_list() for 3-channel frames: each element an (H, W, 3) view with each pixel's 3 bytes contiguous; apertureSize 3,
+    5 or 7.  Every map equals cv_canny_color() of that frame alone.  Returns a list of (H, W) maps."""
+    return _run_list(frames, 0.0, float(threshold1), float(threshold2), out, ctx, bgr=True, cv_l2=bool(L2gradient),
+                     aperture=int(apertureSize))

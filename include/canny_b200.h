@@ -213,11 +213,12 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
                                         int n_frames, int height, int width, float sigma, int min_val, int max_val,
                                         uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
 
-/* OpenCV semantics: the edge maps of cv::Canny(image, edges, threshold1, threshold2, 3, l2_gradient) (OpenCV 4.x), bit for bit,
- * for 8-bit frames with 1 channel or 3 interleaved channels (in any order: B,G,R as cv::Mat holds them, R,G,B, ...), any size of at
- * least 1 x 1.  The entry points above compute the reference's Canny instead; the differences:
+/* OpenCV semantics: the edge maps of cv::Canny(image, edges, threshold1, threshold2, aperture_size, l2_gradient) (OpenCV 4.x), bit
+ * for bit, for 8-bit frames with 1 channel or 3 interleaved channels (in any order: B,G,R as cv::Mat holds them, R,G,B, ...), any
+ * size of at least 1 x 1.  The entry points above compute the reference's Canny instead; the differences:
  *   blur            reference: Gaussian from sigma, renormalised at borders      here: none
- *   gradient        reference: Sobel, replicate for gx, drop for gy                here: Sobel 3x3, BORDER_REPLICATE for both
+ *   gradient        reference: Sobel, replicate for gx, drop for gy                here: Sobel of aperture_size 3, 5 or 7,
+ *                                                                                        BORDER_REPLICATE for both
  *   magnitude       reference: floor(sqrt(gx^2 + gy^2))                            here: |dx| + |dy|, or dx^2 + dy^2 against squared
  *                                                                                        thresholds when l2_gradient != 0
  *   direction, NMS  reference: atan2 bins, `>` on both sides                       here: fixed-point tan 22.5 deg (13573 / 2^15),
@@ -234,11 +235,23 @@ int b200_canny_batch_device_bgr_strided(b200_ctx* ctx, const uint8_t* d_bgr, int
  * y*in_row_pitch + channels*x, and its 0 / 255 result is written to d_edges + f*out_frame_stride + y*out_row_pitch + x; no other
  * byte of d_edges is written.  Chunks, stream slots and b200_ctx_set_chunk_frames as the batch calls.  Asynchronous on the
  * context's stream.
- * Before any device work: B200_ERR_UNSUPPORTED for channels other than 1 and 3 or a height above 4 194 240 (65535 x 64) rows;
- * B200_ERR_INVALID_ARG for a NaN or infinite threshold; B200_ERR_UNSUPPORTED for a threshold whose floor (after the L2 squaring)
- * does not fit in int32, where OpenCV's own conversion overflows; then the layout checks of b200_canny_batch_device_strided (in_row_pitch >= channels*width), except that
- * frames of 1 pixel per side are accepted.
- * Frames of different sizes in one call: b200_cv_canny_frames_device, below b200_frame. */
+ * Apertures, as cv::getDerivKernels builds them (dx: derivative taps across columns, smoothing taps down rows; dy: the transpose):
+ *   3: smoothing 1 2 1, derivative -1 0 1;
+ *   5: smoothing 1 4 6 4 1, derivative -1 -2 0 2 1; exact integers, |dx|, |dy| <= 12240;
+ *   7: smoothing 1 6 15 20 15 6 1, derivative -1 -4 -5 0 5 4 1; both derivatives are scaled by 1/16 and rounded half to even
+ *      (cvRound), |dx|, |dy| <= 10200, and both thresholds are divided by 16 before the swap, the L2 clamp, the squaring and the
+ *      floor (so the int32 check below applies to the divided value).
+ * Before any device work, in this order: B200_ERR_UNSUPPORTED for channels other than 1 and 3; B200_ERR_INVALID_ARG for an
+ * aperture_size other than 3, 5 and 7 (cv::Canny rejects those too); B200_ERR_UNSUPPORTED for a height above 4 194 240 (65535 x 64)
+ * rows; B200_ERR_INVALID_ARG for a NaN or infinite threshold; B200_ERR_UNSUPPORTED for a threshold whose floor (after the L2
+ * squaring) does not fit in int32, where OpenCV's own conversion overflows; then the layout checks of
+ * b200_canny_batch_device_strided (in_row_pitch >= channels*width), except that frames of 1 pixel per side are accepted.
+ * b200_cv_canny_device_strided is the same call with aperture_size 3.
+ * Frames of different sizes in one call: b200_cv_canny_aperture_frames_device, below b200_frame. */
+int b200_cv_canny_aperture_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride,
+                                          int n_frames, int height, int width, int channels, double threshold1, double threshold2,
+                                          int aperture_size, int l2_gradient, uint8_t* d_edges, int64_t out_row_pitch,
+                                          int64_t out_frame_stride);
 int b200_cv_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride, int n_frames,
                                  int height, int width, int channels, double threshold1, double threshold2, int l2_gradient,
                                  uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
@@ -266,19 +279,24 @@ typedef struct b200_frame {
 int b200_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val);
 int b200_canny_frames_device_bgr(b200_ctx* ctx, const b200_frame* frames, int n_frames, float sigma, int min_val, int max_val);
 
-/* cv2.Canny(frame_i, threshold1, threshold2, apertureSize=3, L2gradient=l2_gradient) of a list of frames of different sizes in one
- * call: b200_cv_canny_device_strided's semantics with b200_canny_frames_device's lists (a dataset of photos of many sizes, prepared
- * for an edge-conditioned model).  Frame i's map is bit for bit the one b200_cv_canny_device_strided gives for that frame alone.
+/* cv2.Canny(frame_i, threshold1, threshold2, apertureSize=aperture_size, L2gradient=l2_gradient) of a list of frames of different
+ * sizes in one call: b200_cv_canny_aperture_device_strided's semantics with b200_canny_frames_device's lists (a dataset of photos of
+ * many sizes, prepared for an edge-conditioned model).  Frame i's map is bit for bit the one b200_cv_canny_aperture_device_strided
+ * gives for that frame alone.
  *   pixel (y, x) of frame i is the `channels` bytes (1 or 3 interleaved) at in + y*in_row_pitch + channels*x, and its 0 / 255 result
  *   is written to out + y*out_row_pitch + x.  No other output byte is written.
  * Frames of any size from 1 x 1 up; no limit on the height beyond the 2^31 pixels below.  `frames` is host memory, read only during
  * the call.  Chunks (about 75 Mpix, b200_ctx_set_chunk_frames), stream slots and asynchrony as b200_canny_frames_device.
- * Before any device work, in this order: B200_ERR_UNSUPPORTED for channels other than 1 and 3; the threshold checks of
- * b200_cv_canny_device_strided (B200_ERR_INVALID_ARG for NaN or inf, B200_ERR_UNSUPPORTED for a floor outside int32); then the list
+ * Before any device work, in this order: B200_ERR_UNSUPPORTED for channels other than 1 and 3; B200_ERR_INVALID_ARG for an
+ * aperture_size other than 3, 5 and 7; the threshold checks of b200_cv_canny_aperture_device_strided (B200_ERR_INVALID_ARG for NaN
+ * or inf, B200_ERR_UNSUPPORTED for a floor outside int32, after the division for aperture 7); then the list
  * checks of b200_canny_frames_device with `channels` bytes per input pixel and frames from 1 x 1: B200_ERR_INVALID_ARG for a null
  * `frames`, `in` or `out`, n_frames <= 0, an empty frame, a negative pitch or one below a row (channels*width input bytes, width
  * output bytes), an extent above 2^48 bytes, an output extent that overlaps any input extent or any other output extent (inputs may
- * overlap); B200_ERR_UNSUPPORTED for a frame of 2^31 pixels or more. */
+ * overlap); B200_ERR_UNSUPPORTED for a frame of 2^31 pixels or more.
+ * b200_cv_canny_frames_device is the same call with aperture_size 3. */
+int b200_cv_canny_aperture_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
+                                         double threshold2, int aperture_size, int l2_gradient);
 int b200_cv_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
                                 double threshold2, int l2_gradient);
 

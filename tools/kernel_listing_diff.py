@@ -1,6 +1,7 @@
 """Compares two builds of libcanny_b200.so kernel by kernel (runs on the CPU box; needs cuobjdump):
   * ptxas resources (registers, stack, spills, static shared memory) from the output of `python -m canny_edge_b200.build --force -v`;
-  * the `cuobjdump -sass` listing of every function, without the `identifier =` lines (the source path of each cubin).
+  * the `cuobjdump -sass` listing of every function, without the `identifier =` lines (the source path of each cubin) and with runs
+    of blanks collapsed (cuobjdump pads its columns to the widest instruction of the cubin, which a new kernel can change).
 A kernel that gained a template parameter keeps its code under a new mangled name: --rename OLD=NEW (substrings of the mangled
 names) pairs the parent's kernel with the new instantiation it must still equal.
     python tools/kernel_listing_diff.py PARENT.so PARENT_BUILD.txt NEW.so NEW_BUILD.txt [--rename OLD=NEW ...] > profiles/...txt
@@ -55,7 +56,7 @@ def sass(so):
             funcs[cur] = []
             continue
         if cur and "identifier =" not in line and line.strip():
-            funcs[cur].append(line.rstrip())
+            funcs[cur].append(" ".join(line.split()))
     return funcs
 
 

@@ -78,6 +78,12 @@ SIGNATURES = {
     "b200_canny_frames_device_bgr": (C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_float, C.c_int, C.c_int]),
     "b200_cv_canny_frames_device": (C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int]),
     "b200_cv_canny_aperture_frames_device": (C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int]),
+    "b200_cv_gaussian_canny_device_strided": (C.c_int, [_ctx, _u8p, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                        C.c_int, C.c_int, C.c_double, C.c_double, C.c_double, C.c_double, C.c_int,
+                                                        C.c_int, _u8p, C.c_int64, C.c_int64]),
+    "b200_cv_gaussian_canny_frames_device": (C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double,
+                                                       C.c_double, C.c_double, C.c_int, C.c_int]),
+    "b200_cv_gaussian_kernel": (C.c_int, [C.c_int, C.c_double, C.POINTER(C.c_int), C.POINTER(C.c_int32)]),
     "b200_profile_stages_device": (C.c_int, [_ctx, _u8p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, _u8p, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "b200_profile_pipeline_device": (C.c_int, [_ctx, _u8p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_int, _u8p, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "b200_hash_edges_device": (C.c_int, [_ctx, _u8p, C.c_size_t, C.c_ulonglong, C.POINTER(C.c_ulonglong)]),

@@ -236,6 +236,32 @@ def cv_canny_device_strided_ptr(ctx: Optional[Context], d_in: int, in_row_pitch:
                                                        int(out_row_pitch), int(out_frame_stride)))
 
 
+def cv_gaussian_canny_device_strided_ptr(ctx: Optional[Context], d_in: int, in_row_pitch: int, in_frame_stride: int, n: int, h: int,
+                                         w: int, channels: int, ksize: Tuple[int, int], sigma_x: float, sigma_y: float,
+                                         threshold1: float, threshold2: float, aperture_size: int, l2_gradient: bool, d_edges: int,
+                                         out_row_pitch: int, out_frame_stride: int) -> None:
+    """cv2.Canny(cv2.GaussianBlur(frame, ksize, sigma_x, sigmaY=sigma_y), threshold1, threshold2, apertureSize=aperture_size,
+    L2gradient=l2_gradient) of every frame, bit for bit (b200_cv_gaussian_canny_device_strided; ksize is (width, height), each side
+    odd and at most 31, or <= 0 to derive it from its sigma).  Layout as cv_canny_device_strided_ptr.  Asynchronous on the
+    context's stream."""
+    kw, kh = ksize
+    check(load().b200_cv_gaussian_canny_device_strided(_h(ctx), C.c_void_p(d_in), int(in_row_pitch), int(in_frame_stride), n, h, w,
+                                                       int(channels), int(kw), int(kh), C.c_double(sigma_x), C.c_double(sigma_y),
+                                                       C.c_double(threshold1), C.c_double(threshold2), int(aperture_size),
+                                                       int(bool(l2_gradient)), C.c_void_p(d_edges), int(out_row_pitch),
+                                                       int(out_frame_stride)))
+
+
+def cv_gaussian_kernel(ksize: int, sigma: float) -> np.ndarray:
+    """The blur's 8.8 fixed-point taps for one axis as the cv_gaussian_canny calls use them (b200_cv_gaussian_kernel): ksize <= 0
+    is derived from sigma as cv2.GaussianBlur does.  Returns int32 taps of the resolved size, summing to 256.  Host code: needs no
+    GPU."""
+    n = C.c_int(0)
+    taps = (C.c_int32 * 31)()
+    check(load().b200_cv_gaussian_kernel(int(ksize), C.c_double(sigma), C.byref(n), taps))
+    return np.array(taps[:n.value], dtype=np.int32)
+
+
 def frame_list(descs) -> C.Array:
     """(in_ptr, in_pitch, out_ptr, out_pitch, h, w) tuples -> the ctypes array of b200_frame that b200_canny_frames_device takes."""
     descs = list(descs)
@@ -262,6 +288,18 @@ def cv_canny_frames_device_ptr(ctx: Optional[Context], descs, channels: int, thr
     at out_ptr + y*out_pitch + x; frames from 1 x 1.  Asynchronous on the context's stream."""
     descs = list(descs)
     check(load().b200_cv_canny_aperture_frames_device(_h(ctx), frame_list(descs), len(descs), int(channels), C.c_double(threshold1),
+                                                      C.c_double(threshold2), int(aperture_size), int(bool(l2_gradient))))
+
+
+def cv_gaussian_canny_frames_device_ptr(ctx: Optional[Context], descs, channels: int, ksize: Tuple[int, int], sigma_x: float,
+                                        sigma_y: float, threshold1: float, threshold2: float, aperture_size: int,
+                                        l2_gradient: bool) -> None:
+    """cv_gaussian_canny_device_strided_ptr's maps for frames of different sizes in one call, bit for bit
+    (b200_cv_gaussian_canny_frames_device).  descs as cv_canny_frames_device_ptr.  Asynchronous on the context's stream."""
+    descs = list(descs)
+    kw, kh = ksize
+    check(load().b200_cv_gaussian_canny_frames_device(_h(ctx), frame_list(descs), len(descs), int(channels), int(kw), int(kh),
+                                                      C.c_double(sigma_x), C.c_double(sigma_y), C.c_double(threshold1),
                                                       C.c_double(threshold2), int(aperture_size), int(bool(l2_gradient))))
 
 

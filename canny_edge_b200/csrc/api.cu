@@ -400,7 +400,23 @@ struct CvSpec {
     int channels;
     bool l2;
     int aperture;   // 3, 5 or 7
+    // cv::GaussianBlur before the Sobel stage (b200_cv_gaussian_canny_*): radii ksize / 2 per axis, both 0 for none (ksize (1, 1)
+    // included: the unblurred kernels run); the 8.8 fixed-point taps of b200_cv_gaussian_kernel, fx[0 .. 2*blur_rx] and
+    // fy[0 .. 2*blur_ry]
+    int blur_rx, blur_ry;
+    int32_t fx[31], fy[31];
 };
+
+// the blur of cv (none when both radii are 0) as the OpenCV front kernel takes it: the taps from the centre out
+static CvBlurParams cv_blur_params(const CvSpec& cv) {
+    CvBlurParams b;
+    memset(&b, 0, sizeof(b));
+    b.rx = cv.blur_rx;
+    b.ry = cv.blur_ry;
+    for (int t = 0; t <= cv.blur_rx; ++t) b.hx[t] = (int16_t)cv.fx[cv.blur_rx + t];
+    for (int t = 0; t <= cv.blur_ry; ++t) b.hy[t] = (int16_t)cv.fy[cv.blur_ry + t];
+    return b;
+}
 
 // Front + hysteresis with cv::Canny's semantics on frames [f0, f0+nf) of slot `slot` (run_frames_device's counterpart): the
 // OpenCV front kernel, then always the list-driven hysteresis kernels with plain 8-connectivity.  The uniform path's density state
@@ -420,7 +436,7 @@ static int run_frames_cv(b200_ctx* ctx, cudaStream_t st, int slot, const uint8_t
     // the list's counter block is zero here (see run_frames_device)
     if (ctx->list_dirty[slot]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
     ctx->list_dirty[slot] = true;
-    CB_TRY(launch_front_cv(ctx, st, fp, cv.channels, cv.l2, cv.aperture));
+    CB_TRY(launch_front_cv(ctx, st, fp, cv_blur_params(cv), cv.channels, cv.l2, cv.aperture));
     HystParams hp;
     memset(&hp, 0, sizeof(hp));
     hp.cls = d_out; hp.cls_pitch = lay.out_pitch; hp.cls_frame_stride = lay.out_frame_stride;
@@ -1007,13 +1023,107 @@ static int cv_thresholds(double t1, double t2, bool l2, int aperture, int* lo, i
     return B200_OK;
 }
 
+// cv::GaussianBlur's arguments (imgproc/src/smooth.dispatch.cpp) for 8-bit input.  Both sigmas finite (B200_ERR_INVALID_ARG; cv2
+// accepts NaN and inf, and its result is then no Gaussian blur); sigma_y <= 0 means sigma_x; a side <= 0 is derived from its sigma
+// when that is > 0, cvRound(sigma*3*2 + 1) | 1 (cvRound: half to even); both sides then odd and positive (B200_ERR_INVALID_ARG, where
+// cv2 asserts); at most 31 (B200_ERR_UNSUPPORTED, this build's limit); negative sigmas count as 0.
+static long long cv_gauss_side(int ksize, double sigma) {
+    if (ksize > 0 || !(sigma > 0)) return ksize;
+    const double d = sigma * 3 * 2 + 1;
+    return d < 1e9 ? ((long long)nearbyint(d) | 1) : (1LL << 40) + 1;   // far above the limit: cv2's int conversion would overflow
+}
+
+static int cv_gauss_sizes(int kw, int kh, double sx, double sy, int* nw, int* nh, double* sx_out, double* sy_out) {
+    if (!isfinite(sx) || !isfinite(sy)) { set_error("Gaussian sigmas must be finite (got %g, %g)", sx, sy); return B200_ERR_INVALID_ARG; }
+    if (sy <= 0) sy = sx;
+    const long long w = cv_gauss_side(kw, sx), h = cv_gauss_side(kh, sy);
+    if (w <= 0 || h <= 0 || (w & 1) == 0 || (h & 1) == 0) {
+        set_error("Gaussian ksize (%d, %d) with sigmas %g, %g: both sides must be odd and positive (or derived from a sigma > 0)", kw,
+                  kh, sx, sy);
+        return B200_ERR_INVALID_ARG;
+    }
+    if (w > 31 || h > 31) {
+        set_error("Gaussian ksize %lld x %lld: at most 31 per side are supported", w, h);
+        return B200_ERR_UNSUPPORTED;
+    }
+    *nw = (int)w; *nh = (int)h;
+    *sx_out = std::max(sx, 0.0); *sy_out = std::max(sy, 0.0);
+    return B200_OK;
+}
+
+// The 8.8 fixed-point taps of cv::GaussianBlur on 8-bit input for one axis of n (odd, 1 .. 31) taps and sigma >= 0:
+// getGaussianKernelBitExact, then the error-diffusion rounding of fixedSmoothInvoker's kernel conversion, summing to exactly 256.
+// The only mul-add pairs have exact products (k * 256, sum * 2), so a contraction into an FMA could not change a result; the one
+// fma of OpenCV's default sigma is written out.
+static void cv_gauss_taps(int n, double sigma, int32_t* f) {
+    double k[31];
+    if (sigma <= 0 && n <= 7) {
+        static const double small[4][7] = {{1}, {0.25, 0.5, 0.25}, {1 / 16., 4 / 16., 6 / 16., 4 / 16., 1 / 16.},
+                                           {1 / 32., 3.5 / 32., 7 / 32., 9 / 32., 7 / 32., 3.5 / 32., 1 / 32.}};
+        for (int i = 0; i < n; ++i) k[i] = small[n / 2][i];
+    } else {
+        const double s = sigma > 0 ? sigma : fma((double)n, 0.15, 0.35);
+        const double c = -0.125 / (s * s);
+        const int h = (n - 1) / 2;
+        double t[15], sum = 0;
+        for (int i = 0; i < h; ++i) {
+            const int x = 1 - n + 2 * i;
+            t[i] = exp((double)(x * x) * c);
+            sum += t[i];
+        }
+        sum = sum * 2 + 1;
+        const double m = 1 / sum;
+        for (int i = 0; i < h; ++i) k[i] = k[n - 1 - i] = t[i] * m;
+        k[h] = 1 * m;
+    }
+    double err = 0;
+    int acc = 0;
+    for (int i = 0; i < n / 2; ++i) {
+        const double a = k[i] * 256 + err;
+        const double v = nearbyint(a);   // cvRound: half to even
+        err = a - v;
+        f[i] = f[n - 1 - i] = (int32_t)v;
+        acc += (int32_t)v;
+    }
+    f[n / 2] = 256 - 2 * acc;
+}
+
+int b200_cv_gaussian_kernel(int ksize, double sigma, int* ksize_out, int32_t* taps) {
+    if (!ksize_out || !taps) { set_error("null output pointer"); return B200_ERR_INVALID_ARG; }
+    int n, n2;
+    double s, s2;
+    CB_TRY(cv_gauss_sizes(ksize, ksize, sigma, sigma, &n, &n2, &s, &s2));
+    for (int i = 0; i < 31; ++i) taps[i] = 0;
+    cv_gauss_taps(n, s, taps);
+    *ksize_out = n;
+    return B200_OK;
+}
+
+// cv::GaussianBlur's arguments of b200_cv_gaussian_canny_*
+struct CvGaussArgs {
+    int ksize_w, ksize_h;
+    double sigma_x, sigma_y;
+};
+
 // The checks of the OpenCV calls that come before the layout's: channel count (UNSUPPORTED), aperture (INVALID_ARG, as cv::Canny
-// rejects it), the uniform call's height (max_height; UNSUPPORTED), thresholds
-static int cv_spec(int channels, int aperture, int height, int max_height, double t1, double t2, int l2_gradient, CvSpec* cv) {
+// rejects it), the blur's arguments when there is one (cv_gauss_sizes), the uniform call's height (max_height; UNSUPPORTED),
+// thresholds
+static int cv_spec(int channels, int aperture, const CvGaussArgs* blur, int height, int max_height, double t1, double t2,
+                   int l2_gradient, CvSpec* cv) {
+    *cv = CvSpec();
     if (channels != 1 && channels != 3) { set_error("channels must be 1 or 3 (got %d)", channels); return B200_ERR_UNSUPPORTED; }
     if (aperture != 3 && aperture != 5 && aperture != 7) {
         set_error("aperture size must be 3, 5 or 7 (got %d)", aperture);
         return B200_ERR_INVALID_ARG;
+    }
+    if (blur) {
+        int nw, nh;
+        double sx, sy;
+        CB_TRY(cv_gauss_sizes(blur->ksize_w, blur->ksize_h, blur->sigma_x, blur->sigma_y, &nw, &nh, &sx, &sy));
+        cv_gauss_taps(nw, sx, cv->fx);
+        cv_gauss_taps(nh, sy, cv->fy);
+        cv->blur_rx = nw / 2;
+        cv->blur_ry = nh / 2;
     }
     if (height > max_height) { set_error("height %d: at most %d rows (65535 tiles of 64)", height, max_height); return B200_ERR_UNSUPPORTED; }
     cv->channels = channels;
@@ -1027,7 +1137,18 @@ int b200_cv_canny_aperture_device_strided(b200_ctx* ctx, const uint8_t* d_in, in
                                           int aperture_size, int l2_gradient, uint8_t* d_edges, int64_t out_row_pitch,
                                           int64_t out_frame_stride) {
     CvSpec cv;
-    CB_TRY(cv_spec(channels, aperture_size, height, kCvMaxHeight, threshold1, threshold2, l2_gradient, &cv));
+    CB_TRY(cv_spec(channels, aperture_size, nullptr, height, kCvMaxHeight, threshold1, threshold2, l2_gradient, &cv));
+    return batch_device_impl(ctx, d_in, in_row_pitch, in_frame_stride, n_frames, height, width, 0.f, 0, 0, d_edges, out_row_pitch,
+                             out_frame_stride, channels, &cv);
+}
+
+int b200_cv_gaussian_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride,
+                                          int n_frames, int height, int width, int channels, int ksize_w, int ksize_h, double sigma_x,
+                                          double sigma_y, double threshold1, double threshold2, int aperture_size, int l2_gradient,
+                                          uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride) {
+    const CvGaussArgs blur = {ksize_w, ksize_h, sigma_x, sigma_y};
+    CvSpec cv;
+    CB_TRY(cv_spec(channels, aperture_size, &blur, height, kCvMaxHeight, threshold1, threshold2, l2_gradient, &cv));
     return batch_device_impl(ctx, d_in, in_row_pitch, in_frame_stride, n_frames, height, width, 0.f, 0, 0, d_edges, out_row_pitch,
                              out_frame_stride, channels, &cv);
 }
@@ -1254,7 +1375,7 @@ static int run_ragged_cv_chunk(b200_ctx* ctx, cudaStream_t st, int s, const b200
     // the list's counter block is zero here (see run_frames_device)
     if (ctx->list_dirty[s]) CB_CUDA(cudaMemsetAsync(fp.kept_count, 0, 64, st));
     ctx->list_dirty[s] = true;
-    CB_TRY(launch_front_cv_ragged(ctx, st, fp, (int)items.size(), cv.channels, cv.l2, cv.aperture));
+    CB_TRY(launch_front_cv_ragged(ctx, st, fp, cv_blur_params(cv), (int)items.size(), cv.channels, cv.l2, cv.aperture));
     RaggedHystParams hp;
     memset(&hp, 0, sizeof(hp));
     hp.frames = fp.rframes;
@@ -1343,7 +1464,16 @@ int b200_cv_canny_aperture_frames_device(b200_ctx* ctx, const b200_frame* frames
                                          double threshold2, int aperture_size, int l2_gradient) {
     CvSpec cv;
     // a list's 1-D grid has no height limit
-    CB_TRY(cv_spec(channels, aperture_size, 0, INT_MAX, threshold1, threshold2, l2_gradient, &cv));
+    CB_TRY(cv_spec(channels, aperture_size, nullptr, 0, INT_MAX, threshold1, threshold2, l2_gradient, &cv));
+    return frames_device_impl(ctx, frames, n_frames, 0.f, 0, 0, channels, &cv);
+}
+
+int b200_cv_gaussian_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, int ksize_w, int ksize_h,
+                                         double sigma_x, double sigma_y, double threshold1, double threshold2, int aperture_size,
+                                         int l2_gradient) {
+    const CvGaussArgs blur = {ksize_w, ksize_h, sigma_x, sigma_y};
+    CvSpec cv;
+    CB_TRY(cv_spec(channels, aperture_size, &blur, 0, INT_MAX, threshold1, threshold2, l2_gradient, &cv));
     return frames_device_impl(ctx, frames, n_frames, 0.f, 0, 0, channels, &cv);
 }
 

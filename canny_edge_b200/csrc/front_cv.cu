@@ -1,7 +1,9 @@
 // front_cv.cu — the front kernel of the OpenCV-compatible path (b200_cv_canny_aperture_device_strided, and
 // b200_cv_canny_aperture_frames_device through the RAGGED variant below): 1- or 3-channel u8 frames -> class map (0 / 1 weak / 255
 // strong) plus the weak-pixel hand-over of the list-driven hysteresis kernels, with cv::Canny's arithmetic (apertureSize K = 3, 5 or
-// 7) bit for bit.  No blur: the K x K Sobel kernels on the input, BORDER_REPLICATE for both derivatives.
+// 7) bit for bit.  No blur: the K x K Sobel kernels on the input, BORDER_REPLICATE for both derivatives.  With a blur class BR > 0
+// (b200_cv_gaussian_canny_*: BR = 3 for radii up to 3, 15 up to 15; the radii and taps in CvBlurParams), phase 1 is stage_blurred:
+// cv::GaussianBlur's 8-bit fixed-point blur on the staged tile, so s_in holds the blurred frame and phases 2-4 are the same code.
 //
 // One CTA = one 128 x 64 tile of one frame, 288 threads (9 warps); R = K / 2:
 //   1. staging: input rows y0-1-R .. y0+64+R, pixels x0-16 .. x0+143 (C bytes each) into shared memory, with the coordinates
@@ -58,19 +60,137 @@ __host__ __device__ constexpr int deriv_tap(int K, int t) {
                   : (t == 0 ? -1 : t == 1 ? -4 : t == 2 ? -5 : t == 3 ? 0 : t == 4 ? 5 : t == 5 ? 4 : 1);
 }
 
-template <int C, int K>
+template <int C, int K, int BR = 0>
 struct Smem {
     static constexpr int kSH = kTH + 2 + 2 * (K / 2);          // staged rows: y0-1-R .. y0+64+R
     static constexpr int in_row = C * kSW;                     // bytes per staged row, a multiple of 16
     static constexpr int in_bytes = kSH * in_row;
     static constexpr int m_off = (in_bytes + 15) & ~15;
     static constexpr int sum_off = m_off + kMR * kMP * 4;      // per-warp weak counts, then the CTA's list base
-    static constexpr int total = sum_off + 16 * 4;
+    // Gaussian pre-blur (BR = 3 or 15, the largest radius of the class; 0: none): the raw rows and one strip of column sums alias
+    // s_m and s_sum, which phase 2 writes only after the blur has filled s_in.  Raw pixel u of a row is x0 - kXOff + u; the column
+    // pass covers raw pixels kULo .. kUHi-1 (every pixel the row pass reads for staged pixels 8 .. 151, a superset of what phase 2
+    // reads); the row pass writes staged pixels 8 .. 151.
+    static constexpr int kXOff = BR <= 3 ? 16 : 32;
+    static constexpr int raw_row = C * (kSW - 32 + 2 * kXOff);  // 160 or 192 pixels, a multiple of 16 bytes
+    static constexpr int raw_rows = kSH + 2 * BR;
+    static constexpr int raw_bytes = raw_rows * raw_row;
+    static constexpr int kULo = BR <= 3 ? 4 : 8, kUHi = BR <= 3 ? 156 : 184;
+    static constexpr int v_row = C * (kUHi - kULo);            // u16 column sums per strip row
+    // strip rows: every staged row for gray; for 3 channels as many as keep 3 CTAs per SM (radius <= 3) or 2 (radius <= 15)
+    static constexpr int strip = C == 1 ? kSH : BR <= 3 ? 4 : 16;
+    static constexpr int blur_bytes = raw_bytes + strip * v_row * 2;
+    static constexpr int total = BR == 0 ? sum_off + 16 * 4 : std::max(sum_off + 16 * 4, m_off + blur_bytes);
 };
 
-template <int C, bool L2, bool RAGGED, int K>
+// reflect-101 index into 0 .. n-1 (OpenCV's BORDER_REFLECT_101 / BORDER_DEFAULT), repeated with period 2(n - 1) when the kernel is
+// wider than the frame; a 1-pixel side always maps to 0
+__device__ __forceinline__ int reflect101(int x, int n) {
+    if ((unsigned)x < (unsigned)n) return x;
+    if (n == 1) return 0;
+    const int per = 2 * (n - 1);
+    x %= per;
+    if (x < 0) x += per;
+    return x < n ? x : per - x;
+}
+
+// Phase 1 with cv::GaussianBlur before the Sobel stage: s_in receives, at every staged position phase 2 reads, the blurred pixel B at
+// the position's clamped coordinates (cv::Canny's BORDER_REPLICATE applies to B, not to the raw frame), so phases 2-4 are unchanged.
+//   a. raw rows y0-1-R-ry .. y0+64+R+ry and pixels x0-kXOff .. through reflect101 into s_raw: 16-byte loads where the chunk lies
+//      inside the row and is aligned (no reflection needed there), byte loads elsewhere;
+//   b. per strip of staged rows: the column pass (8.8 taps of fy, folded: each tap multiplies the sum of the two mirrored rows) of
+//      each staged row's clamped row into u16 sums (<= 255 * 256), then the row pass over them with fx, (sum + 2^15) >> 16 into s_in.
+// Every sum is an exact integer below 2^24, so the order of summation does not matter.
+template <int C, int K, int BR>
+__device__ __forceinline__ void stage_blurred(const CvBlurParams& b, unsigned char* smem, const uint8_t* in_f, long long in_pitch,
+                                              int x0, int y0, int W, int H) {
+    using S = Smem<C, K, BR>;
+    constexpr int R = K / 2;
+    const int tid = threadIdx.x;
+    const int rx = b.rx, ry = b.ry;
+    unsigned char* s_in = smem;
+    unsigned char* s_raw = smem + S::m_off;
+    uint16_t* s_v = reinterpret_cast<uint16_t*>(smem + S::m_off + S::raw_bytes);
+    {
+        constexpr int kChunks = S::raw_row / 16;
+        const long long row_bytes = (long long)C * W;
+        const long long xb = (long long)(x0 - S::kXOff) * C;
+        const int n_rows = S::kSH + 2 * ry;
+        for (int i = tid; i < n_rows * kChunks; i += kThreads) {
+            const int r = i / kChunks, q = i - r * kChunks;
+            const int y = reflect101(y0 - 1 - R - ry + r, H);
+            const uint8_t* row = in_f + (long long)y * in_pitch;
+            const long long b0 = xb + 16 * q;
+            uint4 v;
+            if (b0 >= 0 && b0 + 16 <= row_bytes && ((reinterpret_cast<uintptr_t>(row + b0) & 15) == 0)) {
+                v = __ldg(reinterpret_cast<const uint4*>(row + b0));
+            } else {
+                uint32_t wd[4] = {0, 0, 0, 0};
+#pragma unroll
+                for (int e = 0; e < 16; ++e) {
+                    const int s = 16 * q + e;
+                    const int x = reflect101(x0 - S::kXOff + s / C, W);
+                    wd[e >> 2] |= (uint32_t)row[(long long)x * C + (s % C)] << (8 * (e & 3));
+                }
+                v = make_uint4(wd[0], wd[1], wd[2], wd[3]);
+            }
+            *reinterpret_cast<uint4*>(s_raw + r * S::raw_row + 16 * q) = v;
+        }
+    }
+    __syncthreads();
+    constexpr int kVGroups = S::v_row / 4;                      // 4 column sums per thread and step
+    constexpr int kOutLo = 8, kOutGroups = C * 144 / 4;          // staged pixels 8 .. 151, 4 bytes per thread and step
+#pragma unroll 1
+    for (int r0 = 0; r0 < S::kSH; r0 += S::strip) {
+        // column pass: strip row sr holds the sums of staged row r0 + sr, centred on its clamped row (raw row qc + ry)
+        for (int i = tid; i < S::strip * kVGroups; i += kThreads) {
+            const int sr = i / kVGroups, g = i - sr * kVGroups;
+            if (r0 + sr >= S::kSH) break;
+            const int qc = min(max(y0 - 1 - R + r0 + sr, 0), H - 1) - (y0 - 1 - R);
+            const unsigned char* src = s_raw + (qc + ry) * S::raw_row + C * S::kULo + 4 * g;
+            const uint32_t w0 = *reinterpret_cast<const uint32_t*>(src);
+            int a[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) a[e] = b.hy[0] * (int)((w0 >> (8 * e)) & 255);
+#pragma unroll
+            for (int t = 1; t <= BR; ++t) {
+                if (t > ry) break;
+                const uint32_t wu = *reinterpret_cast<const uint32_t*>(src - t * S::raw_row);
+                const uint32_t wd = *reinterpret_cast<const uint32_t*>(src + t * S::raw_row);
+#pragma unroll
+                for (int e = 0; e < 4; ++e) a[e] += b.hy[t] * (int)(((wu >> (8 * e)) & 255) + ((wd >> (8 * e)) & 255));
+            }
+            *reinterpret_cast<uint2*>(s_v + sr * S::v_row + 4 * g) =
+                make_uint2((uint32_t)a[0] | (uint32_t)a[1] << 16, (uint32_t)a[2] | (uint32_t)a[3] << 16);
+        }
+        __syncthreads();
+        // row pass: staged pixel s of staged row r0 + sr is B at the clamped column, raw pixel xc - x0 + kXOff
+        for (int i = tid; i < S::strip * kOutGroups; i += kThreads) {
+            const int sr = i / kOutGroups, g = i - sr * kOutGroups;
+            if (r0 + sr >= S::kSH) break;
+            uint32_t word = 0;
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const int ob = C * kOutLo + 4 * g + e, s = ob / C, c = ob - s * C;
+                const int u = min(max(x0 - 16 + s, 0), W - 1) - x0 + S::kXOff;
+                const uint16_t* vp = s_v + sr * S::v_row + (u - S::kULo) * C + c;
+                int acc = b.hx[0] * (int)vp[0];
+#pragma unroll
+                for (int t = 1; t <= BR; ++t) {
+                    if (t > rx) break;
+                    acc += b.hx[t] * ((int)vp[-t * C] + (int)vp[t * C]);
+                }
+                word |= (uint32_t)((acc + 32768) >> 16) << (8 * e);
+            }
+            *reinterpret_cast<uint32_t*>(s_in + (r0 + sr) * S::in_row + C * kOutLo + 4 * g) = word;
+        }
+        __syncthreads();
+    }
+}
+
+template <int C, bool L2, bool RAGGED, int K, int BR>
 __global__ void __launch_bounds__(kThreads)
-front_cv_kernel(const FrontParams p) {
+front_cv_kernel(const FrontParams p, const CvBlurParams blur) {
     extern __shared__ __align__(16) unsigned char smem[];
     using S = Smem<C, K>;
     constexpr int R = K / 2;
@@ -92,8 +212,10 @@ front_cv_kernel(const FrontParams p) {
     const uint8_t* in_f = RAGGED ? fd.in : p.in + (long long)frame * p.in_frame_stride;
     const long long in_pitch = RAGGED ? fd.in_pitch : p.in_pitch;
 
-    // ---- 1. staging, clamped coordinates ----
-    {
+    // ---- 1. staging, clamped coordinates (BR > 0: of the blurred frame, stage_blurred) ----
+    if constexpr (BR > 0) {
+        stage_blurred<C, K, BR>(blur, smem, in_f, in_pitch, x0, y0, W, H);
+    } else {
         constexpr int kChunks = S::in_row / 16;
         const long long row_bytes = (long long)C * W;
         const long long xb = (long long)(x0 - 16) * C;         // byte of staged pixel 0 within its row (a multiple of 16 - 48C)
@@ -117,8 +239,8 @@ front_cv_kernel(const FrontParams p) {
             }
             *reinterpret_cast<uint4*>(s_in + r * S::in_row + 16 * q) = v;
         }
+        __syncthreads();
     }
-    __syncthreads();
 
     // ---- 2. gradients, magnitude, direction class of the 130 x 66 region ----
     if (tid < 2 * (kTW + 2)) {
@@ -306,48 +428,62 @@ front_cv_kernel(const FrontParams p) {
     }
 }
 
-template <int C, bool L2, bool RAGGED, int K>
-static int launch_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, dim3 grid) {
+template <int C, bool L2, bool RAGGED, int K, int BR>
+static int launch_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CvBlurParams& blur, dim3 grid) {
     static bool configured[64] = {false};  // per instantiation, per device
     if (!configured[ctx->device & 63]) {
-        CB_CUDA(cudaFuncSetAttribute(front_cv_kernel<C, L2, RAGGED, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<C, K>::total));
+        CB_CUDA(cudaFuncSetAttribute(front_cv_kernel<C, L2, RAGGED, K, BR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     Smem<C, K, BR>::total));
         configured[ctx->device & 63] = true;
     }
     {
         ProfScope ps(ctx, st, 0);
-        front_cv_kernel<C, L2, RAGGED, K><<<grid, kThreads, Smem<C, K>::total, st>>>(p);
+        front_cv_kernel<C, L2, RAGGED, K, BR><<<grid, kThreads, Smem<C, K, BR>::total, st>>>(p, blur);
     }
     CB_CUDA(cudaGetLastError());
     ctx->launches++;
     return B200_OK;
 }
 
-// the instantiation for channels (1 or 3), l2 and aperture (3, 5 or 7; checked by the caller)
+// the instantiation for channels (1 or 3), l2, aperture (3, 5 or 7; checked by the caller) and the blur's radius class (the larger
+// of blur.rx and blur.ry: 0 none, <= 3, <= 15)
 template <bool RAGGED>
-static int launch_cv_any(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, dim3 grid, int channels, bool l2, int aperture) {
+static int launch_cv_any(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CvBlurParams& blur, dim3 grid, int channels,
+                         bool l2, int aperture) {
+    const int br = std::max(blur.rx, blur.ry);
+    if (blur.rx < 0 || blur.ry < 0 || br > 15) {
+        set_error("OpenCV front kernel: blur radii %d, %d (0 .. 15 are supported)", blur.rx, blur.ry);
+        return B200_ERR_UNSUPPORTED;
+    }
+#define CB_CV_LAUNCH_BR(K, BR)                                                                                                             \
+    if (channels == 1) return l2 ? launch_cv<1, true, RAGGED, K, BR>(ctx, st, p, blur, grid) : launch_cv<1, false, RAGGED, K, BR>(ctx, st, p, blur, grid); \
+    if (channels == 3) return l2 ? launch_cv<3, true, RAGGED, K, BR>(ctx, st, p, blur, grid) : launch_cv<3, false, RAGGED, K, BR>(ctx, st, p, blur, grid);
 #define CB_CV_LAUNCH(K)                                                                                                                  \
     if (aperture == K) {                                                                                                               \
-        if (channels == 1) return l2 ? launch_cv<1, true, RAGGED, K>(ctx, st, p, grid) : launch_cv<1, false, RAGGED, K>(ctx, st, p, grid); \
-        if (channels == 3) return l2 ? launch_cv<3, true, RAGGED, K>(ctx, st, p, grid) : launch_cv<3, false, RAGGED, K>(ctx, st, p, grid); \
+        if (br == 0) { CB_CV_LAUNCH_BR(K, 0) }                                                                                         \
+        else if (br <= 3) { CB_CV_LAUNCH_BR(K, 3) }                                                                                    \
+        else { CB_CV_LAUNCH_BR(K, 15) }                                                                                                \
     }
     CB_CV_LAUNCH(3)
     CB_CV_LAUNCH(5)
     CB_CV_LAUNCH(7)
 #undef CB_CV_LAUNCH
+#undef CB_CV_LAUNCH_BR
     set_error("OpenCV front kernel: %d channels, aperture %d (1 or 3 channels, aperture 3, 5 or 7 are supported)", channels, aperture);
     return B200_ERR_UNSUPPORTED;
 }
 
 }  // namespace fcv
 
-int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, int channels, bool l2, int aperture) {
+int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p_in, const CvBlurParams& blur, int channels, bool l2,
+                    int aperture) {
     FrontParams p = p_in;
     if (!p.parent || !p.kept_list || !p.kept_count) { set_error("internal: OpenCV front kernel without a weak-pixel list"); return B200_ERR_INVALID_ARG; }
     // aligned 32-bit class stores need base, row pitch and frame stride on 4-byte boundaries (tile columns are multiples of 4)
     p.cls_words = ((reinterpret_cast<uintptr_t>(p.cls) | (uintptr_t)p.cls_pitch | (uintptr_t)(p.n_frames > 1 ? p.cls_frame_stride : 0)) & 3) == 0;
     const dim3 grid((p.width + fcv::kTW - 1) / fcv::kTW, (p.height + fcv::kTH - 1) / fcv::kTH, p.n_frames);
     ctx->front_fast++;
-    return fcv::launch_cv_any<false>(ctx, st, p, grid, channels, l2, aperture);
+    return fcv::launch_cv_any<false>(ctx, st, p, blur, grid, channels, l2, aperture);
 }
 
 void ragged_items_cv(int frame, int height, int width, std::vector<RaggedItem>& items) {
@@ -355,7 +491,8 @@ void ragged_items_cv(int frame, int height, int width, std::vector<RaggedItem>& 
         for (int x0 = 0; x0 < width; x0 += fcv::kTW) items.push_back(RaggedItem{frame, x0, y0, std::min(height, y0 + fcv::kTH)});
 }
 
-int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, int channels, bool l2, int aperture) {
+int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CvBlurParams& blur, int n_items, int channels,
+                           bool l2, int aperture) {
     if (!p.parent || !p.kept_list || !p.kept_count || !p.rframes || !p.ritems) {
         set_error("internal: ragged OpenCV front kernel without its table or weak-pixel list");
         return B200_ERR_INVALID_ARG;
@@ -363,7 +500,7 @@ int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p,
     if (n_items <= 0) return B200_OK;
     const dim3 grid(n_items);
     ctx->front_fast++;
-    return fcv::launch_cv_any<true>(ctx, st, p, grid, channels, l2, aperture);
+    return fcv::launch_cv_any<true>(ctx, st, p, blur, grid, channels, l2, aperture);
 }
 
 }  // namespace cb

@@ -98,6 +98,13 @@ struct FrontParams {
     const CUtensorMap_st* rtmaps;
 };
 
+// front_cv's second parameter: cv::GaussianBlur before the Sobel stage (b200_cv_gaussian_canny_*).  Radii (ksize / 2) per axis, both
+// 0 for no blur; the 8.8 fixed-point taps from the centre out (hx[t] = fx[rx + t] = fx[rx - t]), zero past the radius
+struct CvBlurParams {
+    int rx, ry;
+    int16_t hx[16], hy[16];
+};
+
 // ---- ragged chunks: frames of different sizes in one launch --------------------------------------
 // One frame of a chunk as the kernels see it.  Frames are whole images (row 0 is the image's row 0).  Union-find slots and list
 // indices stay dense and launch-relative: pixel (y, x) of the frame is slot base + y*width + x, base being the sum of h*w over
@@ -301,12 +308,13 @@ int ragged_tensor_map3(const uint8_t* in, long long pitch, int height, int width
 int launch_front3_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, bool use_tma);
 // front_cv.cu (cv::Canny semantics, b200_cv_canny_aperture_device_strided): class map + weak-pixel list of p's frames, channels 1 or
 // 3 interleaved, Sobel aperture 3, 5 or 7, L1 or L2 magnitude against p.lo / p.hi (already divided for aperture 7, floored and, for
-// L2, squared)
-int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int channels, bool l2, int aperture);
+// L2, squared), after cv::GaussianBlur when blur's radii are not both 0
+int launch_front_cv(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CvBlurParams& blur, int channels, bool l2, int aperture);
 // ragged chunks (b200_cv_canny_aperture_frames_device): the work items of one frame (its 128 x 64 tiles), and the launch over n_items items of
 // p.ritems with the frames of p.rframes
 void ragged_items_cv(int frame, int height, int width, std::vector<RaggedItem>& items);
-int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, int n_items, int channels, bool l2, int aperture);
+int launch_front_cv_ragged(b200_ctx* ctx, cudaStream_t st, const FrontParams& p, const CvBlurParams& blur, int n_items, int channels,
+                           bool l2, int aperture);
 // selftest.cu
 int check_div_mode_device(b200_ctx* ctx, float b, float y, float* c, int* mode);
 // hysteresis.cu

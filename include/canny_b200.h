@@ -300,6 +300,44 @@ int b200_cv_canny_aperture_frames_device(b200_ctx* ctx, const b200_frame* frames
 int b200_cv_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, double threshold1,
                                 double threshold2, int l2_gradient);
 
+/* cv::Canny of a Gaussian-blurred frame: the edge maps of
+ *   cv::GaussianBlur(image, blurred, cv::Size(ksize_w, ksize_h), sigma_x, sigma_y);   (default border, BORDER_REFLECT_101)
+ *   cv::Canny(blurred, edges, threshold1, threshold2, aperture_size, l2_gradient);
+ * bit for bit (OpenCV 4.x, 8-bit input), for uniform batches (the layout of b200_cv_canny_aperture_device_strided) and for lists of
+ * frames of different sizes (that of b200_cv_canny_aperture_frames_device).  The blur runs inside the front kernel, on the staged
+ * tile: no blurred frame is written to memory.  For 3-channel frames every channel is blurred, then the per-pixel channel choice of
+ * cv::Canny follows.  The Sobel stage's BORDER_REPLICATE applies to the blurred frame.
+ * Arguments, as cv::GaussianBlur takes them:
+ *   sigma_y <= 0 means sigma_y = sigma_x;
+ *   a side of ksize that is <= 0 is derived from its sigma when that is > 0: cvRound(sigma*3*2 + 1) | 1, rounding half to even
+ *   (sigma 1.4 -> 9, 2 -> 13, 5 -> 31);
+ *   after that both sides must be odd and positive;
+ *   negative sigmas then count as 0 (sigma 0: OpenCV's default for the size, 0.3*((n-1)*0.5 - 1) + 0.8, and for n = 3, 5, 7 its
+ *   fixed tables 1 2 1 / 4, 1 4 6 4 1 / 16, 1 3.5 7 9 7 3.5 1 / 32);
+ *   ksize (1, 1) is the identity: the maps of the unblurred call.
+ * Arithmetic: per axis, 8.8 fixed-point taps summing to 256 (b200_cv_gaussian_kernel); blurred pixel
+ * B(y, x) = (sum_i sum_j fy[i]*fx[j]*I(r(y+i-ry), r(x+j-rx)) + 2^15) >> 16, r(.) reflecting with period 2*(len-1) when the kernel is
+ * wider than the frame (a 1-pixel side always reads index 0).  Every sum is an exact integer.
+ * Before any device work, in this order: B200_ERR_UNSUPPORTED for channels other than 1 and 3; B200_ERR_INVALID_ARG for an
+ * aperture_size other than 3, 5 and 7; B200_ERR_INVALID_ARG for a NaN or infinite sigma (a deliberate difference: cv2 accepts them,
+ * and its result is then no Gaussian blur); B200_ERR_INVALID_ARG for a side that is not odd and positive after the derivation
+ * (e.g. (0, 0) with sigma 0, (4, 4), (0, 5) with sigma 0), where cv2 asserts; B200_ERR_UNSUPPORTED for a side above 31 (this
+ * build's limit; derived sides pass it above sigma 5); then the checks of the unblurred call: for the uniform call the height, the
+ * thresholds and the layout, for the list the thresholds and the list. */
+int b200_cv_gaussian_canny_device_strided(b200_ctx* ctx, const uint8_t* d_in, int64_t in_row_pitch, int64_t in_frame_stride,
+                                          int n_frames, int height, int width, int channels, int ksize_w, int ksize_h, double sigma_x,
+                                          double sigma_y, double threshold1, double threshold2, int aperture_size, int l2_gradient,
+                                          uint8_t* d_edges, int64_t out_row_pitch, int64_t out_frame_stride);
+int b200_cv_gaussian_canny_frames_device(b200_ctx* ctx, const b200_frame* frames, int n_frames, int channels, int ksize_w, int ksize_h,
+                                         double sigma_x, double sigma_y, double threshold1, double threshold2, int aperture_size,
+                                         int l2_gradient);
+/* The blur's kernel for one axis, as the calls above use it (host code, no device or context needed): ksize and sigma resolved as
+ * above (with sigma_y = sigma_x = sigma), the size in *ksize_out and the 8.8 fixed-point taps in taps[0 .. *ksize_out - 1]
+ * (taps[31], the rest set to 0).  getGaussianKernelBitExact, then each half rounded to 1/256 with the error carried from tap to
+ * tap (half to even), the centre tap making the sum exactly 256.  Errors as above: B200_ERR_INVALID_ARG for a null pointer, a NaN or
+ * infinite sigma, or a size that is not odd and positive; B200_ERR_UNSUPPORTED for a size above 31. */
+int b200_cv_gaussian_kernel(int ksize, double sigma, int* ksize_out, int32_t* taps);
+
 /* The packed form of an edge map — 1 bit per pixel, bit i of byte k <-> pixel 8k+i, ceil(n_px/32)*4 bytes — is what
  * b200_canny_batch_host moves over PCIe.  Both halves are exported for callers that store or ship maps in that form:
  *   b200_pack_edges_device   0 / 255 bytes in DEVICE memory -> packed words in DEVICE memory, asynchronous on the context's
